@@ -7,6 +7,8 @@
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -24,6 +26,11 @@ REG_FIELDS = ["rb", "re", "qb", "qe", "rid", "score", "truesc", "sub", "csub", "
               "secondary", "seedlen0", "n_comp", "is_alt", "frac_rep_bits", "secondary_all"]
 
 _p = lambda a, t: a.ctypes.data_as(C.POINTER(t))
+
+# Where oracle/_ref is not built, the tests that compare with the reference's output compare with a digest of it recorded in
+# tests/golden/reference/ (see its README).  EMAB_RECORD_REFERENCE=<dir> writes the recordings of cases that have none there.
+RECORDED_DIR = os.path.join(ROOT, "tests", "golden", "reference")
+RECORD_TO = os.environ.get("EMAB_RECORD_REFERENCE")
 
 
 def nt4(seq: bytes | str) -> np.ndarray:
@@ -108,6 +115,65 @@ def ref():
 
 def ref_bin(name: str) -> str:
     return os.path.join(REF_DIR, name)
+
+
+def sha(*parts) -> str:
+    """SHA-256 over the parts (bytes as they are, anything else by repr)"""
+    h = hashlib.sha256()
+    for x in parts:
+        h.update(x if isinstance(x, bytes) else repr(x).encode())
+        h.update(b"\0")
+    return h.hexdigest()
+
+
+def recorded_reference(key: str, ours):
+    """The recorded digest of the reference's output for case `key` (tests/golden/reference/digests.json).  In record mode a
+    case without a recording is recorded as `ours` (this build's digest of the same output) into $EMAB_RECORD_REFERENCE."""
+    path = os.path.join(RECORDED_DIR, "digests.json")
+    rec = json.load(open(path)) if os.path.exists(path) else {}
+    if key not in rec and RECORD_TO:
+        os.makedirs(RECORD_TO, exist_ok=True)
+        out = os.path.join(RECORD_TO, "digests.json")
+        new = json.load(open(out)) if os.path.exists(out) else {}
+        new[key] = ours
+        json.dump(new, open(out, "w"), indent=1, sort_keys=True)
+        return ours
+    assert key in rec, f"no recorded reference output for {key} in {path}"
+    return rec[key]
+
+
+def split_sam(text: bytes):
+    """SAM text -> (header lines minus @PG, which echoes argv; records)"""
+    lines = text.split(b"\n")
+    head = [l for l in lines if l.startswith(b"@") and not l.startswith(b"@PG")]
+    body = [l for l in lines if l and not l.startswith(b"@")]
+    return head, body
+
+
+def diff_msg(a, b):
+    for i, (x, y) in enumerate(zip(a, b)):
+        if x != y:
+            return f"first difference at record {i}:\n ours: {x[:300]!r}\n ref:  {y[:300]!r}"
+    return f"record counts differ: {len(a)} vs {len(b)}"
+
+
+def compare_sam_with_reference(key, ours: bytes, run_reference, tmp_path, min_records=1):
+    """This build's SAM text against the reference's on the same input: the header minus @PG and every record, byte for
+    byte.  run_reference(out_path) runs oracle/_ref/ema where it is built; elsewhere the recorded digest of the reference's
+    output for case `key` stands in for it.  Returns this build's records."""
+    h1, b1 = split_sam(ours)
+    if os.path.exists(ref_bin("ema")):
+        out = os.path.join(str(tmp_path), "ref.sam")
+        run_reference(out)
+        h2, b2 = split_sam(open(out, "rb").read())
+        assert h1 == h2
+        assert len(b2) >= min_records
+        assert b1 == b2, diff_msg(b1, b2)
+    else:
+        assert len(b1) >= min_records
+        d = sha(b"\n".join(h1), b"\n".join(b1))
+        assert d == recorded_reference(key, d), f"{key}: SAM differs from the reference's recorded output"
+    return b1
 
 
 # ---- batched SW wrappers with one signature for both checkers -------------------------------------

@@ -98,16 +98,20 @@ def test_stage_regions_vs_hostsim(emab):
                 assert np.array_equal(res["regs"][off[2 * i + 1]:off[2 * i + 2]], a2[:n2.value]), (stage, lines[i][1])
 
 
-def test_candidates_vs_reference_c1(emab, ref_lib):
-    """BASELINE config 1 with planted repeats + indels: 10k pairs against the compiled reference."""
+def test_candidates_vs_reference_c1(emab):
+    """BASELINE config 1 with planted repeats + indels: 3000 pairs against the compiled reference (without oracle/_ref:
+    against the recorded digest of the reference's candidates)."""
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("bwa")):
-        pytest.skip("oracle/_ref/bwa missing")
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=emab.index_build)
     ix = emab.Index(p["fasta"])
     ctx = emab.Context(ix)
     lines = helpers.read_bucket(p["bucket"], 3000)
     got, res = pipeline_candidates(emab, ctx, lines)
+    if not helpers.have_ref():
+        d = helpers.sha(got)
+        assert d == helpers.recorded_reference("candidates_c1_rep_3000", d), "candidates differ from the reference's recorded ones"
+        return
+    ref_lib = helpers.ref()
     ref_lib.ref_ema_init.argtypes = [C.c_char_p, C.c_char_p]
     assert ref_lib.ref_ema_init(p["fasta"].encode(), b"10x") == 0
     bad = 0
@@ -162,9 +166,8 @@ def test_rescue_plan_is_transparent(emab, monkeypatch):
     on the golden bucket and on the repeat/indel variant of BASELINE configs[0] (where rescues chain)."""
     from tools import synth
     cases = [(os.path.join(G, "tiny_rep", "ref.fa"), helpers.read_bucket(os.path.join(G, "tiny_rep", "ema-bin-000.10x")))]
-    if os.path.exists(helpers.ref_bin("bwa")):
-        p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
-        cases.append((p["fasta"], helpers.read_bucket(p["bucket"])))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=emab.index_build)
+    cases.append((p["fasta"], helpers.read_bucket(p["bucket"])))
     for pre, lines in cases:
         ix = emab.Index(pre)
         monkeypatch.setenv("EMAB_RESCUE_PLAN", "0")
@@ -189,9 +192,8 @@ def test_wave_plans_are_transparent(emab, monkeypatch):
     DP cells the reference's loops visit — on the golden bucket and on the repeat/indel variant of BASELINE configs[0]."""
     from tools import synth
     cases = [(os.path.join(G, "tiny_rep", "ref.fa"), helpers.read_bucket(os.path.join(G, "tiny_rep", "ema-bin-000.10x")))]
-    if os.path.exists(helpers.ref_bin("bwa")):
-        p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
-        cases.append((p["fasta"], helpers.read_bucket(p["bucket"])))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=emab.index_build)
+    cases.append((p["fasta"], helpers.read_bucket(p["bucket"])))
     for pre, lines in cases:
         ix = emab.Index(pre)
         monkeypatch.setenv("EMAB_EXT_PLAN", "0")

@@ -8,36 +8,32 @@ import subprocess
 import pytest
 
 import helpers
-from test_gpu_sam import CLI, diff_msg, split_sam
+from test_gpu_sam import CLI
 
 pytestmark = pytest.mark.gpu
 
 
 def _data(cfg, platform):
+    import ema_b200
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("ema")):
-        pytest.skip("oracle/_ref/ema missing")
-    return synth.build_config(cfg, helpers.DATA_ROOT, helpers.ref_bin("bwa"), platform=platform)
+    return synth.build_config(cfg, helpers.DATA_ROOT, indexer=ema_b200.index_build, platform=platform)
 
 
-def _run_both(p, platform, in_flag, tmp_path, extra=(), env=None, threads="6"):
-    ref_sam, our_sam = tmp_path / "ref.sam", tmp_path / "ours.sam"
+def _run_both(p, platform, in_flag, tmp_path, key, extra=(), env=None, threads="6"):
+    our_sam = tmp_path / "ours.sam"
     common = ["align", in_flag, p["bucket"], "-r", p["fasta"], "-p", platform] + list(extra)
-    subprocess.run([helpers.ref_bin("ema")] + common + ["-t", "1", "-o", str(ref_sam)], check=True, stderr=subprocess.DEVNULL, env=env)
     subprocess.run([CLI] + common + ["-t", threads, "-o", str(our_sam)], check=True, env=env)
-    h1, b1 = split_sam(our_sam.read_bytes())
-    h2, b2 = split_sam(ref_sam.read_bytes())
-    assert h1 == h2
-    assert len(b2) > 500
-    assert b1 == b2, diff_msg(b1, b2)
-    return b1
+    return helpers.compare_sam_with_reference(
+        key, our_sam.read_bytes(),
+        lambda out: subprocess.run([helpers.ref_bin("ema")] + common + ["-t", "1", "-o", out], check=True, stderr=subprocess.DEVNULL, env=env),
+        tmp_path, min_records=501)
 
 
 @pytest.mark.parametrize("platform,in_flag", [("haplotag", "-s"), ("dbs", "-s"), ("tru", "-1"), ("tellseq", "-1"), ("cpt", "-1")])
 def test_platform_sweep(platform, in_flag, tmp_path):
     cfg = "c1_rep"
     p = _data(cfg, platform)
-    body = _run_both(p, platform, in_flag, tmp_path)
+    body = _run_both(p, platform, in_flag, tmp_path, f"platform_{platform}{in_flag}")
     assert any(b"\tBX:Z:" in l for l in body[:50])
 
 
@@ -48,10 +44,8 @@ def test_platform_sweep_100mbp(platform, in_flag, tmp_path):
     (tests/test_index_build.py pins its files to `bwa index`'s); both programs load it."""
     from tools import synth
     import ema_b200
-    if not os.path.exists(helpers.ref_bin("ema")):
-        pytest.skip("oracle/_ref/ema missing")
     p = synth.build_config("c2", helpers.DATA_ROOT, None, platform=platform, indexer=ema_b200.index_build, n_barcodes=20, tag="_sweep")
-    body = _run_both(p, platform, in_flag, tmp_path)
+    body = _run_both(p, platform, in_flag, tmp_path, f"platform_100mbp_{platform}{in_flag}")
     assert len(body) == 2 * 20 * 200
 
 
@@ -66,13 +60,13 @@ def test_10x_interleaved_fastq(tmp_path):
     synth.write_interleaved_fastq(str(fq), sim, platform="10x")
     q = dict(p)
     q["bucket"] = str(fq)
-    _run_both(q, "10x", "-1", tmp_path)
+    _run_both(q, "10x", "-1", tmp_path, "10x_interleaved_fastq")
 
 
 def test_read_group_and_bx_index(tmp_path):
     """-R (read group header + RG tags) and -i (BX index suffix) reach the header and every record."""
     p = _data("tiny_rep", "10x")
-    body = _run_both(p, "10x", "-s", tmp_path, extra=["-R", "@RG\\tID:rg1\\tSM:sample", "-i", "7"])
+    body = _run_both(p, "10x", "-s", tmp_path, "read_group_and_bx_index", extra=["-R", "@RG\\tID:rg1\\tSM:sample", "-i", "7"])
     assert all(b"RG:Z:rg1" in l for l in body[:100])
 
 
@@ -92,9 +86,9 @@ def test_density_optimiser(platform, in_flag, cfg, tmp_path):
     p = _data(cfg, platform)
     env = _faketime_env(tmp_path)
     d_on = tmp_path / "on"; d_on.mkdir()
-    body_d = _run_both(p, platform, in_flag, d_on, extra=["-d"], env=env)
+    body_d = _run_both(p, platform, in_flag, d_on, f"density_{platform}{in_flag}_{cfg}_on", extra=["-d"], env=env)
     d_off = tmp_path / "off"; d_off.mkdir()
-    body = _run_both(p, platform, in_flag, d_off, env=env)
+    body = _run_both(p, platform, in_flag, d_off, f"density_{platform}{in_flag}_{cfg}_off", env=env)
     assert len(body) == len(body_d)
     if body == body_d:
         pytest.xfail("this data set has no bad cloud that -d re-decides: -d parity holds but the optimiser did not change the output")

@@ -8,24 +8,11 @@ import numpy as np
 import pytest
 
 import helpers
+from helpers import diff_msg, split_sam
 
 pytestmark = pytest.mark.gpu
 G = os.path.join(os.path.dirname(__file__), "golden")
 CLI = os.path.join(helpers.ROOT, "ema_b200", "ema-b200")
-
-
-def split_sam(text: bytes):
-    lines = text.split(b"\n")
-    head = [l for l in lines if l.startswith(b"@") and not l.startswith(b"@PG")]
-    body = [l for l in lines if l and not l.startswith(b"@")]
-    return head, body
-
-
-def diff_msg(a, b):
-    for i, (x, y) in enumerate(zip(a, b)):
-        if x != y:
-            return f"first difference at record {i}:\n ours: {x[:300]!r}\n ref:  {y[:300]!r}"
-    return f"record counts differ: {len(a)} vs {len(b)}"
 
 
 def test_cli_golden_tiny(tmp_path):
@@ -51,52 +38,58 @@ def test_cli_errors(tmp_path):
 def test_session_vs_reference_c1(cfg, tmp_path):
     """BASELINE config 1 (10k pairs, 200 barcodes, 5 Mbp) and its repeat/indel variant against the
     reference binary run on the same files."""
-    if not os.path.exists(helpers.ref_bin("ema")):
-        pytest.skip("oracle/_ref/ema missing")
     import ema_b200
     from tools import synth
-    p = synth.build_config(cfg, helpers.DATA_ROOT, helpers.ref_bin("bwa"))
-    ref_sam = tmp_path / "ref.sam"
-    subprocess.run([helpers.ref_bin("ema"), "align", "-s", p["bucket"], "-r", p["fasta"], "-p", "10x", "-t", "1", "-o", str(ref_sam)],
-                   check=True, stderr=subprocess.DEVNULL)
+    p = synth.build_config(cfg, helpers.DATA_ROOT, indexer=ema_b200.index_build)
     s = ema_b200.Session(p["fasta"], "10x", threads=8)
     body = s.align_bucket(open(p["bucket"], "rb").read())
-    _, b1 = split_sam(body)
-    h2, b2 = split_sam(ref_sam.read_bytes())
-    assert b1 == b2, diff_msg(b1, b2)
-    h1, _ = split_sam(s.header(["ema", "align"]))
-    assert h1 == h2
+    helpers.compare_sam_with_reference(
+        f"session_{cfg}", s.header(["ema", "align"]) + body,
+        lambda out: subprocess.run([helpers.ref_bin("ema"), "align", "-s", p["bucket"], "-r", p["fasta"], "-p", "10x", "-t", "1", "-o", out],
+                                   check=True, stderr=subprocess.DEVNULL), tmp_path, min_records=1)
     st = s.stats
     assert st.n_pairs == p["n_pairs"] and st.launches >= 8
 
 
 def test_em_posteriors_vs_reference(tmp_path):
     """EM posteriors at full precision (the SAM only carries %.5g): within 1e-6 relative of the
-    reference's, with identical chosen alignments (north_star tolerance)."""
-    if not helpers.have_ref():
-        pytest.skip("oracle/_ref missing")
+    reference's, with identical chosen alignments (north_star tolerance).  Without oracle/_ref the reference's posteriors
+    come from tests/golden/reference/em_posteriors_c1_rep.npz."""
     import ctypes as C
     import ema_b200
     from tools import synth
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
-    R = helpers.ref()
-    R.ref_ema_init.argtypes = [C.c_char_p, C.c_char_p]
-    assert R.ref_ema_init(p["fasta"].encode(), b"10x") == 0
-    dump = tmp_path / "gamma.tsv"
-    R.ref_ema_run_bucket.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_int, C.c_int]
-    assert R.ref_ema_run_bucket(p["bucket"].encode(), str(tmp_path / "r.sam").encode(), str(dump).encode(), 0, 1) == 0
-    want = {}
-    for ln in open(dump):
-        f = ln.rstrip("\n").split("\t")
-        chosen = f[-1].split(":")
-        want[(f[0], int(f[1]))] = (int(chosen[0]), int(chosen[1]), float(chosen[2]))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=ema_b200.index_build)
     s = ema_b200.Session(p["fasta"], "10x", threads=8)
     mine = tmp_path / "mine.tsv"
     s.dump_posteriors(str(mine))
     s.align_bucket(open(p["bucket"], "rb").read())
+    rows = [ln.rstrip("\n").split("\t") for ln in open(mine)]
+    want = {}
+    if helpers.have_ref():
+        R = helpers.ref()
+        R.ref_ema_init.argtypes = [C.c_char_p, C.c_char_p]
+        assert R.ref_ema_init(p["fasta"].encode(), b"10x") == 0
+        dump = tmp_path / "gamma.tsv"
+        R.ref_ema_run_bucket.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_int, C.c_int]
+        assert R.ref_ema_run_bucket(p["bucket"].encode(), str(tmp_path / "r.sam").encode(), str(dump).encode(), 0, 1) == 0
+        for ln in open(dump):
+            f = ln.rstrip("\n").split("\t")
+            chosen = f[-1].split(":")
+            want[(f[0], int(f[1]))] = (int(chosen[0]), int(chosen[1]), float(chosen[2]))
+    else:
+        name = "em_posteriors_c1_rep.npz"
+        path = os.path.join(helpers.RECORDED_DIR, name)
+        if not os.path.exists(path) and helpers.RECORD_TO:
+            os.makedirs(helpers.RECORD_TO, exist_ok=True)
+            path = os.path.join(helpers.RECORD_TO, name)
+            np.savez_compressed(path, ident=np.array([r[0] for r in rows], "S"), mate=np.array([int(r[1]) for r in rows], np.int8),
+                                chrom=np.array([int(r[2]) for r in rows], np.int32), pos=np.array([int(r[3]) for r in rows], np.int64),
+                                gamma=np.array([float(r[4]) for r in rows], np.float64))
+        g = np.load(path)
+        for i, m, c, q, y in zip(g["ident"], g["mate"], g["chrom"], g["pos"], g["gamma"]):
+            want[(i.decode(), int(m))] = (int(c), int(q), float(y))
     n, worst = 0, 0.0
-    for ln in open(mine):
-        ident, mate, chrom, pos, gamma = ln.rstrip("\n").split("\t")
+    for ident, mate, chrom, pos, gamma in rows:
         wc, wp, wg = want[(ident, int(mate))]
         assert (wc, wp) == (int(chrom), int(pos)), (ident, mate)
         rel = abs(float(gamma) - wg) / max(abs(wg), 1e-300)
@@ -111,9 +104,7 @@ def test_multi_bucket_pipeline_matches_serial(tmp_path):
     and the CLI's -x output equals the concatenation."""
     import ema_b200
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("bwa")):
-        pytest.skip("oracle/_ref/bwa missing")
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=ema_b200.index_build)
     lines = open(p["bucket"], "rb").read().split(b"\n")
     lines = [l for l in lines if l]
     parts = [b"\n".join(lines[i::4]) + b"\n" for i in range(4)] + [b""]
@@ -149,9 +140,7 @@ def test_multi_device_session_matches_serial(tmp_path):
     import torch
     import ema_b200
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("bwa")):
-        pytest.skip("oracle/_ref/bwa missing")
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=ema_b200.index_build)
     lines = [l for l in open(p["bucket"], "rb").read().split(b"\n") if l]
     parts = [b"\n".join(lines[i::6]) + b"\n" for i in range(6)]
     s1 = ema_b200.Session(p["fasta"], "10x", threads=8)
@@ -182,9 +171,7 @@ def test_single_bucket_split_over_replicas():
     import torch
     import ema_b200
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("bwa")):
-        pytest.skip("oracle/_ref/bwa missing")
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=ema_b200.index_build)
     data = open(p["bucket"], "rb").read()
     serial = ema_b200.Session(p["fasta"], "10x", threads=8).align_bucket(data)
     s2 = ema_b200.Session(p["fasta"], "10x", threads=8)
@@ -197,34 +184,40 @@ def test_single_bucket_split_over_replicas():
 
 def test_raw_fastq_through_count_preproc_align(tmp_path):
     """From RAW 10x reads: `count` -> `preproc` -> `align` with this build against the same three steps of the reference —
-    identical bucket files (host/preproc.cpp), identical SAM (the buckets carry corrected barcodes, trimmed read 1)."""
+    identical bucket files (host/preproc.cpp), identical SAM (the buckets carry corrected barcodes, trimmed read 1).
+    Without oracle/_ref the reference's bucket files and SAM are represented by their recorded digests."""
     import filecmp
+    import ema_b200
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("bwa")):
-        pytest.skip("oracle/_ref/bwa missing")
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=ema_b200.index_build)
     n_contigs, clen, rseed, dup, nbc, ppb, indel = synth.CONFIGS["c1_rep"]
     contigs = synth.make_reference(n_contigs, clen, rseed, dup)
     sim = synth.simulate_pairs(contigs, 40, 60, rseed + 4242, indel=indel)
     fq, wl = str(tmp_path / "raw.fq"), str(tmp_path / "wl.txt")
     synth.write_raw_10x_fastq(fq, wl, sim)
+    have_ref = os.path.exists(helpers.ref_bin("ema"))
     outs = {}
-    for tag, exe in (("ref", helpers.ref_bin("ema")), ("our", CLI)):
+    for tag, exe in ((("ref", helpers.ref_bin("ema")),) if have_ref else ()) + (("our", CLI),):
         with open(fq, "rb") as f:
             subprocess.run([exe, "count", "-w", wl, "-o", str(tmp_path / tag)], stdin=f, check=True, stderr=subprocess.DEVNULL)
         with open(fq, "rb") as f:
             subprocess.run([exe, "preproc", "-w", wl, "-n", "3", "-t", "2", "-o", str(tmp_path / (tag + "_b")), str(tmp_path / tag) + ".ema-ncnt"],
                            stdin=f, check=True, stderr=subprocess.DEVNULL)
         outs[tag] = tmp_path / (tag + "_b")
-    names = sorted(os.listdir(outs["ref"]))
-    assert names == sorted(os.listdir(outs["our"])) == ["ema-bin-000", "ema-bin-001", "ema-bin-002", "ema-nobc"]
-    for n in names:
-        assert filecmp.cmp(outs["ref"] / n, outs["our"] / n, shallow=False), n
+    names = sorted(os.listdir(outs["our"]))
+    assert names == ["ema-bin-000", "ema-bin-001", "ema-bin-002", "ema-nobc"]
+    if have_ref:
+        assert names == sorted(os.listdir(outs["ref"]))
+        for n in names:
+            assert filecmp.cmp(outs["ref"] / n, outs["our"] / n, shallow=False), n
+    else:
+        for n in names:
+            d = helpers.sha((outs["our"] / n).read_bytes())
+            assert d == helpers.recorded_reference(f"raw_fastq_preproc_{n}", d), n
     bucket = str(outs["our"] / "ema-bin-001")
-    ref_sam, our_sam = tmp_path / "ref.sam", tmp_path / "our.sam"
-    subprocess.run([helpers.ref_bin("ema"), "align", "-s", bucket, "-r", p["fasta"], "-p", "10x", "-t", "1", "-o", str(ref_sam)], check=True, stderr=subprocess.DEVNULL)
+    our_sam = tmp_path / "our.sam"
     subprocess.run([CLI, "align", "-s", bucket, "-r", p["fasta"], "-p", "10x", "-t", "8", "-o", str(our_sam)], check=True, stderr=subprocess.DEVNULL)
-    _, b1 = split_sam(ref_sam.read_bytes())
-    _, b2 = split_sam(our_sam.read_bytes())
-    assert b1 == b2, diff_msg(b1, b2)
-    assert len(b1) > 1000
+    helpers.compare_sam_with_reference(
+        "raw_fastq_align", our_sam.read_bytes(),
+        lambda out: subprocess.run([helpers.ref_bin("ema"), "align", "-s", bucket, "-r", p["fasta"], "-p", "10x", "-t", "1", "-o", out],
+                                   check=True, stderr=subprocess.DEVNULL), tmp_path, min_records=1001)

@@ -138,11 +138,14 @@ def test_seeding_hot_equals_exact(hs, K):
     assert n_sec > 0
 
 
+@pytest.mark.gpu
 def test_seeding_hot_equals_exact_c1_rep(hs):
     """the same on the 5 Mbp reference with planted repeats and indel-bearing reads (BASELINE configs[0] variant), at
-    the index's own table depth: 1400 reads, and the traffic of the two forms side by side"""
+    the index's own table depth: 1400 reads, and the traffic of the two forms side by side.  The index is built by
+    emab_index_build (files byte-identical to `bwa index`'s: tests/test_index_build.py), hence the GPU mark."""
+    import ema_b200
     from tools import synth
-    p = synth.build_config("c1_rep", helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    p = synth.build_config("c1_rep", helpers.DATA_ROOT, indexer=ema_b200.index_build)
     hi = C.c_void_p(hs.hs_index_load(p["fasta"].encode()))
     assert hs.hs_kmer_k(hi) >= 8
     hs.hs_collect_intv_touches.restype = C.c_int64
@@ -160,13 +163,13 @@ def test_seeding_hot_equals_exact_c1_rep(hs):
     assert sectors * 32 < 0.6 * touches * 64, (sectors, touches)
 
 
+@pytest.mark.gpu
 def test_seeding_hot_staircase(hs, tmp_path):
     """forward sweeps whose interval size changes 46 times (a staircase of planted prefixes): long prev/curr lists, every
-    k-mer table level and several FM steps recorded, multi-step backward rounds — default form against the exact one"""
-    import subprocess
+    k-mer table level and several FM steps recorded, multi-step backward rounds — default form against the exact one
+    (index by emab_index_build, hence the GPU mark)"""
+    import ema_b200
     from tools import synth
-    if not os.path.exists(helpers.ref_bin("bwa")):
-        pytest.skip("oracle/_ref/bwa not built")
     rng = np.random.default_rng(123)
     contigs = synth.make_reference(1, 80_000, 7, 0)
     S = rng.integers(0, 4, 70, dtype=np.uint8)
@@ -179,7 +182,7 @@ def test_seeding_hot_staircase(hs, tmp_path):
             c[pos + k] = (S[k] + 1) & 3
     fa = str(tmp_path / "ref.fa")
     synth.write_fasta(fa, contigs)
-    subprocess.run([helpers.ref_bin("bwa"), "index", fa], check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    ema_b200.index_build(fa)
     hi = C.c_void_p(hs.hs_index_load(fa.encode()))
     n_long = 0
     for K in (-1, 0, 3):
@@ -249,26 +252,43 @@ def _chains(lib, fn, idx, s, *flt):
     return ch[:n], sd[:ns.value]
 
 
-@pytest.mark.parametrize("cfg,limit,device_like", [("tiny_rep", 480, 0), ("c1_rep", 700, 0), ("c1_rep", 400, 1)])
-def test_stages_vs_reference(hs, ref_lib, cfg, limit, device_like):
+@pytest.mark.parametrize("cfg,limit,device_like", [("tiny_rep", 480, 0), pytest.param("c1_rep", 700, 0, marks=pytest.mark.gpu),
+                                                    pytest.param("c1_rep", 400, 1, marks=pytest.mark.gpu)])
+def test_stages_vs_reference(hs, cfg, limit, device_like):
     """chains after mem_chain_flt, regions after mem_chain2aln, after mem_sort_dedup_patch, after
     mate rescue, and the final candidates: all bit-exact against the compiled reference.  device_like: with the data flow
     of the device pipeline's default forms — intervals of the seed_hot.cuh algorithm (x1 = 0) and the occurrences' SA
-    values gathered ahead of the chaining, as k_sa_gather hands them to k_chain."""
+    values gathered ahead of the chaining, as k_sa_gather hands them to k_chain.  Where oracle/_ref is not built, all of
+    it against the recorded digest of the reference's stage outputs on the same reads.  The c1_rep cases index their
+    5 Mbp reference with emab_index_build (hence the GPU mark); tiny_rep uses the committed index."""
     from tools import synth
     hs.hs_set_device_like(device_like)
-    p = synth.build_config(cfg, helpers.DATA_ROOT, helpers.ref_bin("bwa"))
+    if cfg == "tiny_rep":
+        p = {"fasta": os.path.join(G, "tiny_rep", "ref.fa"), "bucket": os.path.join(G, "tiny_rep", "ema-bin-000.10x")}
+    else:
+        import ema_b200
+        p = synth.build_config(cfg, helpers.DATA_ROOT, indexer=ema_b200.index_build)
     pre = p["fasta"].encode()
     hi = C.c_void_p(hs.hs_index_load(pre))
-    ri = C.c_void_p(ref_lib.ref_idx_load(pre))
+    ref_lib = helpers.ref() if helpers.have_ref() else None
+    ri = C.c_void_p(ref_lib.ref_idx_load(pre)) if ref_lib else None
+    parts = []
     rng = np.random.default_rng(5)
     for f in helpers.read_bucket(p["bucket"], limit):
         reads = [helpers.nt4(f[2]), helpers.nt4(f[4])]
         if rng.random() < 0.05:
             reads[0][rng.integers(0, len(reads[0]))] = 4
         for s in reads:
-            a, b = _chains(hs, "hs_chain", hi, s), _chains(ref_lib, "ref_chain", ri, s, 1)
-            assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), ("chain", f[1])
-            assert np.array_equal(_regs(hs, "hs_align1", hi, s, 0), _regs(ref_lib, "ref_chain2aln", ri, s)), ("chain2aln", f[1])
-            assert np.array_equal(_regs(hs, "hs_align1", hi, s, 1), _regs(ref_lib, "ref_align1", ri, s)), ("align1", f[1])
+            a = _chains(hs, "hs_chain", hi, s)
+            r0, r1 = _regs(hs, "hs_align1", hi, s, 0), _regs(hs, "hs_align1", hi, s, 1)
+            if ref_lib:
+                b = _chains(ref_lib, "ref_chain", ri, s, 1)
+                assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), ("chain", f[1])
+                assert np.array_equal(r0, _regs(ref_lib, "ref_chain2aln", ri, s)), ("chain2aln", f[1])
+                assert np.array_equal(r1, _regs(ref_lib, "ref_align1", ri, s)), ("align1", f[1])
+            else:
+                parts += [x.tobytes() + str(x.shape).encode() for x in (a[0], a[1], r0, r1)]
     hs.hs_set_device_like(0)
+    if not ref_lib:
+        d = helpers.sha(*parts)
+        assert d == helpers.recorded_reference(f"stages_{cfg}_{limit}", d)

@@ -57,19 +57,29 @@ def test_pack_matches_committed_index(tmp_path):
 
 @pytest.mark.parametrize("crlf", [False, True])
 def test_pack_matches_bwa_on_messy_fasta(tmp_path, crlf):
-    if not os.path.exists(BWA):
-        pytest.skip("oracle/_ref/bwa not built")
     fa = str(tmp_path / "m.fa")
     _messy_fasta(fa, crlf=crlf)
     ema_b200.index_pack_fasta(fa, str(tmp_path / "ours"))
-    subprocess.run([BWA, "fa2pac", "-f", fa, str(tmp_path / "theirs")], check=True, capture_output=True)
-    for e in (".pac", ".ann", ".amb"):
-        assert filecmp.cmp(str(tmp_path / "ours") + e, str(tmp_path / "theirs") + e, shallow=False), e
+    _same_as_bwa(f"fa2pac_messy_crlf{int(crlf)}", ["fa2pac", "-f", fa, str(tmp_path / "theirs")], str(tmp_path / "ours"),
+                 str(tmp_path / "theirs"), (".pac", ".ann", ".amb"))
 
 
 def _same_index(a, b):
     for e in EXTS:
         assert filecmp.cmp(a + e, b + e, shallow=False), "%s differs" % e
+
+
+def _same_as_bwa(key, bwa_args, ours, theirs, exts=EXTS):
+    """ours.<ext> against what `bwa <bwa_args>` writes to theirs.<ext>: the files themselves where oracle/_ref/bwa is built,
+    elsewhere the recorded digests of bwa's files for case `key`"""
+    if os.path.exists(BWA):
+        subprocess.run([BWA] + bwa_args, check=True, capture_output=True)
+        for e in exts:
+            assert filecmp.cmp(ours + e, theirs + e, shallow=False), "%s differs" % e
+        return
+    for e in exts:
+        d = helpers.sha(open(ours + e, "rb").read())
+        assert d == helpers.recorded_reference(key + e, d), "%s differs" % e
 
 
 @pytest.mark.gpu
@@ -86,8 +96,6 @@ def test_build_matches_committed_index(tmp_path, chunk_bits, monkeypatch):
 
 @pytest.mark.gpu
 def test_build_matches_bwa_messy_and_repeats(tmp_path):
-    if not os.path.exists(BWA):
-        pytest.skip("oracle/_ref/bwa not built")
     from tools import synth
     # (a) ambiguity codes etc.; (b) 5 Mbp with planted 2-10 kb repeats; (c) a text that is one long tandem repeat plus
     # a poly-A tail (deep ties, suffixes that run into the end of the text)
@@ -100,21 +108,17 @@ def test_build_matches_bwa_messy_and_repeats(tmp_path):
     unit = rng.integers(0, 4, 97, dtype=np.uint8)
     synth.write_fasta(fa_c, [np.concatenate([np.tile(unit, 400), rng.integers(0, 4, 1000, dtype=np.uint8), np.zeros(300, np.uint8)]),
                              np.concatenate([np.zeros(200, np.uint8), np.tile(unit, 50)])])
-    for fa in (fa_a, fa_b, fa_c):
+    for tag, fa in (("a", fa_a), ("b", fa_b), ("c", fa_c)):
         ema_b200.index_build(fa, fa + ".ours")
-        subprocess.run([BWA, "index", "-p", fa + ".theirs", fa], check=True, capture_output=True)
-        _same_index(fa + ".ours", fa + ".theirs")
+        _same_as_bwa(f"bwa_index_messy_and_repeats_{tag}", ["index", "-p", fa + ".theirs", fa], fa + ".ours", fa + ".theirs")
 
 
 @pytest.mark.gpu
 def test_build_matches_bwa_above_50mbp(tmp_path):
     """above 50 Mbp the reference switches from SA-IS to bwtsw (bwa/bwtindex.c:276); the files must still be identical"""
-    if not os.path.exists(BWA):
-        pytest.skip("oracle/_ref/bwa not built")
     from tools import synth
     fa = str(tmp_path / "big.fa")
     synth.write_fasta(fa, synth.make_reference(4, 13_000_000, 11, dup_every=200_000))
     st = ema_b200.index_build(fa, fa + ".ours")
-    subprocess.run([BWA, "index", "-p", fa + ".theirs", fa], check=True, capture_output=True)
-    _same_index(fa + ".ours", fa + ".theirs")
+    _same_as_bwa("bwa_index_above_50mbp", ["index", "-p", fa + ".theirs", fa], fa + ".ours", fa + ".theirs")
     assert st["l_pac"] == 52_000_000

@@ -1,7 +1,8 @@
 """CPU tests (-m "not gpu"): `ema-b200 count` / `preproc` (host/preproc.cpp) against the reference binary (oracle/_ref/ema) on a
 synthetic raw 10x FASTQ — whitelisted barcodes, one- and two-base errors with matching low qualities, N bases, barcodes not
 on the list, short reads, a quality character below '!'.  Every output file must be byte-identical: the census (.ema-ncnt in
-the reference's hash-map order, .ema-fcnt incl. block dumps), every ema-bin-NNN and ema-nobc, with and without -h / -b."""
+the reference's hash-map order, .ema-fcnt incl. block dumps), every ema-bin-NNN and ema-nobc, with and without -h / -b.
+Where oracle/_ref is not built, the reference's files are represented by their recorded digests (tests/golden/reference)."""
 import filecmp
 import os
 import subprocess
@@ -13,6 +14,7 @@ import helpers
 
 CLI = os.path.join(helpers.ROOT, "ema_b200", "ema-b200")
 REF = helpers.ref_bin("ema")
+HAVE_REF = os.path.exists(REF)
 ACGT = np.frombuffer(b"ACGT", dtype=np.uint8)
 
 
@@ -71,8 +73,6 @@ def run(cmd, stdin_path, cwd=None):
 
 @pytest.fixture(scope="module")
 def raw(tmp_path_factory):
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/ema not built")
     if not os.path.exists(CLI):
         subprocess.run(["make", "-s", "-C", os.path.join(helpers.ROOT, "ema_b200", "csrc")], check=True)
     d = tmp_path_factory.mktemp("raw")
@@ -81,32 +81,54 @@ def raw(tmp_path_factory):
     return d, fq, wl
 
 
-def same_dir(a, b):
-    names = sorted(os.listdir(a))
-    assert names == sorted(os.listdir(b)) and names
+def same_as_reference(key, ours, ref=None):
+    """this build's files {name: path} against the reference's files of the same names ({name: path}, where it ran) or,
+    without oracle/_ref, against the recorded digests of the reference's files for case `key`"""
+    assert ours
+    if HAVE_REF:
+        assert sorted(ref) == sorted(ours)
+        for n in ours:
+            assert filecmp.cmp(ref[n], ours[n], shallow=False), n
+        return sorted(ours)
+    names = sorted(ours)
+    assert names == helpers.recorded_reference(f"{key}/names", names)
     for n in names:
-        assert filecmp.cmp(os.path.join(a, n), os.path.join(b, n), shallow=False), n
+        d = helpers.sha(open(ours[n], "rb").read())
+        assert d == helpers.recorded_reference(f"{key}/{n}", d), n
     return names
+
+
+def files(d):
+    return {n: os.path.join(d, n) for n in os.listdir(d)}
+
+
+def programs():
+    """(tag, executable) of the runs to compare: the reference's where it is built, then this build's"""
+    return ((("ref", REF),) if HAVE_REF else ()) + (("our", CLI),)
 
 
 def test_count_files_identical(raw):
     d, fq, wl = raw
-    run([REF, "count", "-w", wl, "-o", str(d / "ref")], fq)
-    run([CLI, "count", "-w", wl, "-o", str(d / "our")], fq)
-    for ext in (".ema-ncnt", ".ema-fcnt"):
-        assert filecmp.cmp(str(d / "ref") + ext, str(d / "our") + ext, shallow=False), ext
+    for tag, exe in programs():
+        run([exe, "count", "-w", wl, "-o", str(d / tag)], fq)
+    exts = (".ema-ncnt", ".ema-fcnt")
+    same_as_reference("count", {e: str(d / "our") + e for e in exts}, {e: str(d / "ref") + e for e in exts})
     assert os.path.getsize(str(d / "our") + ".ema-ncnt") > 8 + 12 * 30
 
 
 @pytest.mark.parametrize("flags", [[], ["-h"], ["-b"], ["-h", "-t", "3", "-n", "5"]])
 def test_preproc_buckets_identical(raw, flags, tmp_path):
     d, fq, wl = raw
-    if not os.path.exists(str(d / "ref.ema-ncnt")):
-        run([REF, "count", "-w", wl, "-o", str(d / "ref")], fq)
+    # the census both programs correct with: the reference's (this build's where the reference is not built; the two are
+    # byte-identical, test_count_files_identical)
+    census = str(d / ("ref" if HAVE_REF else "our"))
+    if not os.path.exists(census + ".ema-ncnt"):
+        run([REF if HAVE_REF else CLI, "count", "-w", wl, "-o", census], fq)
     n = ["-n", "7"] if "-n" not in flags else []
-    run([REF, "preproc", "-w", wl, "-o", str(tmp_path / "ref_out")] + n + flags + [str(d / "ref.ema-ncnt")], fq)
-    run([CLI, "preproc", "-w", wl, "-o", str(tmp_path / "our_out")] + n + flags + [str(d / "ref.ema-ncnt")], fq)
-    names = same_dir(str(tmp_path / "ref_out"), str(tmp_path / "our_out"))
+    for tag, exe in programs():
+        run([exe, "preproc", "-w", wl, "-o", str(tmp_path / (tag + "_out"))] + n + flags + [census + ".ema-ncnt"], fq)
+    names = same_as_reference("preproc" + "".join(flags), files(str(tmp_path / "our_out")),
+                              files(str(tmp_path / "ref_out")) if HAVE_REF else None)
     assert "ema-nobc" in names and "ema-bin-000" in names
     assert sum(os.path.getsize(str(tmp_path / "our_out" / x)) for x in names if x.startswith("ema-bin")) > 500_000
 
@@ -133,10 +155,14 @@ def test_count_block_dumps(raw):
         total += sum(int.from_bytes(data[pos + 24 * i + 16:pos + 24 * i + 24], "little") for i in range(n))
         pos += 24 * n; blocks += 1
     assert blocks >= 3 and pos == len(data)
-    ref = open(str(d / "ref.ema-fcnt"), "rb").read() if os.path.exists(str(d / "ref.ema-fcnt")) else None
-    if ref:
-        n = int.from_bytes(ref[:8], "little")
-        assert total == sum(int.from_bytes(ref[8 + 24 * i + 16:8 + 24 * i + 24], "little") for i in range(n))
+    # the one-block census of the same reads: the reference's, or where it is not built this build's (byte-identical to
+    # the reference's, test_count_files_identical)
+    tag, exe = programs()[0]
+    if not os.path.exists(str(d / tag) + ".ema-fcnt"):
+        run([exe, "count", "-w", wl, "-o", str(d / tag)], fq)
+    ref = open(str(d / tag) + ".ema-fcnt", "rb").read()
+    n = int.from_bytes(ref[:8], "little")
+    assert total == sum(int.from_bytes(ref[8 + 24 * i + 16:8 + 24 * i + 24], "little") for i in range(n))
 
 
 @pytest.mark.parametrize("case", ["empty", "no_final_newline", "one_pair"])
@@ -148,12 +174,12 @@ def test_preproc_edge_inputs(raw, case, tmp_path):
     small = {"empty": b"", "no_final_newline": b"\n".join(lines[:8 * 50]), "one_pair": b"\n".join(lines[:8]) + b"\n"}[case]
     sfq = str(tmp_path / "s.fq")
     open(sfq, "wb").write(small)
-    for tag, exe in (("ref", REF), ("our", CLI)):
+    for tag, exe in programs():
         run([exe, "count", "-w", wl, "-o", str(tmp_path / tag)], sfq)
         run([exe, "preproc", "-w", wl, "-n", "4", "-o", str(tmp_path / (tag + "_out")), str(tmp_path / tag) + ".ema-ncnt"], sfq)
-    for ext in (".ema-ncnt", ".ema-fcnt"):
-        assert filecmp.cmp(str(tmp_path / "ref") + ext, str(tmp_path / "our") + ext, shallow=False), ext
-    same_dir(str(tmp_path / "ref_out"), str(tmp_path / "our_out"))
+    exts = (".ema-ncnt", ".ema-fcnt")
+    same_as_reference(f"edge_{case}_count", {e: str(tmp_path / "our") + e for e in exts}, {e: str(tmp_path / "ref") + e for e in exts})
+    same_as_reference(f"edge_{case}_preproc", files(str(tmp_path / "our_out")), files(str(tmp_path / "ref_out")) if HAVE_REF else None)
 
 
 def test_preproc_several_count_files(raw, tmp_path):
@@ -164,11 +190,11 @@ def test_preproc_several_count_files(raw, tmp_path):
     parts = [b"\n".join(lines[:half]) + b"\n", b"\n".join(lines[half:])]
     for i, p in enumerate(parts):
         open(str(tmp_path / f"p{i}.fq"), "wb").write(p)
-    for tag, exe in (("ref", REF), ("our", CLI)):
+    for tag, exe in programs():
         for i in range(2):
             run([exe, "count", "-w", wl, "-o", str(tmp_path / f"{tag}{i}")], str(tmp_path / f"p{i}.fq"))
         run([exe, "preproc", "-w", wl, "-n", "6", "-t", "2", "-o", str(tmp_path / (tag + "_out")), str(tmp_path / f"{tag}0.ema-ncnt"), str(tmp_path / f"{tag}1.ema-ncnt")], fq)
-    same_dir(str(tmp_path / "ref_out"), str(tmp_path / "our_out"))
+    same_as_reference("several_count_files", files(str(tmp_path / "our_out")), files(str(tmp_path / "ref_out")) if HAVE_REF else None)
 
 
 def make_haplotag_fastq(path, n_pairs=3000, seed=3):
@@ -198,14 +224,13 @@ def make_haplotag_fastq(path, n_pairs=3000, seed=3):
 def test_haplotag_count_and_preproc(flags, tmp_path):
     """-p: barcodes from the BX:Z: tag of the name line, all 96^4 combinations known, no correction, reads untrimmed — and
     the reference's quirks (the first pair is never bucketed, the tag is bounded by the previous pair's last line)"""
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/ema not built")
     fq = str(tmp_path / "h.fq")
     make_haplotag_fastq(fq)
-    for tag, exe in (("ref", REF), ("our", CLI)):
+    for tag, exe in programs():
         run([exe, "count", "-p", "-o", str(tmp_path / tag)], fq)
         run([exe, "preproc", "-p", "-n", "5", "-o", str(tmp_path / (tag + "_out"))] + flags + [str(tmp_path / tag) + ".ema-ncnt"], fq)
-    assert filecmp.cmp(str(tmp_path / "ref.ema-ncnt"), str(tmp_path / "our.ema-ncnt"), shallow=False)
+    key = "haplotag" + "".join(flags)
+    same_as_reference(key + "_count", {"ncnt": str(tmp_path / "our.ema-ncnt")}, {"ncnt": str(tmp_path / "ref.ema-ncnt")})
     assert not os.path.exists(str(tmp_path / "our.ema-fcnt")) and not os.path.exists(str(tmp_path / "ref.ema-fcnt"))
-    names = same_dir(str(tmp_path / "ref_out"), str(tmp_path / "our_out"))
+    names = same_as_reference(key + "_preproc", files(str(tmp_path / "our_out")), files(str(tmp_path / "ref_out")) if HAVE_REF else None)
     assert sum(os.path.getsize(str(tmp_path / "our_out" / x)) for x in names if x.startswith("ema-bin")) > 300_000
