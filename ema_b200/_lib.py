@@ -296,6 +296,22 @@ def align_pairs(ctx: Context, reads, stage=3, want_regs=False):
     return dict(n_regs=n_regs, alns=alns, regs=regs, stats=st)
 
 
+def bgzf_eof() -> bytes:
+    """The 28-byte empty BGZF member that ends a BAM file (emab_bgzf_eof)."""
+    p, n = C.c_void_p(), C.c_uint64()
+    _check(lib().emab_bgzf_eof(C.byref(p), C.byref(n)))
+    return C.string_at(p, n.value)
+
+
+def bgzf_compress(ctx: Context, data: bytes) -> bytes:
+    """emab_bgzf_compress: BGZF members of `data` (one per 65 280-byte chunk), compressed on the device."""
+    cap = len(data) + (len(data) // 65280 + 1) * 64
+    out = C.create_string_buffer(cap)
+    n = C.c_uint64()
+    _check(lib().emab_bgzf_compress(ctx._h, data, C.c_uint64(len(data)), out, C.c_uint64(cap), C.byref(n)))
+    return out.raw[:n.value]
+
+
 class RunStats(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("parse_ms", "encode_ms", "align_ms", "kernel_ms", "cloud_ms", "flatten_ms", "em_ms",
                                           "em_kernel_ms", "format_ms", "total_ms", "ms_seed", "ms_chain", "ms_align1", "ms_rescue",
@@ -341,12 +357,23 @@ class Session:
     """The operator the reference's main() calls (find_clouds_and_align and friends) on one GPU:
     emab_session_open / emab_sam_header / emab_align_bucket / emab_align_fastq."""
 
+    OUTPUTS = {"sam": 0, "bam": 1}
+
     def __init__(self, ref_path: str, platform: str = "10x", device: int = 0, rg: str | None = None, bx_index: str | None = None,
-                 apply_opt: bool = False, threads: int = 1):
+                 apply_opt: bool = False, threads: int = 1, output: str = "sam"):
+        """output="bam": header() and every align call return BGZF members of BAM instead of SAM text
+        (a BAM file is header, the calls' bytes in order, then bgzf_eof())."""
         self._h = C.c_void_p()
         _check(lib().emab_session_open(ref_path.encode(), platform.encode(), device, C.byref(self._h)))
         _check(lib().emab_session_config(self._h, rg.encode() if rg else None, bx_index.encode() if bx_index else None,
                                          int(apply_opt), threads))
+        self.set_output(output)
+
+    def set_output(self, output: str):
+        """emab_session_output: "sam" or "bam" for the calls that follow"""
+        if output not in self.OUTPUTS:
+            raise ValueError(f"unknown output format {output!r} (sam or bam)")
+        _check(lib().emab_session_output(self._h, self.OUTPUTS[output]))
 
     def header(self, argv) -> bytes:
         arr = (C.c_char_p * len(argv))(*[a.encode() for a in argv])

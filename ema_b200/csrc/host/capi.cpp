@@ -83,7 +83,28 @@ int emab_sam_header(emab_session_t *h, int argc, const char *const *argv, char *
 		if (!h) return fail(EMAB_ERR_ARG, "null session");
 		std::string o;
 		emab::sam_header(h->s, argc, argv, &o);
-		return give(o, text, len);
+		if (h->s->output != EMAB_OUTPUT_BAM) return give(o, text, len);
+		std::string raw;
+		emab::bam_header(h->s, o, &raw);
+		const uint64_t cap = raw.size() + (raw.size() / 65280 + 1) * 64;
+		char *p = emab::text_alloc(cap + 1);
+		if (!p) return fail(EMAB_ERR_NOMEM, "out of memory");
+		uint64_t n = 0;
+		int rc = emab_bgzf_compress(h->s->workers[0].ctx, (const uint8_t *)raw.data(), raw.size(), (uint8_t *)p, cap, &n);
+		if (rc) { emab::text_free(p); return rc; }
+		p[n] = 0;
+		*text = p; *len = n;
+		return EMAB_OK;
+	});
+}
+
+int emab_session_output(emab_session_t *h, int format)
+{
+	return guarded([&]() -> int {
+		if (!h) return fail(EMAB_ERR_ARG, "null session");
+		int rc = emab::session_output(h->s, format);
+		if (rc) return fail(rc, h->s->err);
+		return EMAB_OK;
 	});
 }
 

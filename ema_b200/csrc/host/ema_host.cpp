@@ -347,6 +347,36 @@ void sam_header(const Session *s, int argc, const char *const *argv, std::string
 	out->push_back('\n');
 }
 
+void bam_header(const Session *s, const std::string &text, std::string *out)
+{
+	auto u32 = [&](uint32_t v) { for (int k = 0; k < 4; ++k) out->push_back((char)(v >> 8 * k)); };
+	out->append("BAM\1", 4);
+	u32((uint32_t)text.size());
+	out->append(text);
+	u32((uint32_t)s->sq_names.size());
+	for (size_t i = 0; i < s->sq_names.size(); ++i) {
+		u32((uint32_t)s->sq_names[i].size() + 1);
+		out->append(s->sq_names[i]);
+		out->push_back(0);
+		u32((uint32_t)s->sq_len[i]);
+	}
+}
+
+int session_output(Session *s, int format)
+{
+	if (format != EMAB_OUTPUT_SAM && format != EMAB_OUTPUT_BAM) { s->err = "error: unknown output format " + std::to_string(format); return EMAB_ERR_ARG; }
+	if (format == EMAB_OUTPUT_BAM)   // a BAM refID names an @SQ entry: every contig must print as the name of one
+		for (size_t r = 0; r < s->rid2chrom.size(); ++r) {
+			const std::string &nm = s->fai_names[(size_t)s->rid2chrom[r]];
+			if (std::find(s->sq_names.begin(), s->sq_names.end(), nm) == s->sq_names.end()) {
+				s->err = "error: contig " + s->sq_names[r] + " prints as '" + nm + "', which no @SQ entry has: BAM output cannot refer to it";
+				return EMAB_ERR_ARG;
+			}
+		}
+	s->output = format;
+	return EMAB_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 // records
 // ---------------------------------------------------------------------------------------------
@@ -1178,6 +1208,11 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 	for (const std::string &nm : s->fai_names) max_name = std::max(max_name, nm.size());
 	size_t cap = (size_t)n_out * (3 * max_name + s->bx_index.size() + s->rg_id.size() + 2 * 64 * 5 + 256) + 64;
 	for (size_t v : bound_part) cap += v;
+	const bool bam = s->output == EMAB_OUTPUT_BAM;
+	if (bam) {   // raw records fit the text bound plus 64 bytes each; BGZF adds at most a stored block's 31 bytes per 65 280
+		const size_t raw = cap + (size_t)n_out * 64;
+		cap = raw + (raw / 65280 + 1) * 64;
+	}
 	char *buf = text_alloc_pinned(cap + 1);
 	if (!buf) { wk.err = "out of memory"; return EMAB_ERR_NOMEM; }
 	uint64_t total = 0;
@@ -1186,9 +1221,9 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 		memset(&job, 0, sizeof job);
 		job.n_recs = (int32_t)n_out; job.n_bc = nb; job.recs = descs.data(); job.bc_off = bc_off.data(); job.bc_text = bc_text.data();
 		job.bx_index = s->bx_index.c_str(); job.rg_id = s->has_rg ? s->rg_id.c_str() : nullptr; job.is_haplotag = s->is_haplotag ? 1 : 0;
-		int rc = emab_sam_format(wk.ctx, &job, buf, (uint64_t)cap, &total);
+		int rc = bam ? emab_bam_format(wk.ctx, &job, buf, (uint64_t)cap, &total) : emab_sam_format(wk.ctx, &job, buf, (uint64_t)cap, &total);
 		if (rc) { wk.err = emab_last_error(); text_free(buf); return rc; }
-		st.launches += 4;
+		st.launches += emab_last_launches(wk.ctx);
 		st.d2h_bytes += (int64_t)total;
 		st.h2d_bytes += (int64_t)n_out * (int64_t)sizeof(emab_sam_rec_t) + (int64_t)bc_text.size();
 		st.format_kernel_ms = emab_last_kernel_ms(wk.ctx);

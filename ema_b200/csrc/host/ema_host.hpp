@@ -149,6 +149,7 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 		cv.wait(g, [&] { return cloud_turn >= ticket; });
 		if (cloud_turn == ticket) { ++cloud_turn; cv.notify_all(); }
 	}
+	int output = EMAB_OUTPUT_SAM;         // what the align calls return: SAM text or BGZF members of BAM records
 	std::string err;
 	std::string gamma_dump;               // test hook: path for full-precision posteriors of the chosen alignments
 	emab_run_stats_t last{};
@@ -186,6 +187,9 @@ void text_free(void *p);
 int session_open(const char *ref_path, const char *platform, int device, Session **out, std::string *err);
 void session_close(Session *s);
 void sam_header(const Session *s, int argc, const char *const *argv, std::string *out);
+// the uncompressed BAM header (SAM spec v1 §4.2): magic, the header text, the @SQ names and lengths
+void bam_header(const Session *s, const std::string &text, std::string *out);
+int session_output(Session *s, int format);   // EMAB_OUTPUT_SAM / EMAB_OUTPUT_BAM
 int session_set_workers(Session *s, int n_workers);
 int session_add_device(Session *s, int device);  // before session_set_workers
 // find_clouds_and_align (src/align.c:214) over the *contents* of the input file(s); SAM text in a malloc'ed buffer

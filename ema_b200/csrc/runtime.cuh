@@ -76,7 +76,7 @@ struct emab_ctx {
 	int spin_us = 150;               // how long mode 0 polls before it starts sleeping (EMAB_SPIN_US)
 	double last_ms = 0;
 	int last_launches = 0;
-	DevBuf b[48];            // device scratch slots, meaning assigned by each entry point
+	DevBuf b[52];            // device scratch slots, meaning assigned by each entry point
 	HostBuf h[8];            // pinned host result buffers, owned by the ctx and valid until its next call
 	unsigned long long *d_counters = nullptr;  // 16 x u64 instrumentation / work counters
 	int n_sm = 148;
@@ -95,8 +95,13 @@ struct emab_ctx {
 	unsigned text_len = 0;
 	int text_pairs = 0;
 	bool sam_tables_ready = false;  // contig names + rid -> name map resident (slot 45: emab_sam_tables)
-	size_t sam_chrom_off = 0, sam_rid_off = 0;
+	size_t sam_chrom_off = 0, sam_rid_off = 0, sam_sq_off = 0;
+	std::string bam_unmapped_contig; // a contig of the index whose .fai name no @SQ entry has (BAM refuses then); empty: none
 };
+
+// BGZF members of d_in[0..n) (device memory) into the host buffer out (bgzf.cu); records ev1 after the last kernel.
+// Slots 48-51.  *launches = kernels launched.
+int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches);
 
 // first statement of every entry point that takes a ctx: a worker thread of the host pipeline (or any caller's
 // thread) starts on device 0, and a stream or buffer of another device is an invalid argument there

@@ -242,6 +242,20 @@ int emab_parse_bucket(emab_ctx_t *ctx, const char *text, uint64_t text_len, int 
 int emab_align_pairs_resident(emab_ctx_t *ctx, int n_pairs, const int64_t *off, emab_pairs_result_t *result, emab_stats_t *stats);
 int emab_sam_tables(emab_ctx_t *ctx, int n_chrom, const char *const *names, int n_rid, const int32_t *rid2chrom);
 int emab_sam_format(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len);
+/* emab_bam_format = the same records as BAM (SAM spec v1 §4.2), compressed on the device into BGZF members; only the members
+ *                    are copied to `out`.  Decoded the way `samtools view` prints them they are emab_sam_format's lines.
+ *                    refID / next_refID: the first @SQ entry (contig of the index) with the .fai name the SAM line prints.
+ *                    Fails with EMAB_ERR_ARG where BAM cannot hold the record: a read name longer than 254 bytes, a quality
+ *                    string whose length differs from its read's, a quality byte outside '!'..'~'; and when a contig's
+ *                    .fai name has no @SQ entry.
+ * emab_bgzf_compress = the device compressor on its own: in[0..len) cut at multiples of 65 280 bytes, one BGZF member per
+ *                    chunk (gzip header with the BC field, one raw DEFLATE block — LZ77 in the 32 KB window with dynamic
+ *                    Huffman codes, or stored when that is smaller — CRC-32, ISIZE), packed into `out`.  The encoder is
+ *                    deterministic: csrc/bgzf.cuh compiled for the host makes the same bytes.
+ * emab_bgzf_eof     = the 28-byte empty member that ends a BGZF file (static storage; needs no GPU). */
+int emab_bam_format(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len);
+int emab_bgzf_compress(emab_ctx_t *ctx, const uint8_t *in, uint64_t len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+int emab_bgzf_eof(const uint8_t **p, uint64_t *len);
 /* pinned host memory for callers that want their input buffers to take the fast H2D path */
 void *emab_pinned_alloc(uint64_t bytes);
 void emab_pinned_free(void *p);
@@ -286,7 +300,16 @@ int emab_em_batch(emab_ctx_t *ctx, const emab_em_problem_t *problem, double *gam
  *                          barcode-sorted FASTQ(s); d2 == NULL means interleaved (-1 only)
  * SAM text is returned in a malloc'ed buffer the caller releases with emab_free().  Output is in
  * barcode order — byte-identical to the reference run with -t 1 (MI cloud ids included; they
- * continue across calls on one session like the reference's process-wide counter). */
+ * continue across calls on one session like the reference's process-wide counter).
+ *   emab_session_output  = EMAB_OUTPUT_SAM (default) or EMAB_OUTPUT_BAM.  In BAM mode emab_sam_header returns BGZF members
+ *                          holding the BAM header (magic, the same header text, the @SQ names and lengths), and every align
+ *                          call returns (or passes to its write callback) whole BGZF members of its records instead of SAM
+ *                          text: blocks never span calls.  A BAM file is the header's bytes, every call's bytes in order,
+ *                          then emab_bgzf_eof's block.  Fails when a contig's .fai name has no @SQ entry.  In BAM mode
+ *                          emab_run_stats_t.sam_bytes counts the compressed bytes returned and format_kernel_ms includes
+ *                          the compression kernels. */
+#define EMAB_OUTPUT_SAM 0
+#define EMAB_OUTPUT_BAM 1
 typedef struct emab_session emab_session_t;
 
 typedef struct {
@@ -294,17 +317,18 @@ typedef struct {
 	double ms_seed, ms_chain, ms_align1, ms_rescue, ms_finalize;
 	double gate_wait_ms;                              /* time spent waiting for a pipeline phase (emab_align_buckets) */
 	int64_t h2d_bytes, d2h_bytes;
-	int64_t n_pairs, n_barcodes, n_cands, n_clouds, sam_bytes;
+	int64_t n_pairs, n_barcodes, n_cands, n_clouds, sam_bytes;  /* sam_bytes: bytes returned (BAM: compressed) */
 	int64_t extend_cells, global_cells, local_cells, occ_touches;
 	int32_t launches, pad;
 	int64_t ext_planned_cells, ext_unplanned, glob_planned_cells, glob_unplanned;
 	double ms_ext_wave, ms_glob_wave;
-	double format_kernel_ms;                          /* device time of the SAM text kernels */
+	double format_kernel_ms;                          /* device time of the SAM text kernels (BAM: records + BGZF compression) */
 } emab_run_stats_t;
 
 int emab_session_open(const char *ref_path, const char *platform, int device, emab_session_t **out);
 void emab_session_close(emab_session_t *s);
 int emab_session_config(emab_session_t *s, const char *rg, const char *bx_index, int apply_opt, int n_threads);
+int emab_session_output(emab_session_t *s, int format);
 int emab_sam_header(emab_session_t *s, int argc, const char *const *argv, char **text, uint64_t *len);
 int emab_align_bucket(emab_session_t *s, const char *data, uint64_t len, char **sam, uint64_t *sam_len);
 int emab_align_fastq(emab_session_t *s, const char *d1, uint64_t l1, const char *d2, uint64_t l2, char **sam, uint64_t *sam_len);
