@@ -319,7 +319,8 @@ class RunStats(C.Structure):
                [(n, C.c_int64) for n in ("n_pairs", "n_barcodes", "n_cands", "n_clouds", "sam_bytes", "extend_cells", "global_cells",
                                          "local_cells", "occ_touches")] + [("launches", C.c_int32), ("pad", C.c_int32)] + \
                [(n, C.c_int64) for n in ("ext_planned_cells", "ext_unplanned", "glob_planned_cells", "glob_unplanned")] + \
-               [("ms_ext_wave", C.c_double), ("ms_glob_wave", C.c_double), ("format_kernel_ms", C.c_double)]
+               [("ms_ext_wave", C.c_double), ("ms_glob_wave", C.c_double), ("format_kernel_ms", C.c_double)] + \
+               [(n, C.c_double) for n in ("sort_ms", "gather_ms", "compress_ms", "index_ms")]
 
 
 class PinnedText:
@@ -358,16 +359,42 @@ class Session:
     emab_session_open / emab_sam_header / emab_align_bucket / emab_align_fastq."""
 
     OUTPUTS = {"sam": 0, "bam": 1}
+    SORT_OFF, SORT_COORD, SORT_COORD_NOINDEX = 0, 1, 2
+    _WRITE_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64)
 
     def __init__(self, ref_path: str, platform: str = "10x", device: int = 0, rg: str | None = None, bx_index: str | None = None,
-                 apply_opt: bool = False, threads: int = 1, output: str = "sam"):
+                 apply_opt: bool = False, threads: int = 1, output: str = "sam", sort: bool = False, max_host_bytes: int = 0):
         """output="bam": header() and every align call return BGZF members of BAM instead of SAM text
-        (a BAM file is header, the calls' bytes in order, then bgzf_eof())."""
+        (a BAM file is header, the calls' bytes in order, then bgzf_eof()).
+        sort=True (BAM only): align calls return b"" and hold their records (at most max_host_bytes of host memory, 0: no
+        cap); finish() returns them as one coordinate-sorted body and its BAI (file: header, body, bgzf_eof())."""
         self._h = C.c_void_p()
         _check(lib().emab_session_open(ref_path.encode(), platform.encode(), device, C.byref(self._h)))
         _check(lib().emab_session_config(self._h, rg.encode() if rg else None, bx_index.encode() if bx_index else None,
                                          int(apply_opt), threads))
         self.set_output(output)
+        if sort:
+            self.set_sort(True, max_host_bytes)
+
+    def set_sort(self, on: bool, max_host_bytes: int = 0, index: bool = True):
+        """emab_session_sort: coordinate-sorted BAM for the calls that follow (index=False: no BAI, any contig length)"""
+        mode = (self.SORT_COORD if index else self.SORT_COORD_NOINDEX) if on else self.SORT_OFF
+        _check(lib().emab_session_sort(self._h, mode, C.c_uint64(max_host_bytes)))
+
+    def finish(self) -> tuple[bytes, bytes]:
+        """emab_session_finish: (sorted BGZF body without the EOF block, .bai bytes; b"" without an index)"""
+        parts = []
+
+        def write(_u, p, n):
+            parts.append(C.string_at(p, n))
+            return 0
+        cb = self._WRITE_CB(write)
+        bai, n = C.c_void_p(), C.c_uint64()
+        _check(lib().emab_session_finish(self._h, cb, None, C.byref(bai), C.byref(n)))
+        idx = C.string_at(bai, n.value) if bai.value else b""
+        if bai.value:
+            lib().emab_free(bai)
+        return b"".join(parts), idx
 
     def set_output(self, output: str):
         """emab_session_output: "sam" or "bam" for the calls that follow"""

@@ -134,9 +134,11 @@ __global__ void k_bgzf_gather(const uint8_t *__restrict__ slots, const unsigned 
 
 // slots: 48 tokens (4 bytes per input byte), 49 one 64 KB member slot per chunk, 50 sizes / offsets / scan scratch,
 // 51 the packed members
-int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches)
+int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches,
+                         const unsigned long long **d_member_off)
 {
 	*out_len = 0; *launches = 0;
+	if (d_member_off) *d_member_off = nullptr;
 	cudaStream_t st = c->stream;
 	if (n == 0) { CUDA_TRY(cudaEventRecord(c->ev1, st)); return EMAB_OK; }
 	const uint64_t nc = (n + CHUNK - 1) / CHUNK;
@@ -170,6 +172,7 @@ int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *
 	CUDA_TRY(cudaGetLastError());
 	*launches = 3;
 	*out_len = total;
+	if (d_member_off) *d_member_off = d_off;
 	return EMAB_OK;
 }
 

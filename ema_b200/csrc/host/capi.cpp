@@ -94,6 +94,7 @@ int emab_sam_header(emab_session_t *h, int argc, const char *const *argv, char *
 		if (rc) { emab::text_free(p); return rc; }
 		p[n] = 0;
 		*text = p; *len = n;
+		h->s->header_bytes = n;
 		return EMAB_OK;
 	});
 }
@@ -108,12 +109,39 @@ int emab_session_output(emab_session_t *h, int format)
 	});
 }
 
+int emab_session_sort(emab_session_t *h, int on, uint64_t max_host_bytes)
+{
+	return guarded([&]() -> int {
+		if (!h) return fail(EMAB_ERR_ARG, "null session");
+		int rc = emab::session_sort(h->s, on, max_host_bytes);
+		if (rc) return fail(rc, h->s->err);
+		return EMAB_OK;
+	});
+}
+
+int emab_session_finish(emab_session_t *h, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len)
+{
+	return guarded([&]() -> int {
+		if (!h || !w || (bai && !bai_len)) return fail(EMAB_ERR_ARG, "null argument");
+		int rc = emab::session_finish(h->s, w, uw, bai, bai_len);
+		if (rc) return fail(rc, h->s->err);
+		return EMAB_OK;
+	});
+}
+
+// an align call that fails in sorted mode leaves its run incomplete: session_finish refuses it
+static int align_rc(emab_session_t *h, int rc)
+{
+	if (rc) emab::sort_call_failed(h->s, rc);
+	return rc;
+}
+
 int emab_align_bucket(emab_session_t *h, const char *data, uint64_t len, char **sam, uint64_t *sam_len)
 {
 	return guarded([&]() -> int {
 		if (!h || (!data && len)) return fail(EMAB_ERR_ARG, "null argument");
 		size_t n = 0;
-		int rc = emab::align_special_fastq(h->s, data, (size_t)len, sam, &n);
+		int rc = align_rc(h, emab::align_special_fastq(h->s, data, (size_t)len, sam, &n));
 		*sam_len = n;
 		if (rc) return fail(rc, h->s->err);
 		return EMAB_OK;
@@ -126,7 +154,7 @@ int emab_align_buckets(emab_session_t *h, int n, const char *const *data, const 
 		if (!h || n < 0 || (n && (!data || !len || !sam || !sam_len))) return fail(EMAB_ERR_ARG, "null argument");
 		std::vector<size_t> l(n), ol(n);
 		for (int i = 0; i < n; ++i) l[i] = (size_t)len[i];
-		int rc = emab::align_special_fastq_multi(h->s, n, data, l.data(), sam, ol.data());
+		int rc = align_rc(h, emab::align_special_fastq_multi(h->s, n, data, l.data(), sam, ol.data()));
 		for (int i = 0; i < n; ++i) sam_len[i] = ol[i];
 		if (rc) return fail(rc, h->s->err);
 		return EMAB_OK;
@@ -158,7 +186,7 @@ int emab_align_fastq(emab_session_t *h, const char *d1, uint64_t l1, const char 
 	return guarded([&]() -> int {
 		if (!h || (!d1 && l1)) return fail(EMAB_ERR_ARG, "null argument");
 		size_t n = 0;
-		int rc = emab::align_fastq(h->s, d1, (size_t)l1, d2, (size_t)l2, sam, &n);
+		int rc = align_rc(h, emab::align_fastq(h->s, d1, (size_t)l1, d2, (size_t)l2, sam, &n));
 		*sam_len = n;
 		if (rc) return fail(rc, h->s->err);
 		return EMAB_OK;
@@ -169,7 +197,7 @@ int emab_align_fastq_stream(emab_session_t *h, emab_read_cb r1, void *u1, emab_r
 {
 	return guarded([&]() -> int {
 		if (!h || !r1 || !w) return fail(EMAB_ERR_ARG, "null argument");
-		int rc = emab::align_fastq_stream(h->s, r1, u1, r2, u2, w, uw, batch_pairs);
+		int rc = align_rc(h, emab::align_fastq_stream(h->s, r1, u1, r2, u2, w, uw, batch_pairs));
 		if (rc) return fail(rc, h->s->err);
 		return EMAB_OK;
 	});

@@ -336,7 +336,7 @@ void session_close(Session *s)
 void sam_header(const Session *s, int argc, const char *const *argv, std::string *out)
 {  // src/align.c:193-212
 	char buf[2048];
-	out->append("@HD\tVN:1.3\tSO:unsorted\n");
+	out->append(s->sort != EMAB_SORT_OFF ? "@HD\tVN:1.3\tSO:coordinate\n" : "@HD\tVN:1.3\tSO:unsorted\n");
 	for (size_t i = 0; i < s->sq_names.size(); ++i) {
 		snprintf(buf, sizeof buf, "@SQ\tSN:%s\tLN:%d\n", s->sq_names[i].c_str(), s->sq_len[i]);
 		out->append(buf);
@@ -373,8 +373,88 @@ int session_output(Session *s, int format)
 				return EMAB_ERR_ARG;
 			}
 		}
+	if (format != EMAB_OUTPUT_BAM && s->sort != EMAB_SORT_OFF) { s->err = "error: coordinate sorting is on: turn it off before leaving BAM output"; return EMAB_ERR_ARG; }
 	s->output = format;
 	return EMAB_OK;
+}
+
+static void drop_runs(Session *s)
+{
+	std::lock_guard<std::mutex> g(s->run_mu);
+	s->runs.clear();
+	s->sort_held = 0;
+	s->sort_rc = 0;
+	s->sort_err.clear();
+}
+
+int session_sort(Session *s, int on, uint64_t max_host_bytes)
+{
+	if (on != EMAB_SORT_OFF && on != EMAB_SORT_COORD && on != EMAB_SORT_COORD_NOINDEX) { s->err = "error: unknown sort mode " + std::to_string(on); return EMAB_ERR_ARG; }
+	if (on != EMAB_SORT_OFF && s->output != EMAB_OUTPUT_BAM) { s->err = "error: coordinate sorting needs BAM output"; return EMAB_ERR_ARG; }
+	if (on == EMAB_SORT_COORD)
+		for (size_t i = 0; i < s->sq_names.size(); ++i)
+			if (s->sq_len[i] > (1 << 29) - 1) {
+				s->err = "error: contig " + s->sq_names[i] + " is " + std::to_string(s->sq_len[i]) +
+				         " bp long; a BAI index holds contigs of up to 536870911 bp (2^29 - 1), so no index can be written";
+				return EMAB_ERR_ARG;
+			}
+	drop_runs(s);
+	s->sort = on;
+	s->sort_cap = max_host_bytes;
+	return EMAB_OK;
+}
+
+void sort_call_failed(Session *s, int rc)
+{
+	std::lock_guard<std::mutex> g(s->run_mu);
+	if (s->sort == EMAB_SORT_OFF || s->sort_rc) return;
+	s->sort_rc = rc;
+	s->sort_err = "error: an align call of this sorted run failed (" + s->err + "), so the run cannot be written";
+}
+
+// a sorted call's records and rows join the run under its ticket, unless that takes the bytes held over the cap
+static int hold_run(Session *s, Worker &wk, int ticket, const char *raw, size_t len, std::vector<emab_bam_key_t> &&keys)
+{
+	const uint64_t bytes = len + keys.size() * sizeof(emab_bam_key_t);
+	Session::SortRun r;
+	r.raw.reset(new char[len ? len : 1]);
+	memcpy(r.raw.get(), raw, len);
+	r.keys = std::move(keys);
+	std::lock_guard<std::mutex> g(s->run_mu);
+	if (s->sort_cap && s->sort_held + bytes > s->sort_cap) {
+		wk.err = "error: the sorted run needs more than the " + std::to_string(s->sort_cap) + " bytes of host memory it may hold (" +
+		         std::to_string(s->sort_held + bytes) + " so far); nothing is written";
+		if (!s->sort_rc) { s->sort_rc = EMAB_ERR_OVERFLOW; s->sort_err = wk.err; }
+		return EMAB_ERR_OVERFLOW;
+	}
+	s->sort_held += bytes;
+	s->runs[ticket] = std::move(r);
+	return EMAB_OK;
+}
+
+int session_finish(Session *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len)
+{
+	if (bai) { *bai = nullptr; *bai_len = 0; }
+	if (s->sort == EMAB_SORT_OFF) { s->err = "error: emab_session_finish: coordinate sorting is off"; return EMAB_ERR_ARG; }
+	if (s->sort_rc) { const int rc = s->sort_rc; s->err = s->sort_err; drop_runs(s); return rc; }
+	const double t0 = now_ms();
+	std::vector<emab_bam_run_t> rv;
+	for (auto &kv : s->runs) rv.push_back({kv.second.raw.get(), kv.second.keys.data(), (uint64_t)kv.second.keys.size()});
+	int slice = 0;
+	if (const char *e = getenv("EMAB_SORT_SLICE_CHUNKS")) slice = atoi(e);   // tuning knob: 65 280-byte chunks per compressed slice
+	struct Count { emab_write_cb w; void *uw; uint64_t n; } cnt{w, uw, 0};
+	auto counted = [](void *u, const char *p, uint64_t n) -> int { Count *c = (Count *)u; c->n += n; return c->w(c->uw, p, n); };
+	double ms[4] = {0, 0, 0, 0};
+	emab_ctx_t *ctx = s->workers[0].ctx;
+	const int rc = emab_bam_sort(ctx, (int)rv.size(), rv.data(), (int)s->sq_names.size(), s->header_bytes, slice, counted, &cnt,
+	                             s->sort == EMAB_SORT_COORD ? bai : nullptr, bai_len, ms);
+	if (rc) s->err = emab_last_error();
+	drop_runs(s);
+	memset(&s->last, 0, sizeof s->last);
+	s->last.sort_ms = ms[0]; s->last.gather_ms = ms[1]; s->last.compress_ms = ms[2]; s->last.index_ms = ms[3];
+	s->last.sam_bytes = (int64_t)cnt.n;
+	s->last.total_ms = now_ms() - t0;
+	return rc;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1208,7 +1288,7 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 	for (const std::string &nm : s->fai_names) max_name = std::max(max_name, nm.size());
 	size_t cap = (size_t)n_out * (3 * max_name + s->bx_index.size() + s->rg_id.size() + 2 * 64 * 5 + 256) + 64;
 	for (size_t v : bound_part) cap += v;
-	const bool bam = s->output == EMAB_OUTPUT_BAM;
+	const bool bam = s->output == EMAB_OUTPUT_BAM, sorted = bam && s->sort != EMAB_SORT_OFF;
 	if (bam) {   // raw records fit the text bound plus 64 bytes each; BGZF adds at most a stored block's 31 bytes per 65 280
 		const size_t raw = cap + (size_t)n_out * 64;
 		cap = raw + (raw / 65280 + 1) * 64;
@@ -1221,8 +1301,18 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 		memset(&job, 0, sizeof job);
 		job.n_recs = (int32_t)n_out; job.n_bc = nb; job.recs = descs.data(); job.bc_off = bc_off.data(); job.bc_text = bc_text.data();
 		job.bx_index = s->bx_index.c_str(); job.rg_id = s->has_rg ? s->rg_id.c_str() : nullptr; job.is_haplotag = s->is_haplotag ? 1 : 0;
-		int rc = bam ? emab_bam_format(wk.ctx, &job, buf, (uint64_t)cap, &total) : emab_sam_format(wk.ctx, &job, buf, (uint64_t)cap, &total);
+		std::vector<emab_bam_key_t> keys(sorted ? (size_t)n_out : 0);
+		int rc = sorted ? emab_bam_records(wk.ctx, &job, buf, (uint64_t)cap, &total, keys.data())
+		       : bam ? emab_bam_format(wk.ctx, &job, buf, (uint64_t)cap, &total) : emab_sam_format(wk.ctx, &job, buf, (uint64_t)cap, &total);
 		if (rc) { wk.err = emab_last_error(); text_free(buf); return rc; }
+		if (sorted) {   // the records wait for session_finish; the call itself returns nothing
+			rc = hold_run(s, wk, ticket, buf, (size_t)total, std::move(keys));
+			text_free(buf);
+			buf = text_alloc(1);
+			if (rc || !buf) { text_free(buf); if (!rc) wk.err = "out of memory"; return rc ? rc : EMAB_ERR_NOMEM; }
+			st.d2h_bytes += (int64_t)total + (int64_t)n_out * (int64_t)sizeof(emab_bam_key_t);
+			total = 0;
+		}
 		st.launches += emab_last_launches(wk.ctx);
 		st.d2h_bytes += (int64_t)total;
 		st.h2d_bytes += (int64_t)n_out * (int64_t)sizeof(emab_sam_rec_t) + (int64_t)bc_text.size();

@@ -5,6 +5,8 @@
 #include <cctype>
 #include <condition_variable>
 #include <cstdint>
+#include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -150,6 +152,16 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 		if (cloud_turn == ticket) { ++cloud_turn; cv.notify_all(); }
 	}
 	int output = EMAB_OUTPUT_SAM;         // what the align calls return: SAM text or BGZF members of BAM records
+	// coordinate-sorted BAM (emab_session_sort): every align call's raw records and sort rows, held until session_finish.
+	// Keyed by ticket: tickets are taken in input order in every mode, so the map's order is the unsorted output order.
+	struct SortRun { std::unique_ptr<char[]> raw; std::vector<emab_bam_key_t> keys; };
+	int sort = EMAB_SORT_OFF;
+	uint64_t sort_cap = 0, sort_held = 0;  // cap on the bytes held (0: none), bytes held
+	std::map<int, SortRun> runs;
+	std::mutex run_mu;
+	int sort_rc = 0;                      // a call of this run failed: finish refuses with this code and message
+	std::string sort_err;
+	uint64_t header_bytes = 0;            // size of the BGZF header emab_sam_header returned last (where the body starts)
 	std::string err;
 	std::string gamma_dump;               // test hook: path for full-precision posteriors of the chosen alignments
 	emab_run_stats_t last{};
@@ -190,6 +202,10 @@ void sam_header(const Session *s, int argc, const char *const *argv, std::string
 // the uncompressed BAM header (SAM spec v1 §4.2): magic, the header text, the @SQ names and lengths
 void bam_header(const Session *s, const std::string &text, std::string *out);
 int session_output(Session *s, int format);   // EMAB_OUTPUT_SAM / EMAB_OUTPUT_BAM
+int session_sort(Session *s, int on, uint64_t max_host_bytes);   // EMAB_SORT_*
+// the held runs as one coordinate-sorted BGZF body to w, and its BAI (EMAB_SORT_COORD, bai != nullptr); releases the runs
+int session_finish(Session *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len);
+void sort_call_failed(Session *s, int rc);    // an align call failed in sorted mode: the run cannot be finished
 int session_set_workers(Session *s, int n_workers);
 int session_add_device(Session *s, int device);  // before session_set_workers
 // find_clouds_and_align (src/align.c:214) over the *contents* of the input file(s); SAM text in a malloc'ed buffer

@@ -100,8 +100,10 @@ struct emab_ctx {
 };
 
 // BGZF members of d_in[0..n) (device memory) into the host buffer out (bgzf.cu); records ev1 after the last kernel.
-// Slots 48-51.  *launches = kernels launched.
-int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches);
+// Slots 48-51.  *launches = kernels launched.  d_member_off (optional) receives a device pointer to the members' offsets in
+// out (one per chunk, then the total), valid until the ctx's next call.
+int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches,
+                         const unsigned long long **d_member_off = nullptr);
 
 // first statement of every entry point that takes a ctx: a worker thread of the host pipeline (or any caller's
 // thread) starts on device 0, and a stream or buffer of another device is an invalid argument there

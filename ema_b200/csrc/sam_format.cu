@@ -13,6 +13,7 @@
 //   (scan)                         record offsets, total
 //   k_sam_write  warp / record     the same emitter with a writing writer: short fields by lane 0, strings lane-strided
 //   k_bam_len / (scan) / k_bam_write   the same for BAM records (SAM spec v1 §4.2), then BGZF members (bgzf.cu)
+//   k_bam_key    thread / record   sorted mode: the record's coordinate key, end, bin and length (bam_sort.cu orders them)
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -21,6 +22,7 @@
 #include "../../include/ema_b200.h"
 #include "runtime.cuh"
 #include "bgzf.cuh"
+#include "bai.cuh"
 
 #define TRY(x) do { int rc__ = (x); if (rc__) return rc__; } while (0)
 #ifndef FULL_MASK
@@ -226,17 +228,6 @@ __device__ void emit_record(W &w, const SamTables &t, const emab_sam_rec_t &d)
 
 // ---- BAM (SAM spec v1 §4.2) ----
 
-__device__ int reg2bin(long long beg, long long end)
-{
-	--end;
-	if (beg >> 14 == end >> 14) return ((1 << 15) - 1) / 7 + (int)(beg >> 14);
-	if (beg >> 17 == end >> 17) return ((1 << 12) - 1) / 7 + (int)(beg >> 17);
-	if (beg >> 20 == end >> 20) return ((1 << 9) - 1) / 7 + (int)(beg >> 20);
-	if (beg >> 23 == end >> 23) return ((1 << 6) - 1) / 7 + (int)(beg >> 23);
-	if (beg >> 26 == end >> 26) return ((1 << 3) - 1) / 7 + (int)(beg >> 26);
-	return 0;
-}
-
 // the float nearest to the decimal text of XG:f (what strtof gives; the quotient is formed in double, so a value within
 // 2^-53 of a halfway point between two floats could round differently — the %.5g texts here have at most six digits)
 __device__ float parse_float(const char *s, int n)
@@ -307,7 +298,7 @@ __device__ void emit_bam(W &w, const SamTables &t, const emab_sam_rec_t &d, uint
 	w.le((uint32_t)pos, 4);
 	w.le(pt.id_len[m] + 1, 1);
 	w.le(d.mapq, 1);
-	if (v.rec) { const int rl = ref_len(*v.rec, t.cigars); w.le((uint32_t)reg2bin(pos, pos + (rl > 0 ? rl : 1)), 2); }
+	if (v.rec) { const int rl = ref_len(*v.rec, t.cigars); w.le((uint32_t)bai::reg2bin(pos, pos + (rl > 0 ? rl : 1)), 2); }
 	else w.le(4680, 2);   // reg2bin(-1, 0)
 	w.le((uint32_t)n_cigar, 2);
 	w.le(d.flag, 2);
@@ -386,6 +377,26 @@ k_bam_write(SamTables t, const emab_sam_rec_t *recs, int n, const unsigned long 
 	if (i >= n) return;
 	WarpWriter w{out + off[i], (int)(threadIdx.x & 31)};
 	emit_bam(w, t, recs[i], (uint32_t)(off[i + 1] - off[i] - 4));
+}
+
+// sorted mode: what bam_sort.cu orders and indexes, from the same view emit_bam writes refID, POS, bin and FLAG from
+__global__ void k_bam_key(SamTables t, const emab_sam_rec_t *recs, int n, const unsigned long long *off, emab_bam_key_t *keys)
+{
+	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	const emab_sam_rec_t &d = recs[i];
+	const RecView v = make_view(t, d);
+	const int32_t ref = v.chrom >= 0 ? t.chrom2sq[v.chrom] : -1;
+	const long long pos = v.pos - 1;
+	emab_bam_key_t k;
+	k.key = (unsigned long long)(uint32_t)ref << 32 | (unsigned long long)(uint32_t)(pos + 1) << 1 | ((d.flag & 16) ? 1u : 0u);
+	k.unmapped = (d.flag & 4) ? 1 : 0;
+	const int rl = v.rec && !k.unmapped ? ref_len(*v.rec, t.cigars) : 0;
+	k.end = (uint32_t)(ref >= 0 ? pos + (rl > 0 ? rl : 1) : 0);
+	k.bin = (uint16_t)(ref >= 0 ? bai::reg2bin(pos, k.end) : 4680);   // emit_bam's bin: reads are placed only when mapped
+	k.len = (uint32_t)(off[i + 1] - off[i]);
+	k.pad = 0;
+	keys[i] = k;
 }
 
 }  // namespace
@@ -492,21 +503,19 @@ extern "C" int emab_sam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *o
 	return EMAB_OK;
 }
 
-// The BAM counterpart: records written to slot 33, compressed into BGZF members (bgzf.cu), only the members copied back.
-extern "C" int emab_bam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len)
+// BAM records of a job written to slot 33 (k_bam_len -> scan -> k_bam_write), offsets in slot 47; `fn` names the caller in
+// the messages.  *raw = 0 and nothing launched for an empty job.
+static int bam_records_device(emab_ctx_t *c, const emab_sam_job_t *job, const char *fn, SamTables &t, unsigned long long *raw)
 {
-	CTX_ENTER(c);
-	if (!c || !job || !out_len) return EMAB_ERR_ARG;
-	*out_len = 0;
-	if (!c->sam_tables_ready || !c->text_ready) { snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_format: tables or batch text not on the device"); return EMAB_ERR_ARG; }
+	*raw = 0;
+	if (!c->sam_tables_ready || !c->text_ready) { snprintf(emab_errbuf, sizeof emab_errbuf, "%s: tables or batch text not on the device", fn); return EMAB_ERR_ARG; }
 	if (!c->bam_unmapped_contig.empty()) {
-		snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_format: contig %s has no @SQ entry of its .fai name, so BAM cannot refer to it", c->bam_unmapped_contig.c_str());
+		snprintf(emab_errbuf, sizeof emab_errbuf, "%s: contig %s has no @SQ entry of its .fai name, so BAM cannot refer to it", fn, c->bam_unmapped_contig.c_str());
 		return EMAB_ERR_ARG;
 	}
 	const int n = job->n_recs;
 	if (n == 0) return EMAB_OK;
 	cudaStream_t st = c->stream;
-	SamTables t;
 	TRY(stage_job(c, job, t));
 	const emab_sam_rec_t *d_recs = c->b[46].as<emab_sam_rec_t>();
 	TRY(c->b[47].ensure((size_t)(n + 1) * 8 * 2 + 16));
@@ -525,16 +534,56 @@ extern "C" int emab_bam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *o
 	if (hv[1] != ~0ull) {
 		const unsigned long long r = hv[1] >> 2;
 		const int why = (int)(hv[1] & 3);
-		snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_format: record %llu (pair %u, read %d): %s", r, job->recs[r].pair, job->recs[r].which + 1,
+		snprintf(emab_errbuf, sizeof emab_errbuf, "%s: record %llu (pair %u, read %d): %s", fn, r, job->recs[r].pair, job->recs[r].which + 1,
 		         why == BAM_NAME_LEN ? "read name longer than 254 bytes" : why == BAM_QUAL_LEN ? "quality string length differs from the read's" : "quality byte outside '!'..'~'");
 		return EMAB_ERR_ARG;
 	}
-	const unsigned long long raw = hv[0];
-	TRY(c->b[33].ensure((size_t)raw + 16));
+	*raw = hv[0];
+	TRY(c->b[33].ensure((size_t)*raw + 16));
 	k_bam_write<<<(n * 32 + 255) / 256, 256, 0, st>>>(t, d_recs, n, d_off, c->b[33].as<char>());
+	return EMAB_OK;
+}
+
+// The BAM counterpart: records written to slot 33, compressed into BGZF members (bgzf.cu), only the members copied back.
+extern "C" int emab_bam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len)
+{
+	CTX_ENTER(c);
+	if (!c || !job || !out_len) return EMAB_ERR_ARG;
+	*out_len = 0;
+	SamTables t;
+	unsigned long long raw = 0;
+	TRY(bam_records_device(c, job, "emab_bam_format", t, &raw));
+	if (job->n_recs == 0) return EMAB_OK;
 	int launches = 0;
 	TRY(bgzf_compress_device(c, c->b[33].as<uint8_t>(), raw, (uint8_t *)out, out_cap, out_len, &launches));
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 	c->last_ms = ms; c->last_launches = 4 + launches;
+	return EMAB_OK;
+}
+
+// Sorted mode: the raw records and their sort rows (slot 34) copied back; nothing is compressed per call.
+extern "C" int emab_bam_records(emab_ctx_t *c, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len, emab_bam_key_t *keys)
+{
+	CTX_ENTER(c);
+	if (!c || !job || !out_len || (job->n_recs && !keys)) return EMAB_ERR_ARG;
+	*out_len = 0;
+	SamTables t;
+	unsigned long long raw = 0;
+	TRY(bam_records_device(c, job, "emab_bam_records", t, &raw));
+	const int n = job->n_recs;
+	if (n == 0) return EMAB_OK;
+	if (raw > out_cap) { *out_len = raw; snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_records: %llu bytes do not fit the output buffer", raw); return EMAB_ERR_OVERFLOW; }
+	cudaStream_t st = c->stream;
+	TRY(c->b[34].ensure((size_t)n * sizeof(emab_bam_key_t)));
+	const unsigned long long *d_off = c->b[47].as<unsigned long long>() + (n + 1);
+	k_bam_key<<<(n + 127) / 128, 128, 0, st>>>(t, c->b[46].as<emab_sam_rec_t>(), n, d_off, c->b[34].as<emab_bam_key_t>());
+	CUDA_TRY(cudaEventRecord(c->ev1, st));
+	CUDA_TRY(cudaMemcpyAsync(out, c->b[33].p, (size_t)raw, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(keys, c->b[34].p, (size_t)n * sizeof(emab_bam_key_t), cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(ctx_wait(c));
+	CUDA_TRY(cudaGetLastError());
+	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
+	c->last_ms = ms; c->last_launches = 4;
+	*out_len = raw;
 	return EMAB_OK;
 }

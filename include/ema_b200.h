@@ -254,6 +254,37 @@ int emab_sam_format(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint6
  *                    deterministic: csrc/bgzf.cuh compiled for the host makes the same bytes.
  * emab_bgzf_eof     = the 28-byte empty member that ends a BGZF file (static storage; needs no GPU). */
 int emab_bam_format(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len);
+/* emab_bam_records = emab_bam_format without the compression: the raw BAM records into `out`, and one sort row per record
+ *                    into keys[n_recs], read from the same view of the record as the emitter.  The rows are what
+ *                    emab_bam_sort orders and indexes:
+ *                      key       (uint64)(uint32)refID << 32 | (uint64)(POS + 1) << 1 | reverse (samtools' coordinate key)
+ *                      end       POS + the CIGAR's reference length; POS + 1 if that is 0 or the record is unmapped
+ *                      len       the record's bytes (block_size + 4)
+ *                      bin       reg2bin(POS, end), as the record holds it
+ *                      unmapped  FLAG & 4 */
+typedef struct {
+	uint64_t key;
+	uint32_t end, len;
+	uint16_t bin, unmapped;
+	uint32_t pad;
+} emab_bam_key_t;
+int emab_bam_records(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len, emab_bam_key_t *keys);
+/* emab_bam_sort = one coordinate-sorted BGZF body (and its BAI) from runs of raw records in input order.  A stable radix
+ *                    sort of (key, record index) on the device gives the order; records are gathered on the host in that
+ *                    order into page-locked slices of slice_chunks x 65 280 bytes (0 = 1 024 chunks), each compressed by the
+ *                    device BGZF encoder and passed to w in order (no EOF block).  Members are cut every 65 280 bytes of
+ *                    the whole body, so the bytes do not depend on the slice size.  With bai != NULL the index is built on
+ *                    the device (csrc/bai.cuh states its rules) over n_ref references, with file offsets counted from
+ *                    body_offset (the compressed header's size); free it with emab_free.  ms[4] (optional) receives the
+ *                    wall time of the device sort, the host gather, the compression and the index build. */
+typedef struct {
+	const char *raw;                /* the run's records, back to back */
+	const emab_bam_key_t *keys;     /* one row per record, in the same order */
+	uint64_t n_recs;
+} emab_bam_run_t;
+typedef int (*emab_write_cb)(void *user, const char *text, uint64_t len);
+int emab_bam_sort(emab_ctx_t *ctx, int n_runs, const emab_bam_run_t *runs, int n_ref, uint64_t body_offset, int slice_chunks,
+                  emab_write_cb w, void *uw, char **bai, uint64_t *bai_len, double ms[4]);
 int emab_bgzf_compress(emab_ctx_t *ctx, const uint8_t *in, uint64_t len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
 int emab_bgzf_eof(const uint8_t **p, uint64_t *len);
 /* pinned host memory for callers that want their input buffers to take the fast H2D path */
@@ -323,12 +354,33 @@ typedef struct {
 	int64_t ext_planned_cells, ext_unplanned, glob_planned_cells, glob_unplanned;
 	double ms_ext_wave, ms_glob_wave;
 	double format_kernel_ms;                          /* device time of the SAM text kernels (BAM: records + BGZF compression) */
+	/* emab_session_finish (sorted BAM): wall time of the device sort, the host gather, the compression (slices to the device,
+	 * BGZF kernels, members back and written) and the index build */
+	double sort_ms, gather_ms, compress_ms, index_ms;
 } emab_run_stats_t;
 
 int emab_session_open(const char *ref_path, const char *platform, int device, emab_session_t **out);
 void emab_session_close(emab_session_t *s);
 int emab_session_config(emab_session_t *s, const char *rg, const char *bx_index, int apply_opt, int n_threads);
 int emab_session_output(emab_session_t *s, int format);
+/* Coordinate-sorted BAM (BAM output only).  emab_session_sort(s, on, max_host_bytes):
+ *   EMAB_SORT_OFF        align calls return BGZF members as above (turning sorting off drops the records held so far)
+ *   EMAB_SORT_COORD      align calls return zero bytes; their raw records and sort rows (emab_bam_records) are held in
+ *                        host memory, in input order, until emab_session_finish writes them as one body sorted by
+ *                        samtools' coordinate key (stable: equal keys keep input order, unplaced records last) and returns
+ *                        its BAI.  Refused when a contig is longer than 2^29 - 1 bp, which a BAI cannot index.
+ *   EMAB_SORT_COORD_NOINDEX  the same without the index (any contig length)
+ * max_host_bytes caps the bytes held (raw records + 24 bytes per record; 0: no cap): the align call that would go over it
+ * fails with EMAB_ERR_OVERFLOW, and so does emab_session_finish after it, which then writes nothing.  Runs are not spilled
+ * to disk.  emab_sam_header says SO:coordinate in sorted mode.
+ * emab_session_finish(s, w, uw, bai, bai_len): the sorted BGZF body to w (without the EOF block) and, in EMAB_SORT_COORD,
+ * the .bai in a buffer released with emab_free (bai may be NULL to skip it).  The index's file offsets count the bytes of
+ * the header emab_sam_header returned last.  The held records are released; later calls start a new run. */
+#define EMAB_SORT_OFF 0
+#define EMAB_SORT_COORD 1
+#define EMAB_SORT_COORD_NOINDEX 2
+int emab_session_sort(emab_session_t *s, int on, uint64_t max_host_bytes);
+int emab_session_finish(emab_session_t *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len);
 int emab_sam_header(emab_session_t *s, int argc, const char *const *argv, char **text, uint64_t *len);
 int emab_align_bucket(emab_session_t *s, const char *data, uint64_t len, char **sam, uint64_t *sam_len);
 int emab_align_fastq(emab_session_t *s, const char *d1, uint64_t l1, const char *d2, uint64_t l2, char **sam, uint64_t *sam_len);
@@ -337,7 +389,6 @@ int emab_align_fastq(emab_session_t *s, const char *d1, uint64_t l1, const char 
  * one interleaved input) and receive the SAM body in input order.  Groups are cut into device batches of about batch_pairs
  * pairs (0 = 40 000) at barcode boundaries, up to `workers` batches in flight; memory is bounded by the batches in flight. */
 typedef int64_t (*emab_read_cb)(void *user, char *buf, int64_t cap);
-typedef int (*emab_write_cb)(void *user, const char *text, uint64_t len);
 int emab_align_fastq_stream(emab_session_t *s, emab_read_cb r1, void *u1, emab_read_cb r2, void *u2, emab_write_cb w, void *uw, int batch_pairs);
 /* -x (multi-input) mode: n buckets with up to `workers` of them in flight on this GPU (each worker is a
  * CUDA stream + scratch, so one bucket's kernels overlap another's host work and copies).  sam[i] /
