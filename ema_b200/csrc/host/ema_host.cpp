@@ -29,6 +29,7 @@
 #include <malloc.h>
 #include <memory>
 #include <mutex>
+#include <optional>
 #include <string_view>
 #include <thread>
 #include <unordered_map>
@@ -970,19 +971,18 @@ static const uint8_t *nt4_table()
 // The text a batch's pairs point into: one block (a bucket's contents) or two (-1 and -2 files).
 struct TextSrc { const char *base[2] = {nullptr, nullptr}; size_t len[2] = {0, 0}; };
 
-static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector<Pair> &pairs, const TextSrc &src, char **out_buf, size_t *out_len, emab_run_stats_t &st,
+static int process_pairs(Session *s, Worker &wk, Ticket &tk, const std::vector<Pair> &pairs, const TextSrc &src, char **out_buf, size_t *out_len, emab_run_stats_t &st,
                          const emab_pair_text_t *resident_ptab = nullptr)   // non-null: emab_parse_bucket left text and pair table on wk.ctx's device
 {
-	const int ticket = gp.ticket;
 	const double t0 = now_ms();
 	const size_t np = pairs.size();
 	const int nthr = wk.n_threads;
 	memset(&st, 0, sizeof st);
 	st.n_pairs = (int64_t)np;
 	*out_buf = nullptr; *out_len = 0;
-	if (np == 0) { s->take_cloud_base(ticket, 0); *out_buf = text_alloc(1); return EMAB_OK; }
+	if (np == 0) { *out_buf = text_alloc(1); return EMAB_OK; }
 	// ---- encode and align the whole batch on the device
-	if (wk.off.ensure((2 * np + 1) * 8)) { wk.err = emab_last_error(); s->take_cloud_base(ticket, 0); return EMAB_ERR_NOMEM; }
+	if (wk.off.ensure((2 * np + 1) * 8)) { wk.err = emab_last_error(); return EMAB_ERR_NOMEM; }
 	int64_t *off = (int64_t *)wk.off.p;
 	off[0] = 0;
 	for (size_t i = 0; i < np; ++i) {
@@ -992,8 +992,8 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 	// the batch's text goes to the device as it is (page-locked copy first: the caller's buffer is pageable), with one
 	// record per pair saying where names, bases and qualities are; the device derives the nt4 reads from it
 	const size_t text_len = src.len[0] + src.len[1];
-	if (text_len >= 0xffffffffull) { wk.err = "batch text larger than 4 GB"; s->take_cloud_base(ticket, 0); return EMAB_ERR_ARG; }
-	if (!resident_ptab && (wk.seq.ensure(text_len + 16) || wk.ptab.ensure(np * sizeof(emab_pair_text_t) + 16))) { wk.err = emab_last_error(); s->take_cloud_base(ticket, 0); return EMAB_ERR_NOMEM; }
+	if (text_len >= 0xffffffffull) { wk.err = "batch text larger than 4 GB"; return EMAB_ERR_ARG; }
+	if (!resident_ptab && (wk.seq.ensure(text_len + 16) || wk.ptab.ensure(np * sizeof(emab_pair_text_t) + 16))) { wk.err = emab_last_error(); return EMAB_ERR_NOMEM; }
 	char *text = (char *)wk.seq.p;
 	const emab_pair_text_t *ptab = resident_ptab ? resident_ptab : (const emab_pair_text_t *)wk.ptab.p;
 	int bad_view = 0;
@@ -1024,21 +1024,21 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 		for (int m = 0; m < 2; ++m) { where(pairs[i].read[m], &t.read_off[m], &t.read_len[m]); where(pairs[i].qual[m], &t.qual_off[m], &t.qual_len[m]); }
 	}
 	}
-	if (bad_view) { wk.err = "internal error: a pair's text lies outside the batch text"; s->take_cloud_base(ticket, 0); return EMAB_ERR_ARG; }
+	if (bad_view) { wk.err = "internal error: a pair's text lies outside the batch text"; return EMAB_ERR_ARG; }
 	emab_stats_t ds;
 	emab_pairs_result_t res;
 	const double t1 = now_ms();
-	gp.to(PH_DEVICE);
+	tk.to(PH_DEVICE);
 	const double t1b = now_ms();
 	{
 		int rc = resident_ptab ? emab_align_pairs_resident(wk.ctx, (int)np, off, &res, &ds)
 		                       : emab_align_pairs_text(wk.ctx, (int)np, text, text_len, ptab, off, &res, &ds);
-		if (rc) { wk.err = emab_last_error(); s->take_cloud_base(ticket, 0); return rc; }
+		if (rc) { wk.err = emab_last_error(); return rc; }
 	}
 	const int32_t *n_regs = res.n_regs;
 	const emab_cand_t *alns = res.cands;
 	const double t2a = now_ms();
-	gp.to(PH_POST);
+	tk.to(PH_POST);
 	// POST admission is in bucket order, so the -d turns are handed out in bucket order here
 	std::unique_ptr<TurnPass> density_turn;
 	if (s->apply_opt) density_turn.reset(new TurnPass(s->density));
@@ -1141,7 +1141,7 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 	}
 	const int E = bc_entry_off[nb], C = bc_cloud_off[nb], G = bc_group_off[nb], U = bc_unit_off[nb];
 	const int64_t K = bc_cand_off[nb];
-	if (K > 0x7fffffff) { wk.err = "too many candidates in one batch"; s->take_cloud_base(ticket, 0); return EMAB_ERR_OVERFLOW; }
+	if (K > 0x7fffffff) { wk.err = "too many candidates in one batch"; return EMAB_ERR_OVERFLOW; }
 	st.n_cands = K; st.n_clouds = C;
 	std::vector<int32_t> entry_cand_off(E + 1, 0), entry_mate(E), cand_cloud(K), cand_chrom(K), group_off(G + 1, 0), group_clouds(C),
 	    contrib_off(C + 1, 0), contrib(K), unit_first(U), unit_second(U);
@@ -1211,7 +1211,7 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 		P.group_off = group_off.data(); P.group_clouds = group_clouds.data(); P.cloud_contrib_off = contrib_off.data(); P.cloud_contrib = contrib.data();
 		P.unit_first = unit_first.data(); P.unit_second = unit_second.data();
 		int rc = emab_em_batch(wk.ctx, &P, gamma.data());
-		if (rc) { wk.err = emab_last_error(); s->take_cloud_base(ticket, 0); return rc; }
+		if (rc) { wk.err = emab_last_error(); return rc; }
 		st.em_kernel_ms = emab_last_kernel_ms(wk.ctx);
 		st.h2d_bytes += (int64_t)K * 29 + (int64_t)(E + C + G + U + 4 * nb) * 4;
 		st.d2h_bytes += (int64_t)K * 8;
@@ -1219,7 +1219,7 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 	}
 	const double t5 = now_ms();
 	// ---- choose, mark duplicates, print; cloud ids continue the session-wide counter in barcode order
-	std::vector<int> cloud_base(nb + 1, s->take_cloud_base(ticket, C));
+	std::vector<int> cloud_base(nb + 1, tk.cloud_base(C));
 	for (int b = 0; b < nb; ++b) cloud_base[b + 1] = cloud_base[b] + (int)bcs[b].clouds.size();
 	#pragma omp parallel for num_threads(nthr) schedule(dynamic, 1)
 	for (int b = 0; b < nb; ++b) {
@@ -1306,7 +1306,7 @@ static int process_pairs(Session *s, Worker &wk, GatePass &gp, const std::vector
 		       : bam ? emab_bam_format(wk.ctx, &job, buf, (uint64_t)cap, &total) : emab_sam_format(wk.ctx, &job, buf, (uint64_t)cap, &total);
 		if (rc) { wk.err = emab_last_error(); text_free(buf); return rc; }
 		if (sorted) {   // the records wait for session_finish; the call itself returns nothing
-			rc = hold_run(s, wk, ticket, buf, (size_t)total, std::move(keys));
+			rc = hold_run(s, wk, tk.id, buf, (size_t)total, std::move(keys));
 			text_free(buf);
 			buf = text_alloc(1);
 			if (rc || !buf) { text_free(buf); if (!rc) wk.err = "out of memory"; return rc ? rc : EMAB_ERR_NOMEM; }
@@ -1471,20 +1471,19 @@ static int parse_bucket(Session *s, int nthr, const char *data, size_t len, std:
 
 // read_special_fastq (src/align.c:759-806): one pair per line "BC @id read1 qual1 read2 qual2",
 // lines stably sorted by their first BC_LEN characters.
-static int run_bucket(Session *s, Worker &wk, int ticket, const char *data, size_t len, char **out, size_t *out_len, emab_run_stats_t &st, std::string *err)
+static int run_bucket(Session *s, Worker &wk, Ticket &tk, const char *data, size_t len, char **out, size_t *out_len, emab_run_stats_t &st)
 {
-	GatePass gp(s, ticket);
 	const double tw = now_ms();
-	gp.to(PH_PARSE);
+	tk.to(PH_PARSE);
 	const double t0 = now_ms();
 	// the bucket's text goes to the device once (through a page-locked copy) and is parsed there: line split, stable barcode
 	// sort, tokens, barcode codes (csrc/parse.cu).  What comes back is one record per pair saying where its fields are.
-	if (len >= 0xfffffff0ull) { *err = "bucket larger than 4 GB"; s->take_cloud_base(ticket, 0); return EMAB_ERR_ARG; }
+	if (len >= 0xfffffff0ull) { wk.err = "bucket larger than 4 GB"; return EMAB_ERR_ARG; }
 	// a caller's buffer that is already page-locked (emab_pinned_alloc, cudaHostAlloc, cudaHostRegister) is copied to the
 	// device as it is; anything else goes through this worker's page-locked staging copy first
 	const char *h2d_src = data;
 	if (!emab_is_pinned_host(data)) {
-		if (wk.seq.ensure(len + 16)) { *err = emab_last_error(); s->take_cloud_base(ticket, 0); return EMAB_ERR_NOMEM; }
+		if (wk.seq.ensure(len + 16)) { wk.err = emab_last_error(); return EMAB_ERR_NOMEM; }
 		char *text = (char *)wk.seq.p;
 		const long long n_blk = (long long)((len + (1u << 20) - 1) >> 20);
 		#pragma omp parallel for num_threads(wk.n_threads) schedule(static)
@@ -1499,7 +1498,7 @@ static int run_bucket(Session *s, Worker &wk, int ticket, const char *data, size
 	const emab_pair_text_t *pt = nullptr;
 	const uint64_t *bcs = nullptr;
 	int rc = emab_parse_bucket(wk.ctx, h2d_src, (uint64_t)len, s->bc_len, s->is_haplotag ? 1 : 0, &n, &pt, &bcs);
-	if (rc) { *err = emab_last_error(); s->take_cloud_base(ticket, 0); return rc; }
+	if (rc) { wk.err = emab_last_error(); return rc; }
 	std::vector<Pair> pairs((size_t)n);
 	#pragma omp parallel num_threads(wk.n_threads)
 	{
@@ -1516,12 +1515,109 @@ static int run_bucket(Session *s, Worker &wk, int ticket, const char *data, size
 	const double t1 = now_ms();
 	TextSrc src;
 	src.base[0] = data; src.len[0] = len;
-	rc = process_pairs(s, wk, gp, pairs, src, out, out_len, st, n > 0 ? pt : nullptr);
-	if (rc) *err = wk.err;
+	rc = process_pairs(s, wk, tk, pairs, src, out, out_len, st, n > 0 ? pt : nullptr);
 	st.parse_ms = t1 - t0;
 	st.total_ms += t1 - t0;
 	st.gate_wait_ms += t0 - tw;
 	return rc;
+}
+
+// Sums one batch's stats into a call's.  total_ms (the call's wall time) and sort_ms .. index_ms (session_finish's) are
+// set, not summed.  A field added to emab_run_stats_t fails the size check until it is summed here or named above.
+static void add_stats(emab_run_stats_t &into, const emab_run_stats_t &from)
+{
+	static_assert(sizeof(emab_run_stats_t) == 312, "emab_run_stats_t changed: sum the new field in add_stats");
+	into.parse_ms += from.parse_ms; into.encode_ms += from.encode_ms; into.align_ms += from.align_ms; into.kernel_ms += from.kernel_ms;
+	into.cloud_ms += from.cloud_ms; into.flatten_ms += from.flatten_ms; into.em_ms += from.em_ms; into.em_kernel_ms += from.em_kernel_ms;
+	into.format_ms += from.format_ms; into.format_kernel_ms += from.format_kernel_ms; into.gate_wait_ms += from.gate_wait_ms;
+	into.ms_seed += from.ms_seed; into.ms_chain += from.ms_chain; into.ms_align1 += from.ms_align1; into.ms_rescue += from.ms_rescue;
+	into.ms_finalize += from.ms_finalize; into.ms_ext_wave += from.ms_ext_wave; into.ms_glob_wave += from.ms_glob_wave;
+	into.h2d_bytes += from.h2d_bytes; into.d2h_bytes += from.d2h_bytes;
+	into.n_pairs += from.n_pairs; into.n_barcodes += from.n_barcodes; into.n_cands += from.n_cands; into.n_clouds += from.n_clouds;
+	into.sam_bytes += from.sam_bytes; into.launches += from.launches;
+	into.extend_cells += from.extend_cells; into.global_cells += from.global_cells; into.local_cells += from.local_cells;
+	into.occ_touches += from.occ_touches;
+	into.ext_planned_cells += from.ext_planned_cells; into.ext_unplanned += from.ext_unplanned;
+	into.glob_planned_cells += from.glob_planned_cells; into.glob_unplanned += from.glob_unplanned;
+}
+
+// One batch of a run_batches call: its output, its stats and, when it failed, why.
+struct Batch {
+	char *text = nullptr;   // output block (text_alloc); done() takes it
+	size_t len = 0;
+	emab_run_stats_t st{};
+	int rc = EMAB_OK;
+	std::string err;
+};
+
+// Nothing unwinds out of a worker thread: an exception fails its batch, not the caller's process.
+template <class F>
+static int caught(std::string &err, F &&f)
+{
+	try { return f(); }
+	catch (const std::bad_alloc &) { err = "out of host memory"; return EMAB_ERR_NOMEM; }
+	catch (const std::exception &e) { err = std::string("internal error: ") + e.what(); return EMAB_ERR_ARG; }
+	catch (...) { err = "internal error"; return EMAB_ERR_ARG; }
+}
+
+// The batch runner of -x, the -1/-2 stream and the split bucket.  Batches walk the ordered phases with up to n_workers
+// of them in flight, one per worker; the calling thread is worker 0.  The driver says what a batch is:
+//   next(seq, b)        claims batch seq: 1, or 0 at the end, or < 0 when it fails (why in b.err).  It runs under the
+//                       runner's lock, and the batch's ticket is taken in the same critical section: ticket order is
+//                       input order.
+//   run(wk, tk, seq, b) the batch's work on worker wk: an EMAB_* code, the message of a failure in wk.err.
+//   done(seq, b)        on the same thread after run, its ticket given back, for every claimed batch, failed (b.rc) or
+//                       not.  It may fail the batch itself (b.rc, b.err), and must not throw.
+// caps are the phase gates' capacities (at most one batch per worker), threads_per_batch the OpenMP threads of one batch.
+// The first failure stops new claims, and the call reports the failure of the earliest batch in input order.  s->last
+// becomes the sum of the batches' stats, its total_ms the call's wall time.
+template <class B, class Next, class Run, class Done>
+static int run_batches(Session *s, int n_workers, const int (&caps)[PH_COUNT], int threads_per_batch, Next next, Run run, Done done)
+{
+	for (int k = 0; k < PH_COUNT; ++k) s->gate[k].cap = std::max(1, std::min(caps[k], n_workers));
+	memset(&s->last, 0, sizeof s->last);
+	const double t0 = now_ms();
+	std::mutex mu;
+	int n_claimed = 0, err_seq = -1, err_rc = EMAB_OK;
+	std::string err_msg;
+	auto fail = [&](int seq, int rc, const std::string &msg) {   // under mu
+		if (err_seq < 0 || seq < err_seq) { err_seq = seq; err_rc = rc; err_msg = msg.empty() ? "error" : msg; }
+	};
+	auto worker = [&](int w) {
+		Worker &wk = s->workers[w];
+		emab_ctx_make_current(wk.ctx);   // worker threads start on device 0
+		wk.n_threads = threads_per_batch;
+		for (;;) {
+			B b;
+			int seq;
+			std::optional<Ticket> tk;
+			{
+				std::lock_guard<std::mutex> g(mu);
+				if (err_seq >= 0) return;
+				seq = n_claimed;
+				const int c = caught(b.err, [&] { return next(seq, b); });
+				if (c < 0) fail(seq, c, b.err);
+				if (c <= 0) return;
+				++n_claimed;
+				tk.emplace(s);
+			}
+			wk.err.clear();
+			b.rc = caught(b.err, [&] { const int rc = run(wk, *tk, seq, b); if (rc) b.err = wk.err; return rc; });
+			tk.reset();
+			done(seq, b);
+			std::lock_guard<std::mutex> g(mu);
+			++s->device_buckets[wk.dev_slot];
+			add_stats(s->last, b.st);
+			if (b.rc) fail(seq, b.rc, b.err);
+		}
+	};
+	std::vector<std::thread> th;
+	for (int w = 1; w < n_workers; ++w) th.emplace_back(worker, w);
+	worker(0);
+	for (auto &t : th) t.join();
+	s->last.total_ms = now_ms() - t0;
+	if (err_seq >= 0) s->err = err_msg;
+	return err_rc;
 }
 
 // One bucket over several GPUs (SURVEY.md 8e: fewer buckets than GPUs).  The bucket's pairs — already sorted by barcode —
@@ -1541,45 +1637,18 @@ static int align_pairs_split(Session *s, const std::vector<Pair> &pairs, const T
 	}
 	cut.push_back(n);
 	const int P = (int)cut.size() - 1;
-	std::vector<int> tickets(P);
-	for (int k = 0; k < P; ++k) tickets[k] = s->new_ticket();
-	for (int k = 0; k < PH_COUNT; ++k) s->gate[k].cap = P;
 	std::vector<char *> texts(P, nullptr);
 	std::vector<size_t> lens(P, 0);
-	std::vector<int> rcs(P, 0);
-	std::vector<std::string> errs(P);
-	std::vector<emab_run_stats_t> sts(P);
-	auto body = [&](int k) {
-		Worker &wk = s->workers[k];
-		emab_ctx_make_current(wk.ctx);
-		wk.n_threads = std::max(1, s->n_threads / P);
-		memset(&sts[k], 0, sizeof sts[k]);
-		try {
-			GatePass gp(s, tickets[k]);
-			gp.to(PH_PARSE);
+	int rc = run_batches<Batch>(s, P, {P, P, P}, std::max(1, s->n_threads / P),
+		[&](int k, Batch &) { return k < P ? 1 : 0; },
+		[&](Worker &wk, Ticket &tk, int k, Batch &b) {
+			tk.to(PH_PARSE);
 			std::vector<Pair> part(pairs.begin() + (ptrdiff_t)cut[k], pairs.begin() + (ptrdiff_t)cut[k + 1]);
-			rcs[k] = process_pairs(s, wk, gp, part, src, &texts[k], &lens[k], sts[k]);
-			if (rcs[k]) errs[k] = wk.err;
-		} catch (const std::bad_alloc &) { rcs[k] = EMAB_ERR_NOMEM; errs[k] = "out of host memory"; s->pass_cloud_turn(tickets[k]); }
-		std::lock_guard<std::mutex> g(s->mu);
-		++s->device_buckets[wk.dev_slot];
-	};
-	std::vector<std::thread> th;
-	for (int k = 1; k < P; ++k) th.emplace_back(body, k);
-	body(0);
-	for (auto &t : th) t.join();
-	memset(&s->last, 0, sizeof s->last);
+			return process_pairs(s, wk, tk, part, src, &b.text, &b.len, b.st);
+		},
+		[&](int k, Batch &b) { texts[k] = b.text; lens[k] = b.len; });
 	size_t total = 0;
-	int rc = 0;
-	for (int k = 0; k < P; ++k) {
-		if (rcs[k] && !rc) { rc = rcs[k]; s->err = errs[k]; }
-		total += lens[k];
-		double *a = &s->last.parse_ms; const double *b = &sts[k].parse_ms;
-		for (int i = 0; i < 16; ++i) a[i] += b[i];
-		int64_t *ai = &s->last.h2d_bytes; const int64_t *bi = &sts[k].h2d_bytes;
-		for (int i = 0; i < 11; ++i) ai[i] += bi[i];
-		s->last.launches += sts[k].launches;
-	}
+	for (size_t l : lens) total += l;
 	char *buf = rc ? nullptr : text_alloc(total + 1);
 	if (!rc && !buf) { rc = EMAB_ERR_NOMEM; s->err = "out of memory"; }
 	size_t at = 0;
@@ -1595,23 +1664,24 @@ static int align_pairs_split(Session *s, const std::vector<Pair> &pairs, const T
 
 int align_special_fastq(Session *s, const char *data, size_t len, char **out, size_t *out_len)
 {
-	s->workers[0].n_threads = s->n_threads;
-	std::string err;
+	Worker &wk = s->workers[0];
+	wk.n_threads = s->n_threads;
 	if (s->replicas.size() > 1 && s->workers.size() > 1) {  // several GPUs, one bucket: split it
 		std::vector<Pair> pairs;
-		int rc = parse_bucket(s, s->n_threads, data, len, pairs, &err);
-		if (rc) { s->err = err; return rc; }
+		int rc = parse_bucket(s, s->n_threads, data, len, pairs, &s->err);
+		if (rc) return rc;
 		TextSrc src;
 		src.base[0] = data; src.len[0] = len;
 		if (pairs.size() >= 2000) return align_pairs_split(s, pairs, src, out, out_len);
-		GatePass gp(s, s->new_ticket());
-		gp.to(PH_PARSE);
-		rc = process_pairs(s, s->workers[0], gp, pairs, src, out, out_len, s->last);
-		if (rc) s->err = s->workers[0].err;
+		Ticket tk(s);
+		tk.to(PH_PARSE);
+		rc = process_pairs(s, wk, tk, pairs, src, out, out_len, s->last);
+		if (rc) s->err = wk.err;
 		return rc;
 	}
-	int rc = run_bucket(s, s->workers[0], s->new_ticket(), data, len, out, out_len, s->last, &err);
-	if (rc) s->err = err;
+	Ticket tk(s);
+	const int rc = run_bucket(s, wk, tk, data, len, out, out_len, s->last);
+	if (rc) s->err = wk.err;
 	return rc;
 }
 
@@ -1630,65 +1700,17 @@ int align_special_fastq_multi(Session *s, int n, const char *const *data, const 
 	if (s->n_threads <= 8) { caps[PH_PARSE] = 2; caps[PH_POST] = 2; }
 	if (const char *e = getenv("EMAB_GATE_CAPS")) sscanf(e, "%d,%d,%d", &caps[0], &caps[1], &caps[2]);  // tuning knob
 	caps[PH_DEVICE] *= (int)s->replicas.size();   // the cap is per GPU
-	for (int k = 0; k < PH_COUNT; ++k) s->gate[k].cap = W > 1 ? std::max(1, std::min(caps[k], W)) : 1;
-	const int cap = W > 1 ? std::max(s->gate[PH_PARSE].cap, s->gate[PH_POST].cap) : 1;
+	const int cap = std::max(1, std::min(std::max(caps[PH_PARSE], caps[PH_POST]), W));   // buckets in one CPU phase at once
 	int per = std::max(1, s->n_threads / cap);
 	if (const char *e = getenv("EMAB_PHASE_THREADS")) per = std::max(1, atoi(e));   // tuning knob: OpenMP threads of one bucket's CPU phase
-	std::vector<int> tickets(n);
-	for (int i = 0; i < n; ++i) { tickets[i] = s->new_ticket(); out[i] = nullptr; out_len[i] = 0; }
-	std::atomic<int> next(0), first_err(0);
-	std::vector<std::string> errs(W);
-	std::vector<emab_run_stats_t> sum(W);
-	for (auto &x : sum) memset(&x, 0, sizeof x);
-	const double t0 = now_ms();
-	auto body = [&](int w) {
-		Worker &wk = s->workers[w];
-		emab_ctx_make_current(wk.ctx);   // worker threads start on device 0
-		wk.n_threads = per;
-		for (;;) {
-			const int i = next.fetch_add(1);
-			if (i >= n) break;
-			emab_run_stats_t st;
-			memset(&st, 0, sizeof st);
-			int rc = 0;
-			try {  // nothing unwinds out of a worker thread: an allocation failure fails this call, not the process
-				rc = first_err.load() ? (GatePass(s, tickets[i]).to(PH_POST), s->take_cloud_base(tickets[i], 0), 0) : run_bucket(s, wk, tickets[i], data[i], len[i], &out[i], &out_len[i], st, &errs[w]);
-			} catch (const std::bad_alloc &) { rc = EMAB_ERR_NOMEM; errs[w] = "out of host memory"; s->pass_cloud_turn(tickets[i]); }
-			catch (const std::exception &e) { rc = EMAB_ERR_ARG; errs[w] = std::string("internal error: ") + e.what(); s->pass_cloud_turn(tickets[i]); }
-			{ std::lock_guard<std::mutex> g(s->mu); ++s->device_buckets[wk.dev_slot]; }
-			if (rc) { int z = 0; first_err.compare_exchange_strong(z, rc); if (errs[w].empty()) errs[w] = "error"; }
-			double *a = &sum[w].parse_ms; const double *b = &st.parse_ms;
-			for (int k = 0; k < 16; ++k) a[k] += b[k];
-			int64_t *ai = &sum[w].h2d_bytes; const int64_t *bi = &st.h2d_bytes;
-			for (int k = 0; k < 11; ++k) ai[k] += bi[k];
-			sum[w].launches += st.launches;
-			sum[w].ext_planned_cells += st.ext_planned_cells; sum[w].ext_unplanned += st.ext_unplanned;
-			sum[w].glob_planned_cells += st.glob_planned_cells; sum[w].glob_unplanned += st.glob_unplanned;
-			sum[w].ms_ext_wave += st.ms_ext_wave; sum[w].ms_glob_wave += st.ms_glob_wave;
-		}
-	};
-	std::vector<std::thread> th;
-	for (int w = 1; w < W; ++w) th.emplace_back(body, w);
-	body(0);
-	for (auto &t : th) t.join();
-	memset(&s->last, 0, sizeof s->last);
-	for (int w = 0; w < W; ++w) {
-		double *a = &s->last.parse_ms; const double *b = &sum[w].parse_ms;
-		for (int k = 0; k < 16; ++k) a[k] += b[k];
-		int64_t *ai = &s->last.h2d_bytes; const int64_t *bi = &sum[w].h2d_bytes;
-		for (int k = 0; k < 11; ++k) ai[k] += bi[k];
-		s->last.launches += sum[w].launches;
-		s->last.ext_planned_cells += sum[w].ext_planned_cells; s->last.ext_unplanned += sum[w].ext_unplanned;
-		s->last.glob_planned_cells += sum[w].glob_planned_cells; s->last.glob_unplanned += sum[w].glob_unplanned;
-		s->last.ms_ext_wave += sum[w].ms_ext_wave; s->last.ms_glob_wave += sum[w].ms_glob_wave;
-	}
-	s->last.total_ms = now_ms() - t0;
-	if (first_err.load()) {
-		for (int w = 0; w < W; ++w) if (!errs[w].empty()) { s->err = errs[w]; break; }
+	for (int i = 0; i < n; ++i) { out[i] = nullptr; out_len[i] = 0; }
+	const int rc = run_batches<Batch>(s, W, caps, per,
+		[&](int i, Batch &) { return i < n ? 1 : 0; },
+		[&](Worker &wk, Ticket &tk, int i, Batch &b) { return run_bucket(s, wk, tk, data[i], len[i], &b.text, &b.len, b.st); },
+		[&](int i, Batch &b) { out[i] = b.text; out_len[i] = b.len; });
+	if (rc)
 		for (int i = 0; i < n; ++i) { text_free(out[i]); out[i] = nullptr; }
-		return first_err.load();
-	}
-	return EMAB_OK;
+	return rc;
 }
 
 // ---- standard FASTQ (src/align.c:632-744, src/techs.c:5-69) -----------------------------------------
@@ -1883,80 +1905,41 @@ int align_fastq_stream(Session *s, emab_read_cb r1, void *u1, emab_read_cb r2, v
 	cut.paired_files = r2 != nullptr;
 	cut.batch_pairs = batch_pairs > 0 ? batch_pairs : 40000;
 	const int W = std::max(1, (int)s->workers.size());
-	int caps[PH_COUNT] = {3, 3, 3};
-	caps[PH_DEVICE] *= (int)s->replicas.size();
-	for (int k = 0; k < PH_COUNT; ++k) s->gate[k].cap = W > 1 ? std::max(1, std::min(caps[k], W)) : 1;
-	const int per = std::max(1, s->n_threads / (W > 1 ? std::min(3, W) : 1));
-	std::mutex cut_mu, out_mu;
+	struct StreamBatch : Batch { std::string t1, t2; };   // the batch's text of each input
+	std::mutex out_mu;
 	std::condition_variable out_cv;
-	int next_seq = 0, write_seq = 0;       // batches are numbered as they are cut and written in that order
-	std::atomic<int> first_err(0);
-	std::string first_msg;
-	memset(&s->last, 0, sizeof s->last);
-	const double t0 = now_ms();
-	auto body = [&](int wi) {
-		Worker &wk = s->workers[wi];
-		emab_ctx_make_current(wk.ctx);
-		wk.n_threads = W > 1 ? per : s->n_threads;
-		for (;;) {
-			std::string t1, t2;
-			int seq, ticket;
-			{
-				std::lock_guard<std::mutex> g(cut_mu);
-				if (first_err.load()) break;
-				const int rc = cut.next(&t1, &t2);
-				if (rc < 0) { int z = 0; if (first_err.compare_exchange_strong(z, rc)) first_msg = cut.err; break; }
-				if (rc == 0) break;
-				seq = next_seq++;
-				ticket = s->new_ticket();
-			}
-			char *text = nullptr;
-			size_t text_len = 0;
-			emab_run_stats_t st;
-			memset(&st, 0, sizeof st);
-			int rc = 0;
-			std::string msg;
-			try {
-				GatePass gp(s, ticket);
-				gp.to(PH_PARSE);
-				std::vector<Pair> pairs;
-				const double tp = now_ms();
-				rc = parse_fastq_pairs(s, t1.data(), t1.size(), cut.paired_files ? t2.data() : nullptr, t2.size(), pairs, &msg);
-				const double tq = now_ms();
-				if (rc) s->pass_cloud_turn(ticket);
-				else {
-					TextSrc src;
-					src.base[0] = t1.data(); src.len[0] = t1.size();
-					if (cut.paired_files) { src.base[1] = t2.data(); src.len[1] = t2.size(); }
-					rc = process_pairs(s, wk, gp, pairs, src, &text, &text_len, st);
-					if (rc) msg = wk.err;
-					st.parse_ms = tq - tp;
-					st.total_ms += tq - tp;
-				}
-			} catch (const std::bad_alloc &) { rc = EMAB_ERR_NOMEM; msg = "out of host memory"; s->pass_cloud_turn(ticket); }
-			if (rc) { int z = 0; if (first_err.compare_exchange_strong(z, rc)) { std::lock_guard<std::mutex> g(out_mu); first_msg = msg; } }
-			{   // deliver in input order
-				std::unique_lock<std::mutex> g(out_mu);
-				out_cv.wait(g, [&] { return write_seq == seq; });
-				if (!rc && !first_err.load() && text_len && w(uw, text, (uint64_t)text_len) != 0) { int z = 0; if (first_err.compare_exchange_strong(z, EMAB_ERR_IO)) first_msg = "error: write failed"; }
-				double *a = &s->last.parse_ms; const double *bb = &st.parse_ms;
-				for (int k = 0; k < 16; ++k) a[k] += bb[k];
-				int64_t *ai = &s->last.h2d_bytes; const int64_t *bi = &st.h2d_bytes;
-				for (int k = 0; k < 11; ++k) ai[k] += bi[k];
-				s->last.launches += st.launches;
-				++write_seq;
-				out_cv.notify_all();
-			}
-			text_free(text);
-		}
-	};
-	std::vector<std::thread> th;
-	for (int wi = 1; wi < W; ++wi) th.emplace_back(body, wi);
-	body(0);
-	for (auto &t : th) t.join();
-	s->last.total_ms = now_ms() - t0;
-	if (first_err.load()) { s->err = first_msg; return first_err.load(); }
-	return EMAB_OK;
+	int write_seq = 0;       // batches are written in input order, none after a failed one
+	bool failed = false;
+	return run_batches<StreamBatch>(s, W, {3, 3, 3 * (int)s->replicas.size()}, std::max(1, s->n_threads / std::min(3, W)),
+		[&](int, StreamBatch &b) {
+			const int rc = cut.next(&b.t1, &b.t2);
+			if (rc < 0) b.err = cut.err;
+			return rc;
+		},
+		[&](Worker &wk, Ticket &tk, int, StreamBatch &b) {
+			tk.to(PH_PARSE);
+			std::vector<Pair> pairs;
+			const double tp = now_ms();
+			int rc = parse_fastq_pairs(s, b.t1.data(), b.t1.size(), cut.paired_files ? b.t2.data() : nullptr, b.t2.size(), pairs, &wk.err);
+			if (rc) return rc;
+			const double tq = now_ms();
+			TextSrc src;
+			src.base[0] = b.t1.data(); src.len[0] = b.t1.size();
+			if (cut.paired_files) { src.base[1] = b.t2.data(); src.len[1] = b.t2.size(); }
+			rc = process_pairs(s, wk, tk, pairs, src, &b.text, &b.len, b.st);
+			b.st.parse_ms = tq - tp;
+			return rc;
+		},
+		[&](int seq, StreamBatch &b) {   // a worker takes no new batch before its text is written: memory stays bounded
+			std::unique_lock<std::mutex> g(out_mu);
+			out_cv.wait(g, [&] { return write_seq == seq; });
+			if (b.rc) failed = true;
+			else if (!failed && b.len && w(uw, b.text, (uint64_t)b.len) != 0) { failed = true; b.rc = EMAB_ERR_IO; b.err = "error: write failed"; }
+			++write_seq;
+			out_cv.notify_all();
+			text_free(b.text);
+			b.text = nullptr;
+		});
 }
 
 // the whole input in memory, the whole SAM text back: the stream above with memory on both ends

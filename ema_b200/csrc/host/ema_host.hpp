@@ -43,7 +43,7 @@ struct PinnedBuf {  // grow-only pinned host buffer (fast H2D path)
 };
 
 // A pipeline phase that admits buckets strictly in ticket order, at most `cap` of them inside at once.
-// Every ticket passes every phase exactly once (GatePass below guarantees it, error paths included), so
+// Every ticket passes every phase exactly once (Ticket below guarantees it, error paths included), so
 // ordered admission cannot deadlock and the in-order hand-out of cloud ids never waits on a later bucket.
 struct PhaseGate {
 	std::mutex mu;
@@ -104,7 +104,7 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 	std::vector<int> device_ids;
 	std::vector<long long> device_buckets; // buckets each replica has processed (reporting)
 	std::string ref_path;
-	std::vector<Worker> workers;          // buckets in flight (-x mode / emab_align_buckets); workers[0] serves single calls
+	std::vector<Worker> workers;          // batches in flight (-x, the -1/-2 stream, a split bucket); workers[0] serves single calls
 	const Platform *tech = nullptr;
 	int bc_len = 16;
 	bool is_haplotag = false;
@@ -134,7 +134,7 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 	PhaseGate gate[PH_COUNT];             // parse+encode | device pipeline | clouds, EM, SAM text
 	OrderedTurn density;                  // -d: bad clouds are optimised bucket by bucket in input order
 	int new_ticket() { std::lock_guard<std::mutex> g(mu); return next_ticket++; }
-	int take_cloud_base(int ticket, int n_clouds)
+	int take_cloud_base(int ticket, int n_clouds)   // only through Ticket, which takes every ticket's turn exactly once
 	{
 		std::unique_lock<std::mutex> g(mu);
 		cv.wait(g, [&] { return cloud_turn == ticket; });
@@ -143,13 +143,6 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 		++cloud_turn;
 		cv.notify_all();
 		return base;
-	}
-	// a ticket that failed before (or after) its turn: make sure the turn is not left waiting for it
-	void pass_cloud_turn(int ticket)
-	{
-		std::unique_lock<std::mutex> g(mu);
-		cv.wait(g, [&] { return cloud_turn >= ticket; });
-		if (cloud_turn == ticket) { ++cloud_turn; cv.notify_all(); }
 	}
 	int output = EMAB_OUTPUT_SAM;         // what the align calls return: SAM text or BGZF members of BAM records
 	// coordinate-sorted BAM (emab_session_sort): every align call's raw records and sort rows, held until session_finish.
@@ -167,25 +160,32 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 	emab_run_stats_t last{};
 };
 
-// One bucket's walk through the phases: to(ph) leaves the current phase and enters ph (phases are visited
-// in increasing order); the destructor walks through whatever is left so that later tickets are admitted.
-struct GatePass {
-	Session *s; int ticket; int cur = -1;
-	GatePass(Session *s_, int t) : s(s_), ticket(t) {}
+// One bucket's ticket, taken at construction in input order.  to(ph) leaves the current phase and enters ph (phases are
+// visited in increasing order); cloud_base(n) takes the bucket's turn at the session's cloud-id counter, once.  Every
+// ticket must take its turn and pass every phase, or later tickets wait forever, so the destructor gives back what the
+// bucket did not use, on every return and exception: first the turn, then the phases not yet walked.  Waiting for the
+// turn inside phase `cur` cannot deadlock: a ticket only waits for earlier tickets, and an earlier ticket never needs a
+// gate slot a later one holds, because gates admit in ticket order (every earlier ticket is already past `cur`'s
+// admission, and no later ticket has entered a phase after `cur`).
+struct Ticket {
+	Session *s; const int id; int cur = -1; bool turn_taken = false;
+	explicit Ticket(Session *s_) : s(s_), id(s_->new_ticket()) {}
 	void to(int ph)
 	{
 		if (cur >= 0) s->gate[cur].leave();
-		for (int k = cur + 1; k < ph; ++k) { s->gate[k].enter(ticket); s->gate[k].leave(); }
-		s->gate[ph].enter(ticket);
+		for (int k = cur + 1; k < ph; ++k) { s->gate[k].enter(id); s->gate[k].leave(); }
+		s->gate[ph].enter(id);
 		cur = ph;
 	}
-	~GatePass()
+	int cloud_base(int n_clouds) { turn_taken = true; return s->take_cloud_base(id, n_clouds); }
+	~Ticket()
 	{
+		if (!turn_taken) s->take_cloud_base(id, 0);
 		if (cur >= 0) s->gate[cur].leave();
-		for (int k = cur + 1; k < PH_COUNT; ++k) { s->gate[k].enter(ticket); s->gate[k].leave(); }
+		for (int k = cur + 1; k < PH_COUNT; ++k) { s->gate[k].enter(id); s->gate[k].leave(); }
 	}
-	GatePass(const GatePass &) = delete;
-	GatePass &operator=(const GatePass &) = delete;
+	Ticket(const Ticket &) = delete;
+	Ticket &operator=(const Ticket &) = delete;
 };
 
 // Output text blocks (what emab_free releases).  Blocks of a megabyte or more are recycled through a small pool:
