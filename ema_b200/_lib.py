@@ -320,7 +320,8 @@ class RunStats(C.Structure):
                                          "local_cells", "occ_touches")] + [("launches", C.c_int32), ("pad", C.c_int32)] + \
                [(n, C.c_int64) for n in ("ext_planned_cells", "ext_unplanned", "glob_planned_cells", "glob_unplanned")] + \
                [("ms_ext_wave", C.c_double), ("ms_glob_wave", C.c_double), ("format_kernel_ms", C.c_double)] + \
-               [(n, C.c_double) for n in ("sort_ms", "gather_ms", "compress_ms", "index_ms")]
+               [(n, C.c_double) for n in ("sort_ms", "gather_ms", "compress_ms", "index_ms")] + \
+               [("spill_files", C.c_int64), ("spill_bytes", C.c_int64), ("spill_ms", C.c_double)]
 
 
 class PinnedText:
@@ -363,16 +364,21 @@ class Session:
     _WRITE_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64)
 
     def __init__(self, ref_path: str, platform: str = "10x", device: int = 0, rg: str | None = None, bx_index: str | None = None,
-                 apply_opt: bool = False, threads: int = 1, output: str = "sam", sort: bool = False, max_host_bytes: int = 0):
+                 apply_opt: bool = False, threads: int = 1, output: str = "sam", sort: bool = False, max_host_bytes: int = 0,
+                 spill: str | None = None):
         """output="bam": header() and every align call return BGZF members of BAM instead of SAM text
         (a BAM file is header, the calls' bytes in order, then bgzf_eof()).
         sort=True (BAM only): align calls return b"" and hold their records (at most max_host_bytes of host memory, 0: no
-        cap); finish() returns them as one coordinate-sorted body and its BAI (file: header, body, bgzf_eof())."""
+        cap); finish() returns them as one coordinate-sorted body and its BAI (file: header, body, bgzf_eof()).
+        spill=PREFIX: with a nonzero max_host_bytes, reaching it writes the held records to PREFIX.*.spill files instead of
+        failing, and finish() merges them (see set_spill)."""
         self._h = C.c_void_p()
         _check(lib().emab_session_open(ref_path.encode(), platform.encode(), device, C.byref(self._h)))
         _check(lib().emab_session_config(self._h, rg.encode() if rg else None, bx_index.encode() if bx_index else None,
                                          int(apply_opt), threads))
         self.set_output(output)
+        if spill:
+            self.set_spill(spill)
         if sort:
             self.set_sort(True, max_host_bytes)
 
@@ -380,6 +386,11 @@ class Session:
         """emab_session_sort: coordinate-sorted BAM for the calls that follow (index=False: no BAI, any contig length)"""
         mode = (self.SORT_COORD if index else self.SORT_COORD_NOINDEX) if on else self.SORT_OFF
         _check(lib().emab_session_sort(self._h, mode, C.c_uint64(max_host_bytes)))
+
+    def set_spill(self, prefix: str | None):
+        """emab_session_sort_spill: the prefix of the temporary files a sorted run spills to when it reaches max_host_bytes
+        (None: no spilling, the cap fails the run).  A session setting that set_sort keeps."""
+        _check(lib().emab_session_sort_spill(self._h, prefix.encode() if prefix else None))
 
     def finish(self) -> tuple[bytes, bytes]:
         """emab_session_finish: (sorted BGZF body without the EOF block, .bai bytes; b"" without an index)"""

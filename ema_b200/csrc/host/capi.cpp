@@ -119,6 +119,15 @@ int emab_session_sort(emab_session_t *h, int on, uint64_t max_host_bytes)
 	});
 }
 
+int emab_session_sort_spill(emab_session_t *h, const char *prefix)
+{
+	return guarded([&]() -> int {
+		if (!h) return fail(EMAB_ERR_ARG, "null session");
+		emab::session_sort_spill(h->s, prefix);
+		return EMAB_OK;
+	});
+}
+
 int emab_session_finish(emab_session_t *h, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len)
 {
 	return guarded([&]() -> int {

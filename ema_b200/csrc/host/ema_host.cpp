@@ -33,6 +33,7 @@
 #include <string_view>
 #include <thread>
 #include <unordered_map>
+#include <unistd.h>
 
 namespace emab {
 
@@ -294,6 +295,13 @@ int session_open(const char *ref_path, const char *platform, int device, Session
 		fclose(f);
 	}
 	s->ref_path = ref_path;
+	{   // names this session's spill files apart from those of other sessions and processes sharing a prefix
+		static std::atomic<unsigned> n_open{0};
+		char tok[64];
+		snprintf(tok, sizeof tok, "%d-%u-%llx", (int)getpid(), n_open++,
+		         (unsigned long long)std::chrono::steady_clock::now().time_since_epoch().count() & 0xffffffffffull);
+		s->spill_token = tok;
+	}
 	int rc = emab_index_load(ref_path, device, &s->ix);
 	if (!rc) { s->replicas.push_back(s->ix); s->device_ids.push_back(device); s->device_buckets.push_back(0); }
 	if (rc) { *err = std::string("error: could not load reference at ") + ref_path + ": " + emab_last_error(); delete s; return rc; }
@@ -318,6 +326,12 @@ int session_open(const char *ref_path, const char *platform, int device, Session
 	return EMAB_OK;
 }
 
+static void remove_spills(Session *s)   // under run_mu
+{
+	for (const std::string &p : s->spills) unlink(p.c_str());
+	s->spills.clear();
+}
+
 void session_close(Session *s)
 {
 	if (!s) return;
@@ -326,6 +340,10 @@ void session_close(Session *s)
 		fprintf(stderr, "[emab host profile] buckets per device:");
 		for (size_t d = 0; d < s->replicas.size(); ++d) fprintf(stderr, " cuda:%d=%lld", s->device_ids[d], s->device_buckets[d]);
 		fprintf(stderr, "\n");
+	}
+	{
+		std::lock_guard<std::mutex> g(s->run_mu);
+		remove_spills(s);
 	}
 	for (Worker &w : s->workers) emab_ctx_free(w.ctx);
 	s->workers.clear();
@@ -383,9 +401,16 @@ static void drop_runs(Session *s)
 {
 	std::lock_guard<std::mutex> g(s->run_mu);
 	s->runs.clear();
+	remove_spills(s);
 	s->sort_held = 0;
 	s->sort_rc = 0;
 	s->sort_err.clear();
+}
+
+void session_sort_spill(Session *s, const char *prefix)
+{
+	std::lock_guard<std::mutex> g(s->run_mu);
+	s->spill_prefix = prefix ? prefix : "";
 }
 
 int session_sort(Session *s, int on, uint64_t max_host_bytes)
@@ -408,13 +433,17 @@ int session_sort(Session *s, int on, uint64_t max_host_bytes)
 void sort_call_failed(Session *s, int rc)
 {
 	std::lock_guard<std::mutex> g(s->run_mu);
-	if (s->sort == EMAB_SORT_OFF || s->sort_rc) return;
+	if (s->sort == EMAB_SORT_OFF) return;
+	remove_spills(s);
+	if (s->sort_rc) return;
 	s->sort_rc = rc;
 	s->sort_err = "error: an align call of this sorted run failed (" + s->err + "), so the run cannot be written";
 }
 
-// a sorted call's records and rows join the run under its ticket, unless that takes the bytes held over the cap
-static int hold_run(Session *s, Worker &wk, int ticket, const char *raw, size_t len, std::vector<emab_bam_key_t> &&keys)
+// a sorted call's records and rows join the run under its ticket, unless that takes the bytes held over the cap: then, with
+// a spill prefix, every held run and this one move to *spill (the caller writes them out) and the count starts again
+static int hold_run(Session *s, Worker &wk, int ticket, const char *raw, size_t len, std::vector<emab_bam_key_t> &&keys,
+                    std::map<int, Session::SortRun> *spill)
 {
 	const uint64_t bytes = len + keys.size() * sizeof(emab_bam_key_t);
 	Session::SortRun r;
@@ -422,6 +451,12 @@ static int hold_run(Session *s, Worker &wk, int ticket, const char *raw, size_t 
 	memcpy(r.raw.get(), raw, len);
 	r.keys = std::move(keys);
 	std::lock_guard<std::mutex> g(s->run_mu);
+	if (s->sort_cap && s->sort_held + bytes > s->sort_cap && !s->spill_prefix.empty()) {
+		spill->swap(s->runs);
+		(*spill)[ticket] = std::move(r);
+		s->sort_held = 0;
+		return EMAB_OK;
+	}
 	if (s->sort_cap && s->sort_held + bytes > s->sort_cap) {
 		wk.err = "error: the sorted run needs more than the " + std::to_string(s->sort_cap) + " bytes of host memory it may hold (" +
 		         std::to_string(s->sort_held + bytes) + " so far); nothing is written";
@@ -431,6 +466,53 @@ static int hold_run(Session *s, Worker &wk, int ticket, const char *raw, size_t 
 	s->sort_held += bytes;
 	s->runs[ticket] = std::move(r);
 	return EMAB_OK;
+}
+
+// runs taken by hold_run, sorted on this worker's device and written to the run's next spill files, each holding at most
+// the cap's bytes (a call's run larger than the cap is cut into pieces of whole records)
+static int spill_runs(Session *s, Worker &wk, std::map<int, Session::SortRun> &runs, emab_run_stats_t &st)
+{
+	const double t0 = now_ms();
+	std::vector<emab_bam_run_t> rv;
+	std::vector<uint64_t> seq0;
+	uint64_t held = 0;
+	auto flush = [&]() -> int {
+		if (rv.empty()) return EMAB_OK;
+		std::string path;
+		{
+			std::lock_guard<std::mutex> g(s->run_mu);
+			path = s->spill_prefix + "." + s->spill_token + "." + std::to_string(s->spill_seq++) + ".spill";
+		}
+		uint64_t bytes = 0;
+		const int rc = emab_bam_spill(wk.ctx, (int)rv.size(), rv.data(), seq0.data(), path.c_str(), &bytes);
+		rv.clear(); seq0.clear(); held = 0;
+		if (rc) { wk.err = emab_last_error(); return rc; }
+		std::lock_guard<std::mutex> g(s->run_mu);
+		s->spills.push_back(path);
+		st.spill_files += 1;
+		st.spill_bytes += (int64_t)bytes;
+		return EMAB_OK;
+	};
+	for (auto &kv : runs) {
+		const std::vector<emab_bam_key_t> &k = kv.second.keys;
+		const char *raw = kv.second.raw.get();
+		for (size_t i = 0; i < k.size();) {
+			size_t e = i;
+			uint64_t b = 0;
+			while (e < k.size() && (e == i || held + b + k[e].len + sizeof(emab_bam_key_t) <= s->sort_cap)) b += k[e++].len + sizeof(emab_bam_key_t);
+			if (e == i + 1 && held && held + b > s->sort_cap) { const int rc = flush(); if (rc) return rc; continue; }
+			rv.push_back({raw, k.data() + i, (uint64_t)(e - i)});
+			seq0.push_back((uint64_t)kv.first << 32 | i);
+			for (size_t j = i; j < e; ++j) raw += k[j].len;
+			held += b;
+			i = e;
+			if (e < k.size()) { const int rc = flush(); if (rc) return rc; }
+		}
+	}
+	const int rc = flush();
+	runs.clear();
+	st.spill_ms += now_ms() - t0;
+	return rc;
 }
 
 int session_finish(Session *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len)
@@ -447,8 +529,18 @@ int session_finish(Session *s, emab_write_cb w, void *uw, char **bai, uint64_t *
 	auto counted = [](void *u, const char *p, uint64_t n) -> int { Count *c = (Count *)u; c->n += n; return c->w(c->uw, p, n); };
 	double ms[4] = {0, 0, 0, 0};
 	emab_ctx_t *ctx = s->workers[0].ctx;
-	const int rc = emab_bam_sort(ctx, (int)rv.size(), rv.data(), (int)s->sq_names.size(), s->header_bytes, slice, counted, &cnt,
-	                             s->sort == EMAB_SORT_COORD ? bai : nullptr, bai_len, ms);
+	int rc;
+	if (s->spills.empty()) {
+		rc = emab_bam_sort(ctx, (int)rv.size(), rv.data(), (int)s->sq_names.size(), s->header_bytes, slice, counted, &cnt,
+		                   s->sort == EMAB_SORT_COORD ? bai : nullptr, bai_len, ms);
+	} else {   // spilled runs: merged with what is still held, in windows bounded by the cap
+		std::vector<const char *> paths;
+		for (const std::string &p : s->spills) paths.push_back(p.c_str());
+		std::vector<uint64_t> seq0;
+		for (auto &kv : s->runs) seq0.push_back((uint64_t)kv.first << 32);
+		rc = emab_bam_merge(ctx, (int)paths.size(), paths.data(), (int)rv.size(), rv.data(), seq0.data(), (int)s->sq_names.size(), s->sq_len.data(),
+		                    s->header_bytes, slice, s->sort_cap, counted, &cnt, s->sort == EMAB_SORT_COORD ? bai : nullptr, bai_len, ms);
+	}
 	if (rc) s->err = emab_last_error();
 	drop_runs(s);
 	memset(&s->last, 0, sizeof s->last);
@@ -1306,9 +1398,15 @@ static int process_pairs(Session *s, Worker &wk, Ticket &tk, const std::vector<P
 		       : bam ? emab_bam_format(wk.ctx, &job, buf, (uint64_t)cap, &total) : emab_sam_format(wk.ctx, &job, buf, (uint64_t)cap, &total);
 		if (rc) { wk.err = emab_last_error(); text_free(buf); return rc; }
 		if (sorted) {   // the records wait for session_finish; the call itself returns nothing
-			rc = hold_run(s, wk, tk.id, buf, (size_t)total, std::move(keys));
+			std::map<int, Session::SortRun> spill;
+			rc = hold_run(s, wk, tk.id, buf, (size_t)total, std::move(keys), &spill);
 			text_free(buf);
-			buf = text_alloc(1);
+			buf = nullptr;
+			if (!rc && !spill.empty()) {   // outside every gate and cloud turn: later batches go on while the file is written
+				tk.release();
+				rc = spill_runs(s, wk, spill, st);
+			}
+			if (!rc) buf = text_alloc(1);
 			if (rc || !buf) { text_free(buf); if (!rc) wk.err = "out of memory"; return rc ? rc : EMAB_ERR_NOMEM; }
 			st.d2h_bytes += (int64_t)total + (int64_t)n_out * (int64_t)sizeof(emab_bam_key_t);
 			total = 0;
@@ -1526,7 +1624,7 @@ static int run_bucket(Session *s, Worker &wk, Ticket &tk, const char *data, size
 // set, not summed.  A field added to emab_run_stats_t fails the size check until it is summed here or named above.
 static void add_stats(emab_run_stats_t &into, const emab_run_stats_t &from)
 {
-	static_assert(sizeof(emab_run_stats_t) == 312, "emab_run_stats_t changed: sum the new field in add_stats");
+	static_assert(sizeof(emab_run_stats_t) == 336, "emab_run_stats_t changed: sum the new field in add_stats");
 	into.parse_ms += from.parse_ms; into.encode_ms += from.encode_ms; into.align_ms += from.align_ms; into.kernel_ms += from.kernel_ms;
 	into.cloud_ms += from.cloud_ms; into.flatten_ms += from.flatten_ms; into.em_ms += from.em_ms; into.em_kernel_ms += from.em_kernel_ms;
 	into.format_ms += from.format_ms; into.format_kernel_ms += from.format_kernel_ms; into.gate_wait_ms += from.gate_wait_ms;
@@ -1539,6 +1637,7 @@ static void add_stats(emab_run_stats_t &into, const emab_run_stats_t &from)
 	into.occ_touches += from.occ_touches;
 	into.ext_planned_cells += from.ext_planned_cells; into.ext_unplanned += from.ext_unplanned;
 	into.glob_planned_cells += from.glob_planned_cells; into.glob_unplanned += from.glob_unplanned;
+	into.spill_files += from.spill_files; into.spill_bytes += from.spill_bytes; into.spill_ms += from.spill_ms;
 }
 
 // One batch of a run_batches call: its output, its stats and, when it failed, why.

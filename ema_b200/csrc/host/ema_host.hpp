@@ -152,6 +152,11 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 	uint64_t sort_cap = 0, sort_held = 0;  // cap on the bytes held (0: none), bytes held
 	std::map<int, SortRun> runs;
 	std::mutex run_mu;
+	// spilling (emab_session_sort_spill): with a prefix and a cap, the held runs go to PREFIX.<spill_token>.<n>.spill files
+	// instead of failing; finish merges them with what is still held
+	std::string spill_prefix, spill_token;
+	std::vector<std::string> spills;      // the files of this run (under run_mu)
+	int spill_seq = 0;
 	int sort_rc = 0;                      // a call of this run failed: finish refuses with this code and message
 	std::string sort_err;
 	uint64_t header_bytes = 0;            // size of the BGZF header emab_sam_header returned last (where the body starts)
@@ -169,6 +174,7 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 // admission, and no later ticket has entered a phase after `cur`).
 struct Ticket {
 	Session *s; const int id; int cur = -1; bool turn_taken = false;
+	bool released = false;
 	explicit Ticket(Session *s_) : s(s_), id(s_->new_ticket()) {}
 	void to(int ph)
 	{
@@ -178,12 +184,16 @@ struct Ticket {
 		cur = ph;
 	}
 	int cloud_base(int n_clouds) { turn_taken = true; return s->take_cloud_base(id, n_clouds); }
-	~Ticket()
+	// gives back the turn and the phases now, so that work after it (a spill) holds up no later ticket
+	void release()
 	{
+		if (released) return;
+		released = true;
 		if (!turn_taken) s->take_cloud_base(id, 0);
 		if (cur >= 0) s->gate[cur].leave();
 		for (int k = cur + 1; k < PH_COUNT; ++k) { s->gate[k].enter(id); s->gate[k].leave(); }
 	}
+	~Ticket() { release(); }
 	Ticket(const Ticket &) = delete;
 	Ticket &operator=(const Ticket &) = delete;
 };
@@ -203,6 +213,7 @@ void sam_header(const Session *s, int argc, const char *const *argv, std::string
 void bam_header(const Session *s, const std::string &text, std::string *out);
 int session_output(Session *s, int format);   // EMAB_OUTPUT_SAM / EMAB_OUTPUT_BAM
 int session_sort(Session *s, int on, uint64_t max_host_bytes);   // EMAB_SORT_*
+void session_sort_spill(Session *s, const char *prefix);         // nullptr: no spilling
 // the held runs as one coordinate-sorted BGZF body to w, and its BAI (EMAB_SORT_COORD, bai != nullptr); releases the runs
 int session_finish(Session *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len);
 void sort_call_failed(Session *s, int rc);    // an align call failed in sorted mode: the run cannot be finished

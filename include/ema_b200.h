@@ -285,6 +285,21 @@ typedef struct {
 typedef int (*emab_write_cb)(void *user, const char *text, uint64_t len);
 int emab_bam_sort(emab_ctx_t *ctx, int n_runs, const emab_bam_run_t *runs, int n_ref, uint64_t body_offset, int slice_chunks,
                   emab_write_cb w, void *uw, char **bai, uint64_t *bai_len, double ms[4]);
+/* emab_bam_spill = the runs in the order emab_bam_sort gives them, written to a new file at `path` (created with O_EXCL):
+ *                    a 24-byte header ("EMABSPL1", records, record bytes), one 32-byte row per record (the emab_bam_key_t,
+ *                    then its input position seq0[r] + the record's index in run r), then the raw records, all in that
+ *                    order and uncompressed.  *file_bytes receives the file's size.  A failed create or write removes the
+ *                    file and returns EMAB_ERR_IO with a message naming the path.
+ * emab_bam_merge = emab_bam_sort over spill files and runs still in memory (seq0 as above), for runs larger than host
+ *                    memory: the same bytes as emab_bam_sort over all the records in input order.  It works in windows: a
+ *                    block of about budget / (2 (runs + 1)) bytes (at least one record) is read from each run, the device
+ *                    takes every row up to the smallest last (key, input position) of the blocks that continue, orders
+ *                    them and appends them to the body and the index.  ref_len[n_ref] (the @SQ lengths) sizes the linear
+ *                    index.  ms[0] is the time of the device ordering; ms[1] includes reading the blocks. */
+int emab_bam_spill(emab_ctx_t *ctx, int n_runs, const emab_bam_run_t *runs, const uint64_t *seq0, const char *path, uint64_t *file_bytes);
+int emab_bam_merge(emab_ctx_t *ctx, int n_files, const char *const *paths, int n_runs, const emab_bam_run_t *runs, const uint64_t *seq0,
+                   int n_ref, const int32_t *ref_len, uint64_t body_offset, int slice_chunks, uint64_t budget,
+                   emab_write_cb w, void *uw, char **bai, uint64_t *bai_len, double ms[4]);
 int emab_bgzf_compress(emab_ctx_t *ctx, const uint8_t *in, uint64_t len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
 int emab_bgzf_eof(const uint8_t **p, uint64_t *len);
 /* pinned host memory for callers that want their input buffers to take the fast H2D path */
@@ -357,6 +372,9 @@ typedef struct {
 	/* emab_session_finish (sorted BAM): wall time of the device sort, the host gather, the compression (slices to the device,
 	 * BGZF kernels, members back and written) and the index build */
 	double sort_ms, gather_ms, compress_ms, index_ms;
+	/* sorted BAM with a spill prefix: the spill files this align call wrote, their bytes and the wall time spent on them */
+	int64_t spill_files, spill_bytes;
+	double spill_ms;
 } emab_run_stats_t;
 
 int emab_session_open(const char *ref_path, const char *platform, int device, emab_session_t **out);
@@ -370,9 +388,16 @@ int emab_session_output(emab_session_t *s, int format);
  *                        samtools' coordinate key (stable: equal keys keep input order, unplaced records last) and returns
  *                        its BAI.  Refused when a contig is longer than 2^29 - 1 bp, which a BAI cannot index.
  *   EMAB_SORT_COORD_NOINDEX  the same without the index (any contig length)
- * max_host_bytes caps the bytes held (raw records + 24 bytes per record; 0: no cap): the align call that would go over it
- * fails with EMAB_ERR_OVERFLOW, and so does emab_session_finish after it, which then writes nothing.  Runs are not spilled
- * to disk.  emab_sam_header says SO:coordinate in sorted mode.
+ * max_host_bytes caps the bytes held (raw records + 24 bytes per record; 0: no cap): without a spill prefix, the align call
+ * that would go over it fails with EMAB_ERR_OVERFLOW, and so does emab_session_finish after it, which then writes nothing.
+ * With a spill prefix (emab_session_sort_spill) and a nonzero cap, that call instead takes every held run and its own,
+ * sorts them on its device and writes them to PREFIX.<session token>.<n>.spill (created with O_EXCL, raw and uncompressed;
+ * emab_bam_spill); later calls start holding again while the file is written, so the run holds at most about twice the
+ * cap in host memory.  emab_session_finish then merges the files and the held remainder on the device in windows bounded
+ * by the cap (emab_bam_merge) into the same bytes, body and index, as without spilling.  The files are removed after
+ * finish, when an align call of the run fails, on emab_session_sort and on emab_session_close.  A spill file that cannot
+ * be created or written fails the align call with EMAB_ERR_IO naming the path, and finish then refuses the run.
+ * emab_sam_header says SO:coordinate in sorted mode.
  * emab_session_finish(s, w, uw, bai, bai_len): the sorted BGZF body to w (without the EOF block) and, in EMAB_SORT_COORD,
  * the .bai in a buffer released with emab_free (bai may be NULL to skip it).  The index's file offsets count the bytes of
  * the header emab_sam_header returned last.  The held records are released; later calls start a new run. */
@@ -380,6 +405,9 @@ int emab_session_output(emab_session_t *s, int format);
 #define EMAB_SORT_COORD 1
 #define EMAB_SORT_COORD_NOINDEX 2
 int emab_session_sort(emab_session_t *s, int on, uint64_t max_host_bytes);
+/* the spill prefix of sorted runs (NULL: no spilling).  A session setting: it may be set while sorting is off or between
+ * runs, and emab_session_sort keeps it. */
+int emab_session_sort_spill(emab_session_t *s, const char *prefix);
 int emab_session_finish(emab_session_t *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len);
 int emab_sam_header(emab_session_t *s, int argc, const char *const *argv, char **text, uint64_t *len);
 int emab_align_bucket(emab_session_t *s, const char *data, uint64_t len, char **sam, uint64_t *sam_len);
