@@ -277,8 +277,6 @@ extern "C" void emab_ctx_free(emab_ctx_t *c)
 {
 	if (!c) return;
 	cudaSetDevice(c->device);
-	for (auto &b : c->b) b.release();
-	for (auto &b : c->h) b.release();
 	cudaFree(c->d_counters);
 	cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1); if (c->ev_wait) cudaEventDestroy(c->ev_wait);
 	if (c->stream2) { cudaStreamDestroy(c->stream2); cudaEventDestroy(c->ev_fork); cudaEventDestroy(c->ev_join); }
@@ -473,12 +471,20 @@ static int check_lengths(int n, const int64_t *qoff, const int64_t *toff, int ma
 
 static int sw_grid(emab_ctx *c) { return c->n_sm * 4; }
 
-static int upload_sw_inputs(emab_ctx *c, int n, const uint8_t *q, const int64_t *qoff, const uint8_t *t, const int64_t *toff)
+// The device side of a kernel-level SW batch: queries, targets and their offsets, the per-task argument (h0 or band), the
+// results, and the task order of the thread-per-task kernel.
+struct SwBufs { DevBuf &q, &qoff, &t, &toff, &arg, &out, &order; };
+// the batch calls borrow the pipeline's buffers, dead between calls
+static SwBufs sw_scratch(emab_ctx *c) { return {c->reads, c->read_off, c->intv, c->n_intv, c->seed_lanes, c->occ, c->w_nodes}; }
+// emab_extend_resident_load's, held for emab_extend_resident_run
+static SwBufs sw_resident(emab_ctx *c) { return {c->res_q, c->res_qoff, c->res_t, c->res_toff, c->res_h0, c->res_out, c->res_order}; }
+
+static int upload_sw_inputs(emab_ctx *c, const SwBufs &B, int n, const uint8_t *q, const int64_t *qoff, const uint8_t *t, const int64_t *toff)
 {
-	TRY(upload(c, c->b[0], q, (size_t)qoff[n]));
-	TRY(upload(c, c->b[1], qoff, (size_t)(n + 1) * 8));
-	TRY(upload(c, c->b[2], t, (size_t)toff[n]));
-	TRY(upload(c, c->b[3], toff, (size_t)(n + 1) * 8));
+	TRY(upload(c, B.q, q, (size_t)qoff[n]));
+	TRY(upload(c, B.qoff, qoff, (size_t)(n + 1) * 8));
+	TRY(upload(c, B.t, t, (size_t)toff[n]));
+	TRY(upload(c, B.toff, toff, (size_t)(n + 1) * 8));
 	return EMAB_OK;
 }
 
@@ -492,7 +498,7 @@ extern "C" int emab_set_sw_mode(emab_ctx_t *c, int mode)
 }
 
 // size-sorted task order (similar tasks share a warp: rows advance together) + the widest query
-static int prepare_lanes(emab_ctx *c, int n, const int64_t *qoff, const int64_t *toff, const int32_t *h0, int *qcap)
+static int prepare_lanes(emab_ctx *c, DevBuf &d_order, int n, const int64_t *qoff, const int64_t *toff, const int32_t *h0, int *qcap)
 {
 	std::vector<int32_t> order(n);
 	std::vector<uint64_t> key(n);
@@ -505,13 +511,13 @@ static int prepare_lanes(emab_ctx *c, int n, const int64_t *qoff, const int64_t 
 		order[i] = i;
 	}
 	std::sort(order.begin(), order.end(), [&](int a, int b) { return key[a] != key[b] ? key[a] > key[b] : a < b; });
-	TRY(upload(c, c->b[9], order.data(), (size_t)n * 4));
+	TRY(upload(c, d_order, order.data(), (size_t)n * 4));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));  // `order` is a local
 	*qcap = qmax;
 	return EMAB_OK;
 }
 
-static int launch_extend_lanes(emab_ctx *c, int n, int qcap, int w, int end_bonus, int zdrop)
+static int launch_extend_lanes(emab_ctx *c, const SwBufs &B, int n, int qcap, int w, int end_bonus, int zdrop)
 {
 	const size_t smem = lanes::smem_per_warp(qcap);
 	static size_t configured = 0;
@@ -524,8 +530,8 @@ static int launch_extend_lanes(emab_ctx *c, int n, int qcap, int w, int end_bonu
 	int grid = c->n_sm * per_sm;
 	const int need = (n + 31) / 32;
 	if (grid > need) grid = need;
-	k_extend_lanes<<<grid, 32, smem, c->stream>>>(n, c->b[9].as<int32_t>(), c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<uint8_t>(),
-	                                              c->b[3].as<int64_t>(), c->b[4].as<int32_t>(), w, end_bonus, zdrop, c->b[5].as<int32_t>(), c->d_counters, qcap);
+	k_extend_lanes<<<grid, 32, smem, c->stream>>>(n, B.order.as<int32_t>(), B.q.as<uint8_t>(), B.qoff.as<int64_t>(), B.t.as<uint8_t>(),
+	                                              B.toff.as<int64_t>(), B.arg.as<int32_t>(), w, end_bonus, zdrop, B.out.as<int32_t>(), c->d_counters, qcap);
 	return EMAB_OK;
 }
 
@@ -537,20 +543,21 @@ extern "C" int emab_extend_batch(emab_ctx_t *c, int n, const uint8_t *q, const i
 	if (n == 0) { if (cells) *cells = 0; return EMAB_OK; }
 	TRY(check_lengths(n, qoff, toff, 0));
 	for (int i = 0; i < n; ++i) if (h0[i] <= 0) { snprintf(emab_errbuf, sizeof emab_errbuf, "task %d: h0 must be > 0 (bwa/ksw.c:421)", i); return EMAB_ERR_ARG; }
-	TRY(upload_sw_inputs(c, n, q, qoff, t, toff));
-	TRY(upload(c, c->b[4], h0, (size_t)n * 4));
-	TRY(c->b[5].ensure((size_t)n * 24));
+	const SwBufs B = sw_scratch(c);
+	TRY(upload_sw_inputs(c, B, n, q, qoff, t, toff));
+	TRY(upload(c, B.arg, h0, (size_t)n * 4));
+	TRY(B.out.ensure((size_t)n * 24));
 	CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 64, c->stream));
 	int qcap = 0;
-	if (c->sw_mode != 1) TRY(prepare_lanes(c, n, qoff, toff, h0, &qcap));
+	if (c->sw_mode != 1) TRY(prepare_lanes(c, B.order, n, qoff, toff, h0, &qcap));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
-	if (c->sw_mode != 1) TRY(launch_extend_lanes(c, n, qcap, w, end_bonus, zdrop));
+	if (c->sw_mode != 1) TRY(launch_extend_lanes(c, B, n, qcap, w, end_bonus, zdrop));
 	else
-	k_extend_batch<<<sw_grid(c), SW_WARPS * 32, 0, c->stream>>>(n, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<uint8_t>(), c->b[3].as<int64_t>(),
-	                                                             c->b[4].as<int32_t>(), w, end_bonus, zdrop, c->b[5].as<int32_t>(), c->d_counters);
+	k_extend_batch<<<sw_grid(c), SW_WARPS * 32, 0, c->stream>>>(n, B.q.as<uint8_t>(), B.qoff.as<int64_t>(), B.t.as<uint8_t>(), B.toff.as<int64_t>(),
+	                                                             B.arg.as<int32_t>(), w, end_bonus, zdrop, B.out.as<int32_t>(), c->d_counters);
 	c->last_launches = 1;
 	CUDA_TRY(cudaEventRecord(c->ev1, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[5].p, (size_t)n * 24, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(out, B.out.p, (size_t)n * 24, cudaMemcpyDeviceToHost, c->stream));
 	unsigned long long cnt[2];
 	CUDA_TRY(cudaMemcpyAsync(cnt, c->d_counters, 16, cudaMemcpyDeviceToHost, c->stream));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -565,10 +572,12 @@ extern "C" int emab_extend_resident_load(emab_ctx_t *c, int n, const uint8_t *q,
 	CTX_ENTER(c);
 	if (!c || n <= 0) return EMAB_ERR_ARG;
 	TRY(check_lengths(n, qoff, toff, 0));
-	TRY(upload_sw_inputs(c, n, q, qoff, t, toff));
-	TRY(upload(c, c->b[4], h0, (size_t)n * 4));
-	TRY(c->b[5].ensure((size_t)n * 24));
-	TRY(prepare_lanes(c, n, qoff, toff, h0, &c->res_qcap));
+	c->res_n = 0;
+	const SwBufs B = sw_resident(c);
+	TRY(upload_sw_inputs(c, B, n, q, qoff, t, toff));
+	TRY(upload(c, B.arg, h0, (size_t)n * 4));
+	TRY(B.out.ensure((size_t)n * 24));
+	TRY(prepare_lanes(c, B.order, n, qoff, toff, h0, &c->res_qcap));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));
 	c->res_n = n;
 	return EMAB_OK;
@@ -579,18 +588,19 @@ extern "C" int emab_extend_resident_run(emab_ctx_t *c, int w, int end_bonus, int
 	CTX_ENTER(c);
 	if (!c || c->res_n <= 0 || reps <= 0) return EMAB_ERR_ARG;
 	const int n = c->res_n;
+	const SwBufs B = sw_resident(c);
 	CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 64, c->stream));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
 	for (int r = 0; r < reps; ++r) {
 		CUDA_TRY(cudaMemsetAsync(c->d_counters + 1, 0, 8, c->stream));
-		if (c->sw_mode != 1) TRY(launch_extend_lanes(c, n, c->res_qcap, w, end_bonus, zdrop));
+		if (c->sw_mode != 1) TRY(launch_extend_lanes(c, B, n, c->res_qcap, w, end_bonus, zdrop));
 		else
-		k_extend_batch<<<sw_grid(c), SW_WARPS * 32, 0, c->stream>>>(n, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<uint8_t>(), c->b[3].as<int64_t>(),
-		                                                             c->b[4].as<int32_t>(), w, end_bonus, zdrop, c->b[5].as<int32_t>(), c->d_counters);
+		k_extend_batch<<<sw_grid(c), SW_WARPS * 32, 0, c->stream>>>(n, B.q.as<uint8_t>(), B.qoff.as<int64_t>(), B.t.as<uint8_t>(), B.toff.as<int64_t>(),
+		                                                             B.arg.as<int32_t>(), w, end_bonus, zdrop, B.out.as<int32_t>(), c->d_counters);
 	}
 	c->last_launches = reps;
 	TRY(finish_timed(c));
-	if (out) CUDA_TRY(cudaMemcpy(out, c->b[5].p, (size_t)n * 24, cudaMemcpyDeviceToHost));
+	if (out) CUDA_TRY(cudaMemcpy(out, B.out.p, (size_t)n * 24, cudaMemcpyDeviceToHost));
 	unsigned long long cnt = 0;
 	CUDA_TRY(cudaMemcpy(&cnt, c->d_counters, 8, cudaMemcpyDeviceToHost));
 	if (cells) *cells = (int64_t)(cnt / (unsigned long long)reps);
@@ -614,22 +624,24 @@ extern "C" int emab_global_batch(emab_ctx_t *c, int n, const uint8_t *q, const i
 	}
 	z_stride = (z_stride + 15) & ~(size_t)15;
 	const int grid = sw_grid(c), n_warps = grid * SW_WARPS;
-	TRY(upload_sw_inputs(c, n, q, qoff, t, toff));
-	TRY(upload(c, c->b[4], w, (size_t)n * 4));
-	TRY(c->b[5].ensure((size_t)n * 8));
-	TRY(c->b[6].ensure((size_t)n * max_cigar * 4));
-	TRY(c->b[7].ensure((size_t)n_warps * z_stride));
-	TRY(c->b[8].ensure((size_t)n_warps * max_cigar * 4));
+	const SwBufs B = sw_scratch(c);
+	DevBuf &cigar_buf = c->cub_tmp, &z_buf = c->w_seeds, &tmp_buf = c->w_chains;   // the pipeline's, dead between calls
+	TRY(upload_sw_inputs(c, B, n, q, qoff, t, toff));
+	TRY(upload(c, B.arg, w, (size_t)n * 4));
+	TRY(B.out.ensure((size_t)n * 8));
+	TRY(cigar_buf.ensure((size_t)n * max_cigar * 4));
+	TRY(z_buf.ensure((size_t)n_warps * z_stride));
+	TRY(tmp_buf.ensure((size_t)n_warps * max_cigar * 4));
 	CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 64, c->stream));
-	CUDA_TRY(cudaMemsetAsync(c->b[6].p, 0, (size_t)n * max_cigar * 4, c->stream));
+	CUDA_TRY(cudaMemsetAsync(cigar_buf.p, 0, (size_t)n * max_cigar * 4, c->stream));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
-	k_global_batch<<<grid, SW_WARPS * 32, 0, c->stream>>>(n, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<uint8_t>(), c->b[3].as<int64_t>(),
-	                                                       c->b[4].as<int32_t>(), c->b[5].as<int32_t>(), c->b[6].as<uint32_t>(), max_cigar,
-	                                                       c->b[7].as<uint8_t>(), z_stride, c->b[8].as<uint32_t>(), c->d_counters);
+	k_global_batch<<<grid, SW_WARPS * 32, 0, c->stream>>>(n, B.q.as<uint8_t>(), B.qoff.as<int64_t>(), B.t.as<uint8_t>(), B.toff.as<int64_t>(),
+	                                                       B.arg.as<int32_t>(), B.out.as<int32_t>(), cigar_buf.as<uint32_t>(), max_cigar,
+	                                                       z_buf.as<uint8_t>(), z_stride, tmp_buf.as<uint32_t>(), c->d_counters);
 	c->last_launches = 1;
 	CUDA_TRY(cudaEventRecord(c->ev1, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[5].p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(cigar, c->b[6].p, (size_t)n * max_cigar * 4, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(out, B.out.p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(cigar, cigar_buf.p, (size_t)n * max_cigar * 4, cudaMemcpyDeviceToHost, c->stream));
 	unsigned long long cnt[2];
 	CUDA_TRY(cudaMemcpyAsync(cnt, c->d_counters, 16, cudaMemcpyDeviceToHost, c->stream));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -646,15 +658,16 @@ extern "C" int emab_local_batch(emab_ctx_t *c, int n, const uint8_t *q, const in
 	if (!c || n < 0) return EMAB_ERR_ARG;
 	if (n == 0) { if (cells) *cells = 0; return EMAB_OK; }
 	TRY(check_lengths(n, qoff, toff, KSW_MAX_TLEN));
-	TRY(upload_sw_inputs(c, n, q, qoff, t, toff));
-	TRY(c->b[5].ensure((size_t)n * 28));
+	const SwBufs B = sw_scratch(c);
+	TRY(upload_sw_inputs(c, B, n, q, qoff, t, toff));
+	TRY(B.out.ensure((size_t)n * 28));
 	CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 64, c->stream));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
-	k_local_batch<<<sw_grid(c), SW_WARPS * 32, 0, c->stream>>>(n, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<uint8_t>(), c->b[3].as<int64_t>(),
-	                                                            c->b[5].as<int32_t>(), c->d_counters);
+	k_local_batch<<<sw_grid(c), SW_WARPS * 32, 0, c->stream>>>(n, B.q.as<uint8_t>(), B.qoff.as<int64_t>(), B.t.as<uint8_t>(), B.toff.as<int64_t>(),
+	                                                            B.out.as<int32_t>(), c->d_counters);
 	c->last_launches = 1;
 	CUDA_TRY(cudaEventRecord(c->ev1, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[5].p, (size_t)n * 28, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(out, B.out.p, (size_t)n * 28, cudaMemcpyDeviceToHost, c->stream));
 	unsigned long long cnt[2];
 	CUDA_TRY(cudaMemcpyAsync(cnt, c->d_counters, 16, cudaMemcpyDeviceToHost, c->stream));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));
@@ -681,13 +694,14 @@ extern "C" int emab_sa_batch(emab_ctx_t *c, int n, const int64_t *k, int64_t *ou
 	if (!c || !c->ix || n < 0) return EMAB_ERR_ARG;
 	if (n == 0) return EMAB_OK;
 	for (int i = 0; i < n; ++i) if (k[i] < 0 || (uint64_t)k[i] > c->ix->d.seq_len) { snprintf(emab_errbuf, sizeof emab_errbuf, "SA index out of range"); return EMAB_ERR_ARG; }
-	TRY(upload(c, c->b[0], k, (size_t)n * 8));
-	TRY(c->b[1].ensure((size_t)n * 8));
+	DevBuf &k_buf = c->reads, &out_buf = c->read_off;   // the pipeline's, dead between calls
+	TRY(upload(c, k_buf, k, (size_t)n * 8));
+	TRY(out_buf.ensure((size_t)n * 8));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
-	k_sa_batch<<<(n + 255) / 256, 256, 0, c->stream>>>(c->ix->d, n, c->b[0].as<int64_t>(), c->b[1].as<int64_t>(), mode);
+	k_sa_batch<<<(n + 255) / 256, 256, 0, c->stream>>>(c->ix->d, n, k_buf.as<int64_t>(), out_buf.as<int64_t>(), mode);
 	c->last_launches = 1;
 	CUDA_TRY(cudaEventRecord(c->ev1, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[1].p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(out, out_buf.p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
 	CUDA_TRY(cudaStreamSynchronize(c->stream));
 	CUDA_TRY(cudaGetLastError());
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1); c->last_ms = ms;
@@ -704,23 +718,23 @@ extern "C" int emab_smem_batch(emab_ctx_t *c, int n, const uint8_t *seq, const i
 		int64_t l = off[i + 1] - off[i];
 		if (l < 0 || l > EMAB_MAX_READ_LEN) { snprintf(emab_errbuf, sizeof emab_errbuf, "read %d: length %lld out of range (max %d)", i, (long long)l, EMAB_MAX_READ_LEN); return EMAB_ERR_ARG; }
 	}
-	TRY(upload(c, c->b[0], seq, (size_t)off[n]));
-	TRY(upload(c, c->b[1], off, (size_t)(n + 1) * 8));
-	TRY(c->b[2].ensure((size_t)n * max_intv * sizeof(Intv)));
-	TRY(c->b[3].ensure((size_t)n * 4 + 4));
-	int32_t *d_ovf = c->b[3].as<int32_t>() + n;
+	TRY(upload(c, c->reads, seq, (size_t)off[n]));
+	TRY(upload(c, c->read_off, off, (size_t)(n + 1) * 8));
+	TRY(c->intv.ensure((size_t)n * max_intv * sizeof(Intv)));
+	TRY(c->n_intv.ensure((size_t)n * 4 + 4));
+	int32_t *d_ovf = c->n_intv.as<int32_t>() + n;
 	CUDA_TRY(cudaMemsetAsync(d_ovf, 0, 4, c->stream));
 	CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 64, c->stream));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
 	int max_len = 1;
 	for (int i = 0; i < n; ++i) if (off[i + 1] - off[i] > max_len) max_len = (int)(off[i + 1] - off[i]);
 	int launches = 0;
-	TRY(launch_seed(c, n, max_len, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<Intv>(), max_intv, c->b[3].as<int32_t>(), nullptr, d_ovf,
+	TRY(launch_seed(c, n, max_len, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), c->intv.as<Intv>(), max_intv, c->n_intv.as<int32_t>(), nullptr, d_ovf,
 	                &c->d_counters[2], &launches));
 	c->last_launches = launches;
 	CUDA_TRY(cudaEventRecord(c->ev1, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(intervals, c->b[2].p, (size_t)n * max_intv * sizeof(Intv), cudaMemcpyDeviceToHost, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(n_intv, c->b[3].p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(intervals, c->intv.p, (size_t)n * max_intv * sizeof(Intv), cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(n_intv, c->n_intv.p, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
 	int32_t ovf = 0;
 	unsigned long long cnt[3];
 	CUDA_TRY(cudaMemcpyAsync(&ovf, d_ovf, 4, cudaMemcpyDeviceToHost, c->stream));

@@ -226,13 +226,13 @@ struct MinOp { __device__ u64 operator()(u64 a, u64 b) const { return a < b ? a 
 inline unsigned grid(u64 n, int t) { return (unsigned)((n + t - 1) / t); }
 inline double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
-// cub temp storage in slot 6 (the stream is in order: a buffer regrown by ensure() waits for the work before it)
+// cub temp storage in the ctx's cub_tmp (the stream is in order: a buffer regrown by ensure() waits for the work before it)
 template <class F> int cub_call(emab_ctx *c, F &&f)
 {
 	size_t tb = 0;
 	CUDA_TRY(f(nullptr, tb));
-	TRY(c->b[6].ensure(tb + 16));
-	CUDA_TRY(f(c->b[6].p, tb));
+	TRY(c->cub_tmp.ensure(tb + 16));
+	CUDA_TRY(f(c->cub_tmp.p, tb));
 	return EMAB_OK;
 }
 
@@ -244,13 +244,11 @@ int grow(emab_ctx *c, DevBuf &b, size_t used, size_t need)
 	TRY(n.ensure(need + need / 2));
 	if (used) CUDA_TRY(cudaMemcpyAsync(n.p, b.p, used, cudaMemcpyDeviceToDevice, c->stream));
 	CUDA_TRY(ctx_wait(c));
-	b.release();
-	b = n;
+	b = std::move(n);
 	return EMAB_OK;
 }
 
 // ---- the order of runs held in memory: a stable radix sort of (key, record index) over the runs back to back
-// slots: 34 rows, 35 keys/indices (both buffers of the sort), 36 offsets (input, body, sources), 37 lengths
 struct Order {
 	uint32_t n = 0, p = 0;                  // records, placed records (the unplaced ones come last)
 	emab_bam_key_t *rows = nullptr;         // device: the rows in input order
@@ -273,13 +271,16 @@ int device_order(emab_ctx *c, int n_runs, const emab_bam_run_t *runs, Order &o, 
 	for (int r = 0; r < n_runs; ++r) n64 += runs[r].n_recs;
 	if (n64 >= 0x7fffffffull) { snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_sort: %llu records are more than one sort takes", n64); return EMAB_ERR_ARG; }
 	const uint32_t n = o.n = (uint32_t)n64;
-	TRY(c->b[34].ensure((size_t)n * sizeof(emab_bam_key_t) + 16));
-	TRY(c->b[35].ensure((size_t)n * 24 + 64));
-	TRY(c->b[36].ensure((size_t)(n + 1) * 8 * 3 + 64));
-	emab_bam_key_t *rows = o.rows = c->b[34].as<emab_bam_key_t>();
-	u64 *key = c->b[35].as<u64>(), *key_s = key + n;
+	// the pipeline's wave buffers, dead after it: rows; keys and indices (both buffers of the sort); offsets (input, body,
+	// sources); lengths.  Borrowed, not held, so that a spilling worker ctx grows no buffers of its own.
+	DevBuf &rows_buf = c->ext_keys, &keys_buf = c->ext_order, &offs_buf = c->glob_tasks, &lens_buf = c->glob_keys;
+	TRY(rows_buf.ensure((size_t)n * sizeof(emab_bam_key_t) + 16));
+	TRY(keys_buf.ensure((size_t)n * 24 + 64));
+	TRY(offs_buf.ensure((size_t)(n + 1) * 8 * 3 + 64));
+	emab_bam_key_t *rows = o.rows = rows_buf.as<emab_bam_key_t>();
+	u64 *key = keys_buf.as<u64>(), *key_s = key + n;
 	uint32_t *idx = (uint32_t *)(key_s + n), *idx_s = o.idx_s = idx + n;
-	u64 *in_off = c->b[36].as<u64>(), *uoff = o.uoff = in_off + (n + 1), *src = uoff + (n + 1);
+	u64 *in_off = offs_buf.as<u64>(), *uoff = o.uoff = in_off + (n + 1), *src = uoff + (n + 1);
 	u64 at = 0;
 	for (int r = 0; r < n_runs; ++r) {
 		if (!runs[r].n_recs) continue;
@@ -294,8 +295,8 @@ int device_order(emab_ctx *c, int n_runs, const emab_bam_run_t *runs, Order &o, 
 	o.run_base.resize(o.first.size());
 	for (size_t r = 0; r < o.first.size(); ++r) CUDA_TRY(cudaMemcpyAsync(&o.run_base[r], in_off + o.first[r], 8, cudaMemcpyDeviceToHost, st));
 	TRY(cub_call(c, [&](void *tmp, size_t &tb) { return cub::DeviceRadixSort::SortPairs(tmp, tb, key, key_s, idx, idx_s, (int)n, 0, 64, st); }));
-	TRY(c->b[37].ensure((size_t)(n + 1) * 8 + 64));
-	u64 *slen = c->b[37].as<u64>();
+	TRY(lens_buf.ensure((size_t)(n + 1) * 8 + 64));
+	u64 *slen = lens_buf.as<u64>();
 	uint32_t h_placed = n;
 	uint32_t *d_placed = (uint32_t *)(in_off + n);   // in_off[n] (the total) is no longer needed: run_base holds what the host needs
 	CUDA_TRY(cudaMemcpyAsync(d_placed, &h_placed, 4, cudaMemcpyHostToDevice, st));
@@ -342,7 +343,7 @@ int sorted_rows(emab_ctx *c, int n_runs, const emab_bam_run_t *runs, const uint6
 // waits for the next window.  The index is built on the device from the same rows with state carried across windows
 // (DevRef, the chunk list, the linear index, the previous record's refID and bin); a record is indexed once its member is
 // compressed, since its virtual offset needs the member's file offset.
-// slots: 33 + 48-51 the compressor's, 37 index scratch, 39 virtual offsets; the rest is owned here
+// The slice's device copy, the compressor's buffers and the index scratch are the ctx's scratch; the rest is owned here.
 struct Writer {
 	emab_ctx *c;
 	cudaStream_t st;
@@ -365,12 +366,7 @@ struct Writer {
 	Writer(emab_ctx *c_, int n_ref_, const int32_t *ref_len_, u64 body_offset_, int slice_chunks, emab_write_cb w_, void *uw_, bool index_)
 	    : c(c_), st(c_->stream), n_ref(n_ref_), ref_len(ref_len_), body_offset(body_offset_),
 	      S((u64)(slice_chunks > 0 ? slice_chunks : 1024) * bgzf::CHUNK), w(w_), uw(uw_), index(index_) {}
-	~Writer()
-	{
-		cudaStreamSynchronize(st);
-		in.release(); out.release();
-		for (DevBuf *b : {&moff, &prow, &pu, &trow, &tu, &ckey, &cbeg, &refs, &lin, &state}) b->release();
-	}
+	~Writer() { cudaStreamSynchronize(st); }   // before the members free what the stream may still use
 
 	int start()
 	{
@@ -436,12 +432,13 @@ struct Writer {
 			t[1] += tc - tg;
 			const u64 nc = (b - a + bgzf::CHUNK - 1) / bgzf::CHUNK;
 			TRY(grow(c, moff, (size_t)(m + 1) * 8, (size_t)(m + nc + 1) * 8));
-			TRY(c->b[33].ensure((size_t)(b - a) + 16));
-			CUDA_TRY(cudaMemcpyAsync(c->b[33].p, in.p, (size_t)(b - a), cudaMemcpyHostToDevice, st));
+			DevBuf &slice = c->ext_plans;   // the pipeline's extension plans, dead after it
+			TRY(slice.ensure((size_t)(b - a) + 16));
+			CUDA_TRY(cudaMemcpyAsync(slice.p, in.p, (size_t)(b - a), cudaMemcpyHostToDevice, st));
 			u64 olen = 0;
 			int launches = 0;
 			const u64 *d_moff = nullptr;
-			TRY(bgzf_compress_device(c, c->b[33].as<uint8_t>(), b - a, (uint8_t *)out.p, (uint64_t)out.cap, (uint64_t *)&olen, &launches, &d_moff));
+			TRY(bgzf_compress_device(c, slice.as<uint8_t>(), b - a, (uint8_t *)out.p, (uint64_t)out.cap, (uint64_t *)&olen, &launches, &d_moff));
 			k_member_off<<<grid(nc + 1, 256), 256, 0, st>>>(moff.as<u64>() + m, d_moff, (uint32_t)(nc + 1), written);
 			CUDA_TRY(cudaGetLastError());
 			if (w(uw, (const char *)out.p, olen) != 0) { snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_sort: write failed"); return EMAB_ERR_IO; }
@@ -483,14 +480,16 @@ struct Writer {
 		const emab_bam_key_t *rows = prow.as<emab_bam_key_t>();
 		IdxState *s = state.as<IdxState>();
 		DevRef *drefs = refs.as<DevRef>();
-		TRY(c->b[39].ensure((size_t)q * 8 + 16));
-		u64 *voff = c->b[39].as<u64>();
+		// the pipeline's global-alignment wave buffers, dead after it
+		DevBuf &voff_buf = c->glob_cigars, &chunk_buf = c->glob_keys;
+		TRY(voff_buf.ensure((size_t)q * 8 + 16));
+		u64 *voff = voff_buf.as<u64>();
 		k_voff<<<grid(q, 256), 256, 0, st>>>(pu.as<u64>(), q, moff.as<u64>(), body_offset, voff);
 		if (!p) return EMAB_OK;
 		// chunk starts: flags | starts | count
 		const size_t o_start = ((size_t)p + 15) & ~(size_t)15, o_cnt = o_start + (size_t)p * 4;
-		TRY(c->b[37].ensure(o_cnt + 64));
-		uint8_t *flag = c->b[37].as<uint8_t>();
+		TRY(chunk_buf.ensure(o_cnt + 64));
+		uint8_t *flag = chunk_buf.as<uint8_t>();
 		uint32_t *start = (uint32_t *)(flag + o_start), *d_kn = (uint32_t *)(flag + o_cnt), kn = 0;
 		k_chunk_flag<<<grid(p, 256), 256, 0, st>>>(rows, p, s, flag);
 		TRY(cub_call(c, [&](void *tmp, size_t &tb) {
@@ -539,8 +538,9 @@ struct Writer {
 		// chunks: ends | indices, sorted indices | sorted keys | bins | begs | ends
 		const size_t o_idx = (size_t)kn * 8, o_key = ((o_idx + (size_t)kn * 8) + 15) & ~(size_t)15, o_bin = o_key + (size_t)kn * 8,
 		             o_beg = ((o_bin + (size_t)kn * 2) + 15) & ~(size_t)15, o_end = o_beg + (size_t)kn * 8;
-		TRY(c->b[37].ensure(o_end + (size_t)kn * 8 + 64));
-		char *x = c->b[37].as<char>();
+		DevBuf &chunk_buf = c->glob_keys;   // the pipeline's global-alignment wave keys, dead after it
+		TRY(chunk_buf.ensure(o_end + (size_t)kn * 8 + 64));
+		char *x = chunk_buf.as<char>();
 		u64 *cend = (u64 *)x, *ckey_s = (u64 *)(x + o_key), *sbeg = (u64 *)(x + o_beg), *send = (u64 *)(x + o_end);
 		uint32_t *cidx = (uint32_t *)(x + o_idx), *cidx_s = cidx + kn;
 		uint16_t *cbin = (uint16_t *)(x + o_bin);
@@ -781,15 +781,17 @@ extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *pat
 		W.t[1] += now_ms() - tg;
 		// ---- the device: the bound, the rows at or below it, their order by (key, seq) and their body offsets
 		t0 = now_ms();
-		// slot 34: rows | runs; 35: bound | flags | taken | count | keys, sorted keys | perm; 36: lengths, offsets
+		// the pipeline's wave buffers, dead after it: rows | runs; bound | flags | taken | count | keys, sorted keys | perm;
+		// lengths, offsets
+		DevBuf &rows_buf = c->ext_keys, &take_buf = c->ext_order, &lens_buf = c->glob_tasks;
 		const size_t o_seg = ((size_t)n * sizeof(SpillRow) + 15) & ~(size_t)15;
-		TRY(c->b[34].ensure(o_seg + (size_t)ns * sizeof(RunSeg) + 16));
-		SpillRow *d_rows = c->b[34].as<SpillRow>();
-		RunSeg *d_seg = (RunSeg *)(c->b[34].as<char>() + o_seg);
+		TRY(rows_buf.ensure(o_seg + (size_t)ns * sizeof(RunSeg) + 16));
+		SpillRow *d_rows = rows_buf.as<SpillRow>();
+		RunSeg *d_seg = (RunSeg *)(rows_buf.as<char>() + o_seg);
 		const size_t o_flag = 16, o_taken = (o_flag + n + 15) & ~(size_t)15, o_cnt = o_taken + (size_t)n * 4, o_mk = (o_cnt + 16 + 15) & ~(size_t)15,
 		             o_perm = o_mk + (size_t)n * 32;
-		TRY(c->b[35].ensure(o_perm + (size_t)n * 4 + 64));
-		char *x = c->b[35].as<char>();
+		TRY(take_buf.ensure(o_perm + (size_t)n * 4 + 64));
+		char *x = take_buf.as<char>();
 		MKey *d_bound = (MKey *)x, *mk = (MKey *)(x + o_mk), *mk_s = mk + n;
 		uint8_t *flag = (uint8_t *)(x + o_flag);
 		uint32_t *taken = (uint32_t *)(x + o_taken), *d_cnt = (uint32_t *)(x + o_cnt), *d_perm = (uint32_t *)(x + o_perm);
@@ -807,8 +809,8 @@ extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *pat
 		k_take_keys<<<grid(T, 256), 256, 0, st>>>(d_rows, taken, T, mk);
 		TRY(cub_call(c, [&](void *tmp, size_t &tb) {
 			return cub::DeviceRadixSort::SortPairs(tmp, tb, mk, mk_s, taken, d_perm, (int)T, MKeyBits{}, st); }));
-		TRY(c->b[36].ensure((size_t)(T + 1) * 16 + 64));
-		u64 *slen = c->b[36].as<u64>(), *uoff = slen + (T + 1);
+		TRY(lens_buf.ensure((size_t)(T + 1) * 16 + 64));
+		u64 *slen = lens_buf.as<u64>(), *uoff = slen + (T + 1);
 		k_take_len<<<grid(T + 1, 256), 256, 0, st>>>(d_rows, d_perm, T, slen);
 		TRY(cub_call(c, [&](void *tmp, size_t &tb) { return cub::DeviceScan::ExclusiveSum(tmp, tb, slen, uoff, (int)T + 1, st); }));
 		TRY(W.reserve(T));

@@ -132,8 +132,8 @@ __global__ void k_bgzf_gather(const uint8_t *__restrict__ slots, const unsigned 
 
 }  // namespace
 
-// slots: 48 tokens (4 bytes per input byte), 49 one 64 KB member slot per chunk, 50 sizes / offsets / scan scratch,
-// 51 the packed members
+// scratch of the ctx: bgzf_tokens (4 bytes per input byte), bgzf_members (one 64 KB member slot per chunk), bgzf_off
+// (sizes / offsets / scan scratch), bgzf_out (the packed members)
 int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches,
                          const unsigned long long **d_member_off)
 {
@@ -143,18 +143,18 @@ int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *
 	if (n == 0) { CUDA_TRY(cudaEventRecord(c->ev1, st)); return EMAB_OK; }
 	const uint64_t nc = (n + CHUNK - 1) / CHUNK;
 	if (nc > 0x7fffffffull) { snprintf(emab_errbuf, sizeof emab_errbuf, "bgzf: input too large"); return EMAB_ERR_ARG; }
-	TRY(c->b[48].ensure((size_t)nc * CHUNK * 4));
-	TRY(c->b[49].ensure((size_t)nc * MEMBER_MAX));
+	TRY(c->bgzf_tokens.ensure((size_t)nc * CHUNK * 4));
+	TRY(c->bgzf_members.ensure((size_t)nc * MEMBER_MAX));
 	unsigned long long *d_size = nullptr, *d_off = nullptr;
 	size_t tb = 0;
 	cub::DeviceScan::ExclusiveSum(nullptr, tb, d_size, d_off, (int)nc + 1, st);
 	const size_t o_tmp = ((size_t)(nc + 1) * 16 + 255) & ~(size_t)255;
-	TRY(c->b[50].ensure(o_tmp + tb + 16));
-	d_size = c->b[50].as<unsigned long long>(); d_off = d_size + (nc + 1);
+	TRY(c->bgzf_off.ensure(o_tmp + tb + 16));
+	d_size = c->bgzf_off.as<unsigned long long>(); d_off = d_size + (nc + 1);
 	CUDA_TRY(cudaMemsetAsync(d_size + nc, 0, 8, st));
 	CUDA_TRY(cudaFuncSetAttribute(k_bgzf_member, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(BgSmem)));
-	k_bgzf_member<<<(unsigned)nc, BG_THREADS, sizeof(BgSmem), st>>>(d_in, n, c->b[48].as<uint32_t>(), c->b[49].as<uint8_t>(), d_size);
-	cub::DeviceScan::ExclusiveSum(c->b[50].as<char>() + o_tmp, tb, d_size, d_off, (int)nc + 1, st);
+	k_bgzf_member<<<(unsigned)nc, BG_THREADS, sizeof(BgSmem), st>>>(d_in, n, c->bgzf_tokens.as<uint32_t>(), c->bgzf_members.as<uint8_t>(), d_size);
+	cub::DeviceScan::ExclusiveSum(c->bgzf_off.as<char>() + o_tmp, tb, d_size, d_off, (int)nc + 1, st);
 	unsigned long long total = 0;
 	CUDA_TRY(cudaMemcpyAsync(&total, d_off + nc, 8, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
@@ -164,10 +164,10 @@ int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *
 		snprintf(emab_errbuf, sizeof emab_errbuf, "bgzf: %llu compressed bytes do not fit the output buffer", total);
 		return EMAB_ERR_OVERFLOW;
 	}
-	TRY(c->b[51].ensure((size_t)total + 16));
-	k_bgzf_gather<<<(unsigned)nc, 256, 0, st>>>(c->b[49].as<uint8_t>(), d_off, c->b[51].as<uint8_t>());
+	TRY(c->bgzf_out.ensure((size_t)total + 16));
+	k_bgzf_gather<<<(unsigned)nc, 256, 0, st>>>(c->bgzf_members.as<uint8_t>(), d_off, c->bgzf_out.as<uint8_t>());
 	CUDA_TRY(cudaEventRecord(c->ev1, st));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[51].p, (size_t)total, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(out, c->bgzf_out.p, (size_t)total, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	CUDA_TRY(cudaGetLastError());
 	*launches = 3;
@@ -181,11 +181,12 @@ extern "C" int emab_bgzf_compress(emab_ctx_t *c, const uint8_t *in, uint64_t len
 	CTX_ENTER(c);
 	if (!c || (!in && len) || !out_len) return EMAB_ERR_ARG;
 	*out_len = 0;
-	TRY(c->b[33].ensure((size_t)len + 16));
-	if (len) CUDA_TRY(cudaMemcpyAsync(c->b[33].p, in, (size_t)len, cudaMemcpyHostToDevice, c->stream));
+	DevBuf &d_in = c->ext_plans;   // the pipeline's extension plans: dead between calls
+	TRY(d_in.ensure((size_t)len + 16));
+	if (len) CUDA_TRY(cudaMemcpyAsync(d_in.p, in, (size_t)len, cudaMemcpyHostToDevice, c->stream));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
 	int launches = 0;
-	TRY(bgzf_compress_device(c, c->b[33].as<uint8_t>(), len, out, out_cap, out_len, &launches));
+	TRY(bgzf_compress_device(c, d_in.as<uint8_t>(), len, out, out_cap, out_len, &launches));
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 	c->last_ms = ms; c->last_launches = launches;
 	return EMAB_OK;

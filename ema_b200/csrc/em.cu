@@ -172,7 +172,8 @@ extern "C" int emab_em_batch(emab_ctx_t *c, const emab_em_problem_t *h, double *
 	const double *log_n = log_table.v;
 	EmProblem P;
 	P.n_bc = nb; P.many_clouds = h->many_clouds; P.log_eps = log(1e-50);
-	DevBuf *b = c->b;
+	// the seeding buffers of the pipeline, dead after it; the results it leaves for the formatters are not touched
+	DevBuf &blob = c->packed_reads, &gamma_buf = c->sa_vals, &cw_buf = c->seed_prof;
 	// The eighteen input arrays travel as ONE block: packed into a pinned staging buffer (256-byte aligned parts) and
 	// copied with one cudaMemcpyAsync — eighteen copies from pageable vectors were eighteen synchronous staging
 	// round trips inside the capped post phase of the host pipeline.
@@ -186,11 +187,11 @@ extern "C" int emab_em_batch(emab_ctx_t *c, const emab_em_problem_t *h, double *
 		{h->unit_second, (size_t)U * 4, 0}};
 	size_t total = 0;
 	for (Part &q : parts) { q.off = total; total += (q.bytes + 255) & ~(size_t)255; }
-	TRY(c->h[4].ensure(total + 256));
-	TRY(b[41].ensure(total + 256));   // slots 41-44: the pipeline's slots (reads, candidates, CIGARs) stay valid for emab_sam_format
-	for (const Part &q : parts) if (q.bytes) memcpy((char *)c->h[4].p + q.off, q.src, q.bytes);
-	CUDA_TRY(cudaMemcpyAsync(b[41].p, c->h[4].p, total, cudaMemcpyHostToDevice, c->stream));
-	char *d0 = (char *)b[41].p;
+	TRY(c->em_stage.ensure(total + 256));
+	TRY(blob.ensure(total + 256));
+	for (const Part &q : parts) if (q.bytes) memcpy((char *)c->em_stage.p + q.off, q.src, q.bytes);
+	CUDA_TRY(cudaMemcpyAsync(blob.p, c->em_stage.p, total, cudaMemcpyHostToDevice, c->stream));
+	char *d0 = (char *)blob.p;
 	P.bc_entry_off = (const int32_t *)(d0 + parts[0].off); P.bc_cloud_off = (const int32_t *)(d0 + parts[1].off);
 	P.bc_group_off = (const int32_t *)(d0 + parts[2].off); P.bc_unit_off = (const int32_t *)(d0 + parts[3].off);
 	P.bc_full_em = (const int32_t *)(d0 + parts[4].off); P.entry_cand_off = (const int32_t *)(d0 + parts[5].off);
@@ -200,25 +201,25 @@ extern "C" int emab_em_batch(emab_ctx_t *c, const emab_em_problem_t *h, double *
 	P.group_off = (const int32_t *)(d0 + parts[12].off); P.group_clouds = (const int32_t *)(d0 + parts[13].off);
 	P.cloud_contrib_off = (const int32_t *)(d0 + parts[14].off); P.cloud_contrib = (const int32_t *)(d0 + parts[15].off);
 	P.unit_first = (const int32_t *)(d0 + parts[16].off); P.unit_second = (const int32_t *)(d0 + parts[17].off);
-	if (!c->em_log_ready) {  // the ln(n) table is uploaded once per ctx; slot 30 is nobody else's
-		TRY(up(c, b[30], log_n, sizeof log_table.v));
+	if (!c->em_log_ready) {  // the ln(n) table is uploaded once per ctx
+		TRY(up(c, c->em_log, log_n, sizeof log_table.v));
 		c->em_log_ready = true;
 	}
-	P.log_n = b[30].as<double>();
-	TRY(b[42].ensure((size_t)K * 8));                          P.gamma = b[42].as<double>();
-	TRY(b[43].ensure((size_t)K * 8));                          P.cw = b[43].as<double>();
-	TRY(b[44].ensure((size_t)C * 16 + 16));                    P.exp_cov = b[44].as<double>(); P.weight = P.exp_cov + C;
-	TRY(c->h[5].ensure((size_t)K * 8 + 8));
+	P.log_n = c->em_log.as<double>();
+	TRY(gamma_buf.ensure((size_t)K * 8));                      P.gamma = gamma_buf.as<double>();
+	TRY(cw_buf.ensure((size_t)K * 8));                         P.cw = cw_buf.as<double>();
+	TRY(c->em_cov.ensure((size_t)C * 16 + 16));                P.exp_cov = c->em_cov.as<double>(); P.weight = P.exp_cov + C;
+	TRY(c->em_gamma.ensure((size_t)K * 8 + 8));
 	CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 64, c->stream));
 	CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
 	int blocks = nb;
 	if (blocks > c->n_sm * 8) blocks = c->n_sm * 8;
 	k_em<<<blocks, 128, 0, c->stream>>>(P, 5 /* EM_ITERS, include/align.h:52 */, c->d_counters);
 	CUDA_TRY(cudaEventRecord(c->ev1, c->stream));
-	CUDA_TRY(cudaMemcpyAsync(c->h[5].p, P.gamma, (size_t)K * 8, cudaMemcpyDeviceToHost, c->stream));
+	CUDA_TRY(cudaMemcpyAsync(c->em_gamma.p, P.gamma, (size_t)K * 8, cudaMemcpyDeviceToHost, c->stream));
 	CUDA_TRY(ctx_wait(c));
 	CUDA_TRY(cudaGetLastError());
-	memcpy(gamma_out, c->h[5].p, (size_t)K * 8);
+	memcpy(gamma_out, c->em_gamma.p, (size_t)K * 8);
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 	c->last_ms = ms; c->last_launches = 1;
 	return EMAB_OK;

@@ -88,9 +88,10 @@ extern "C" int emab_int_peak(emab_ctx_t *c, int kind, int iters, double *gops_pe
 {
 	CTX_ENTER(c);
 	if (!c || kind < 0 || kind > 19 || iters <= 0 || !gops_per_s) return EMAB_ERR_ARG;
-	if (c->b[27].ensure(64)) return EMAB_ERR_NOMEM;
+	DevBuf &sink_buf = c->err;   // scratch: only written when the chains' result is 0x7fffffff
+	if (sink_buf.ensure(64)) return EMAB_ERR_NOMEM;
 	const int grid = c->n_sm * 8, block = 256;
-	int *sink = c->b[27].as<int>();
+	int *sink = sink_buf.as<int>();
 	for (int rep = 0; rep < 2; ++rep) {  // first pass warms up
 		CUDA_TRY(cudaEventRecord(c->ev0, c->stream));
 		switch (kind) {

@@ -142,8 +142,7 @@ k_tokens(const char *text, unsigned text_len, const unsigned *starts, unsigned n
 
 // Uploads `text` (host memory; page-locked for speed) and parses it as one preprocessed bucket.  On return the text and
 // the per-pair table are resident for emab_align_pairs_resident / emab_sam_format, and *pairs / *bcs point at the ctx's
-// page-locked copies (valid until its next parse).  Slots: 31 text, 27 pair table, 28/29 parser scratch (free again before
-// the pipeline's mate rescue uses them).
+// page-locked copies (valid until its next parse).
 extern "C" int emab_parse_bucket(emab_ctx_t *c, const char *text, uint64_t text_len, int bc_len, int is_haplotag, int *n_pairs,
                                  const emab_pair_text_t **pairs, const uint64_t **bcs)
 {
@@ -154,13 +153,15 @@ extern "C" int emab_parse_bucket(emab_ctx_t *c, const char *text, uint64_t text_
 	if (text_len == 0) return EMAB_OK;
 	if (text_len >= 0xfffffff0ull) { snprintf(emab_errbuf, sizeof emab_errbuf, "bucket text larger than 4 GB"); return EMAB_ERR_ARG; }
 	cudaStream_t st = c->stream;
+	// the parser's scratch: buffers of the pipeline's seeding and mate rescue, which only run after the parse
+	DevBuf &starts_buf = c->rescue_tasks, &keys_buf = c->rescue_spans, &bcs_buf = c->seed_queue;
 	const unsigned L = (unsigned)text_len;
-	TRY(c->b[31].ensure((size_t)L + 16));
-	CUDA_TRY(cudaMemcpyAsync(c->b[31].p, text, L, cudaMemcpyHostToDevice, st));
-	const char *d_text = c->b[31].as<char>();
+	TRY(c->text.ensure((size_t)L + 16));
+	CUDA_TRY(cudaMemcpyAsync(c->text.p, text, L, cudaMemcpyHostToDevice, st));
+	const char *d_text = c->text.as<char>();
 	// line starts: count the newlines first (the exact room for the start offsets), then select
-	TRY(c->b[22].ensure(16));
-	int *d_err = c->b[22].as<int>();
+	TRY(c->err.ensure(16));
+	int *d_err = c->err.as<int>();
 	CUDA_TRY(cudaMemsetAsync(d_err, 0, 16, st));
 	unsigned *d_count = (unsigned *)(d_err + 2), *d_newlines = (unsigned *)(d_err + 3);
 	k_count_newlines<<<148 * 8, 256, 0, st>>>(d_text, L, d_newlines);
@@ -168,14 +169,14 @@ extern "C" int emab_parse_bucket(emab_ctx_t *c, const char *text, uint64_t text_
 	CUDA_TRY(cudaMemcpyAsync(&n_newlines, d_newlines, 4, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	const size_t max_lines = (size_t)n_newlines + 2;
-	TRY(c->b[28].ensure(max_lines * 4 + 64));
-	unsigned *d_starts = c->b[28].as<unsigned>();
+	TRY(starts_buf.ensure(max_lines * 4 + 64));
+	unsigned *d_starts = starts_buf.as<unsigned>();
 	size_t tb = 0;
 	cub::CountingInputIterator<unsigned> idx(0);
 	IsLineStart pred{d_text};
 	cub::DeviceSelect::If(nullptr, tb, idx, d_starts, d_count, (int)L, pred, st);
-	TRY(c->b[6].ensure(tb + 16));
-	cub::DeviceSelect::If(c->b[6].p, tb, idx, d_starts, d_count, (int)L, pred, st);
+	TRY(c->cub_tmp.ensure(tb + 16));
+	cub::DeviceSelect::If(c->cub_tmp.p, tb, idx, d_starts, d_count, (int)L, pred, st);
 	unsigned n = 0;
 	CUDA_TRY(cudaMemcpyAsync(&n, d_count, 4, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
@@ -183,30 +184,30 @@ extern "C" int emab_parse_bucket(emab_ctx_t *c, const char *text, uint64_t text_
 	// sort keys, least significant word first (LSD over stable sorts = the strncmp order with ties in file order)
 	const int W = is_haplotag ? 2 : (bc_len + 7) / 8 > 0 ? (bc_len + 7) / 8 : 1;
 	const int key_len = is_haplotag ? 12 : bc_len;
-	TRY(c->b[29].ensure((size_t)n * 8 * (W + 2) + (size_t)n * 4 * 2 + 64));
-	unsigned long long *d_keys = c->b[29].as<unsigned long long>(), *d_k0 = d_keys + (size_t)W * n, *d_k1 = d_k0 + n;
+	TRY(keys_buf.ensure((size_t)n * 8 * (W + 2) + (size_t)n * 4 * 2 + 64));
+	unsigned long long *d_keys = keys_buf.as<unsigned long long>(), *d_k0 = d_keys + (size_t)W * n, *d_k1 = d_k0 + n;
 	unsigned *d_p0 = (unsigned *)(d_k1 + n), *d_p1 = d_p0 + n;
 	k_line_keys<<<(n + 255) / 256, 256, 0, st>>>(d_text, L, d_starts, n, key_len, W, d_keys, d_err);
 	k_iota_u32<<<(n + 255) / 256, 256, 0, st>>>(n, d_p0);
 	cub::DeviceRadixSort::SortPairs(nullptr, tb, d_k0, d_k1, d_p0, d_p1, (int)n, 0, 64, st);
-	TRY(c->b[6].ensure(tb + 16));
+	TRY(c->cub_tmp.ensure(tb + 16));
 	unsigned *perm = d_p0, *perm_alt = d_p1;
 	for (int w = W - 1; w >= 0; --w) {
 		k_gather_keys<<<(n + 255) / 256, 256, 0, st>>>(n, perm, d_keys + (size_t)w * n, d_k0);
-		cub::DeviceRadixSort::SortPairs(c->b[6].p, tb, d_k0, d_k1, perm, perm_alt, (int)n, 0, 64, st);
+		cub::DeviceRadixSort::SortPairs(c->cub_tmp.p, tb, d_k0, d_k1, perm, perm_alt, (int)n, 0, 64, st);
 		unsigned *t = perm; perm = perm_alt; perm_alt = t;
 	}
 	// fields
-	TRY(c->b[27].ensure((size_t)n * sizeof(emab_pair_text_t) + 16));
-	TRY(c->b[26].ensure((size_t)n * 8 + 16));
-	k_tokens<<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st>>>(d_text, L, d_starts, n, perm, bc_len, is_haplotag, c->b[27].as<emab_pair_text_t>(),
-	                                                                   c->b[26].as<unsigned long long>(), d_err);
-	TRY(c->h[7].ensure((size_t)n * (sizeof(emab_pair_text_t) + 8) + 64));
-	emab_pair_text_t *h_pairs = (emab_pair_text_t *)c->h[7].p;
-	uint64_t *h_bcs = (uint64_t *)((char *)c->h[7].p + (((size_t)n * sizeof(emab_pair_text_t) + 15) & ~(size_t)15));
+	TRY(c->pairs.ensure((size_t)n * sizeof(emab_pair_text_t) + 16));
+	TRY(bcs_buf.ensure((size_t)n * 8 + 16));
+	k_tokens<<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st>>>(d_text, L, d_starts, n, perm, bc_len, is_haplotag, c->pairs.as<emab_pair_text_t>(),
+	                                                                   bcs_buf.as<unsigned long long>(), d_err);
+	TRY(c->h_parsed.ensure((size_t)n * (sizeof(emab_pair_text_t) + 8) + 64));
+	emab_pair_text_t *h_pairs = (emab_pair_text_t *)c->h_parsed.p;
+	uint64_t *h_bcs = (uint64_t *)((char *)c->h_parsed.p + (((size_t)n * sizeof(emab_pair_text_t) + 15) & ~(size_t)15));
 	int h_err = 0;
-	CUDA_TRY(cudaMemcpyAsync(h_pairs, c->b[27].p, (size_t)n * sizeof(emab_pair_text_t), cudaMemcpyDeviceToHost, st));
-	CUDA_TRY(cudaMemcpyAsync(h_bcs, c->b[26].p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(h_pairs, c->pairs.p, (size_t)n * sizeof(emab_pair_text_t), cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(h_bcs, bcs_buf.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(cudaMemcpyAsync(&h_err, d_err, 4, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	CUDA_TRY(cudaGetLastError());

@@ -488,8 +488,8 @@ extern "C" int emab_set_error_rate(emab_ctx_t *c, double eps)
 	if (!c || !(eps > 0 && eps < 1)) return EMAB_ERR_ARG;
 	ScoreConsts sc;
 	fill_consts(sc, eps);
-	TRY(c->b[23].ensure(sizeof sc));
-	CUDA_TRY(cudaMemcpy(c->b[23].p, &sc, sizeof sc, cudaMemcpyHostToDevice));
+	TRY(c->consts.ensure(sizeof sc));
+	CUDA_TRY(cudaMemcpy(c->consts.p, &sc, sizeof sc, cudaMemcpyHostToDevice));
 	c->consts_ready = true;
 	return EMAB_OK;
 }
@@ -528,9 +528,8 @@ extern "C" int emab_align_pairs(emab_ctx_t *c, int n_pairs, const uint8_t *seq, 
 		if (l > max_len && l <= EMAB_MAX_READ_LEN) max_len = (int)l;
 		if (l < 0 || l > EMAB_MAX_READ_LEN) { snprintf(emab_errbuf, sizeof emab_errbuf, "read %d: length %lld out of range (max %d)", i, (long long)l, EMAB_MAX_READ_LEN); return EMAB_ERR_ARG; }
 	}
-	// slots: 0 seq, 1 off, 2 intv, 3 n_intv, 4 smem scratch, 5 occ_cnt/off, 6 cub temp, 7.. pools
-	TRY(upload(c, c->b[0], seq, (size_t)off[R]));
-	TRY(upload(c, c->b[1], off, (size_t)(R + 1) * 8));
+	TRY(upload(c, c->reads, seq, (size_t)off[R]));
+	TRY(upload(c, c->read_off, off, (size_t)(R + 1) * 8));
 	c->text_ready = false;
 	return align_pairs_core(c, n_pairs, max_len, off[R], (int64_t)off[R] + (int64_t)(R + 1) * 8, stage, want_regs, res, stats, true);
 }
@@ -556,11 +555,11 @@ extern "C" int emab_align_pairs_text(emab_ctx_t *c, int n_pairs, const char *tex
 		if ((uint64_t)pairs[i >> 1].read_off[i & 1] + (uint64_t)l > text_len) { snprintf(emab_errbuf, sizeof emab_errbuf, "read %d lies outside the text", i); return EMAB_ERR_ARG; }
 	}
 	cudaStream_t st = c->stream;
-	TRY(upload(c, c->b[31], text, (size_t)text_len));
-	TRY(upload(c, c->b[27], pairs, (size_t)n_pairs * sizeof(emab_pair_text_t)));
-	TRY(upload(c, c->b[1], off, (size_t)(R + 1) * 8));
-	TRY(c->b[0].ensure((size_t)off[R] + 16));
-	k_encode_reads<<<(R * 32 + 255) / 256, 256, 0, st>>>(c->b[31].as<char>(), c->b[27].as<emab_pair_text_t>(), R, c->b[1].as<int64_t>(), c->b[0].as<uint8_t>());
+	TRY(upload(c, c->text, text, (size_t)text_len));
+	TRY(upload(c, c->pairs, pairs, (size_t)n_pairs * sizeof(emab_pair_text_t)));
+	TRY(upload(c, c->read_off, off, (size_t)(R + 1) * 8));
+	TRY(c->reads.ensure((size_t)off[R] + 16));
+	k_encode_reads<<<(R * 32 + 255) / 256, 256, 0, st>>>(c->text.as<char>(), c->pairs.as<emab_pair_text_t>(), R, c->read_off.as<int64_t>(), c->reads.as<uint8_t>());
 	c->text_ready = true;
 	return align_pairs_core(c, n_pairs, max_len, off[R], (int64_t)text_len + (int64_t)n_pairs * (int64_t)sizeof(emab_pair_text_t) + (int64_t)(R + 1) * 8,
 	                        3, 0, res, stats, false);
@@ -583,9 +582,9 @@ extern "C" int emab_align_pairs_resident(emab_ctx_t *c, int n_pairs, const int64
 		if (l > max_len) max_len = (int)l;
 	}
 	cudaStream_t st = c->stream;
-	TRY(upload(c, c->b[1], off, (size_t)(R + 1) * 8));
-	TRY(c->b[0].ensure((size_t)off[R] + 16));
-	k_encode_reads<<<(R * 32 + 255) / 256, 256, 0, st>>>(c->b[31].as<char>(), c->b[27].as<emab_pair_text_t>(), R, c->b[1].as<int64_t>(), c->b[0].as<uint8_t>());
+	TRY(upload(c, c->read_off, off, (size_t)(R + 1) * 8));
+	TRY(c->reads.ensure((size_t)off[R] + 16));
+	k_encode_reads<<<(R * 32 + 255) / 256, 256, 0, st>>>(c->text.as<char>(), c->pairs.as<emab_pair_text_t>(), R, c->read_off.as<int64_t>(), c->reads.as<uint8_t>());
 	return align_pairs_core(c, n_pairs, max_len, off[R], (int64_t)c->text_len + (int64_t)(R + 1) * 8, 3, 0, res, stats, false);
 }
 
@@ -597,11 +596,11 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 	if (!c->consts_ready) TRY(emab_set_error_rate(c, 0.001));
 	const DevIndex &ix = c->ix->d;
 	cudaStream_t st = c->stream;
-	TRY(c->b[3].ensure((size_t)R * 4));
-	TRY(c->b[5].ensure((size_t)(R + 1) * 4 * 2));
-	int32_t *d_occ_cnt = c->b[5].as<int32_t>(), *d_occ_off = d_occ_cnt + (R + 1);
-	TRY(c->b[22].ensure(16));
-	int *d_err = c->b[22].as<int>();
+	TRY(c->n_intv.ensure((size_t)R * 4));
+	TRY(c->occ.ensure((size_t)(R + 1) * 4 * 2));
+	int32_t *d_occ_cnt = c->occ.as<int32_t>(), *d_occ_off = d_occ_cnt + (R + 1);
+	TRY(c->err.ensure(16));
+	int *d_err = c->err.as<int>();
 	int launches = 0;
 	bool ext_waves_ran = false, glob_waves_ran = false;
 	if (!c->stage_ev[0]) for (int i = 0; i < 16; ++i) CUDA_TRY(cudaEventCreate(&c->stage_ev[i]));
@@ -614,16 +613,16 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 	int32_t T = 0;
 	size_t tmp_bytes = 0;
 	for (;;) {
-		TRY(c->b[2].ensure((size_t)R * max_intv * sizeof(Intv)));
+		TRY(c->intv.ensure((size_t)R * max_intv * sizeof(Intv)));
 		CUDA_TRY(cudaMemsetAsync(d_err, 0, 16, st));
 		CUDA_TRY(cudaMemsetAsync(c->d_counters, 0, 128, st));
 		CUDA_TRY(cudaMemsetAsync(d_occ_cnt, 0, (size_t)(R + 1) * 4, st));
-		TRY(launch_seed(c, R, max_len, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), c->b[2].as<Intv>(), max_intv, c->b[3].as<int32_t>(), d_occ_cnt, d_err,
+		TRY(launch_seed(c, R, max_len, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), c->intv.as<Intv>(), max_intv, c->n_intv.as<int32_t>(), d_occ_cnt, d_err,
 		                &c->d_counters[2], &launches));
 		CUDA_TRY(cudaEventRecord(c->stage_ev[1], st));
 		cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_occ_cnt, d_occ_off, R + 1, st);
-		TRY(c->b[6].ensure(tmp_bytes + 16));
-		cub::DeviceScan::ExclusiveSum(c->b[6].p, tmp_bytes, d_occ_cnt, d_occ_off, R + 1, st);
+		TRY(c->cub_tmp.ensure(tmp_bytes + 16));
+		cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tmp_bytes, d_occ_cnt, d_occ_off, R + 1, st);
 		k_sum64<<<64, 256, 0, st>>>(R, d_occ_cnt, &c->d_counters[1]);
 		launches += 2;
 		int seed_err = 0;
@@ -639,26 +638,26 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 	}
 	const size_t Tn = (size_t)T + 1, NR = (size_t)T + (size_t)RESCUE_ROOM * R + 1;
 	Pools p;
-	TRY(c->b[7].ensure(Tn * sizeof(Seed)));   p.w_seeds = c->b[7].as<Seed>();
-	TRY(c->b[8].ensure(Tn * sizeof(Chain)));  p.w_chains = c->b[8].as<Chain>();
-	TRY(c->b[9].ensure((Tn / 3 + 2 * (size_t)R + 4) * sizeof(BNode)));  p.w_nodes = c->b[9].as<BNode>();
-	TRY(c->b[10].ensure(3 * Tn * 4));         p.w_ord = c->b[10].as<int32_t>();
-	TRY(c->b[11].ensure(Tn * sizeof(Seed)));  p.seeds = c->b[11].as<Seed>();
-	TRY(c->b[12].ensure(Tn * sizeof(Chain))); p.chains = c->b[12].as<Chain>();
-	TRY(c->b[13].ensure(Tn * 8));             p.srt = c->b[13].as<uint64_t>();
-	TRY(c->b[14].ensure(NR * sizeof(Reg)));   p.regs = c->b[14].as<Reg>();
-	TRY(c->b[15].ensure((size_t)(R + 1) * 4 * 3));
-	p.n_chains = c->b[15].as<int32_t>(); p.n_regs = p.n_chains + (R + 1);
+	TRY(c->w_seeds.ensure(Tn * sizeof(Seed)));        p.w_seeds = c->w_seeds.as<Seed>();
+	TRY(c->w_chains.ensure(Tn * sizeof(Chain)));      p.w_chains = c->w_chains.as<Chain>();
+	TRY(c->w_nodes.ensure((Tn / 3 + 2 * (size_t)R + 4) * sizeof(BNode))); p.w_nodes = c->w_nodes.as<BNode>();
+	TRY(c->w_ord.ensure(3 * Tn * 4));                 p.w_ord = c->w_ord.as<int32_t>();
+	TRY(c->seeds.ensure(Tn * sizeof(Seed)));          p.seeds = c->seeds.as<Seed>();
+	TRY(c->chains.ensure(Tn * sizeof(Chain)));        p.chains = c->chains.as<Chain>();
+	TRY(c->srt.ensure(Tn * 8));                       p.srt = c->srt.as<uint64_t>();
+	TRY(c->regs.ensure(NR * sizeof(Reg)));            p.regs = c->regs.as<Reg>();
+	TRY(c->reg_counts.ensure((size_t)(R + 1) * 4 * 3));
+	p.n_chains = c->reg_counts.as<int32_t>(); p.n_regs = p.n_chains + (R + 1);
 	int32_t *d_aln_off = p.n_regs + (R + 1);
 	CUDA_TRY(cudaMemsetAsync(p.n_chains, 0, (size_t)(R + 1) * 4 * 3, st));
 	const int grid = c->n_sm * c->pl_bps, n_warps = grid * PL_WARPS;
 	const size_t z_cap = (size_t)EMAB_MAX_READ_LEN * 1024;
-	TRY(c->b[16].ensure((size_t)n_warps * z_cap));
-	TRY(c->b[17].ensure((size_t)n_warps * EMAB_MAX_CIGAR * 4));
+	TRY(c->bt_z.ensure((size_t)n_warps * z_cap));
+	TRY(c->bt_cigar.ensure((size_t)n_warps * EMAB_MAX_CIGAR * 4));
 	CUDA_TRY(cudaEventRecord(c->stage_ev[2], st));
-	TRY(c->b[42].ensure(Tn * 8));
-	k_sa_gather<<<(R * 32 + 255) / 256, 256, 0, st>>>(ix, R, c->b[1].as<int64_t>(), c->b[2].as<Intv>(), max_intv, c->b[3].as<int32_t>(), d_occ_off, c->b[42].as<int64_t>());
-	k_chain<<<(R + 127) / 128, 128, 0, st>>>(ix, R, c->b[1].as<int64_t>(), c->b[2].as<Intv>(), max_intv, c->b[3].as<int32_t>(), d_occ_off, p, c->b[42].as<int64_t>());
+	TRY(c->sa_vals.ensure(Tn * 8));
+	k_sa_gather<<<(R * 32 + 255) / 256, 256, 0, st>>>(ix, R, c->read_off.as<int64_t>(), c->intv.as<Intv>(), max_intv, c->n_intv.as<int32_t>(), d_occ_off, c->sa_vals.as<int64_t>());
+	k_chain<<<(R + 127) / 128, 128, 0, st>>>(ix, R, c->read_off.as<int64_t>(), c->intv.as<Intv>(), max_intv, c->n_intv.as<int32_t>(), d_occ_off, p, c->sa_vals.as<int64_t>());
 	++launches;
 	CUDA_TRY(cudaEventRecord(c->stage_ev[3], st));
 	if (c->sw_mode == 2) {  // thread-per-read mem_align1_core: wins only when a batch holds many more reads than the GPU has lanes
@@ -668,35 +667,35 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 		per_sm = per_sm > 32 ? 32 : (per_sm < 1 ? 1 : per_sm);
 		int lgrid = c->n_sm * per_sm;
 		if (lgrid > (R + 31) / 32) lgrid = (R + 31) / 32;
-		k_align1_lanes<<<lgrid, 32, smem, st>>>(ix, R, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p, d_err, c->d_counters);
+		k_align1_lanes<<<lgrid, 32, smem, st>>>(ix, R, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p, d_err, c->d_counters);
 	} else {
 		const ExtPlan *d_plans = nullptr;
 		const int32_t *d_chain_off = nullptr;
 		if (c->ext_plan) {
 			// every chain's top-seed extensions ahead of the per-read control flow: plan, two waves (ext_wave.cuh)
-			TRY(c->b[32].ensure((size_t)(R + 1) * 4));
-			int32_t *chain_off = c->b[32].as<int32_t>();
+			TRY(c->chain_off.ensure((size_t)(R + 1) * 4));
+			int32_t *chain_off = c->chain_off.as<int32_t>();
 			cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, p.n_chains, chain_off, R + 1, st);
-			TRY(c->b[6].ensure(tmp_bytes + 16));
-			cub::DeviceScan::ExclusiveSum(c->b[6].p, tmp_bytes, p.n_chains, chain_off, R + 1, st);
+			TRY(c->cub_tmp.ensure(tmp_bytes + 16));
+			cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tmp_bytes, p.n_chains, chain_off, R + 1, st);
 			int32_t NCH = 0;
 			CUDA_TRY(cudaMemcpyAsync(&NCH, chain_off + R, 4, cudaMemcpyDeviceToHost, st));
 			CUDA_TRY(ctx_wait(c));
 			++launches;
 			if (NCH > 0) {
-				TRY(c->b[33].ensure((size_t)NCH * sizeof(ExtPlan)));
-				TRY(c->b[34].ensure((size_t)NCH * 4 + 64));           // lkey, rkey, and their sorted copies
-				TRY(c->b[35].ensure((size_t)NCH * 4 * 4 + 64));       // iota x2, order_l, order_r
-				ExtPlan *plans = c->b[33].as<ExtPlan>();
-				uint8_t *lkey = c->b[34].as<uint8_t>(), *rkey = lkey + NCH, *lkey_s = rkey + NCH, *rkey_s = lkey_s + NCH;
-				int32_t *iota_l = c->b[35].as<int32_t>(), *iota_r = iota_l + NCH, *order_l = iota_r + NCH, *order_r = order_l + NCH;
-				k_ext_plan<Pools><<<(R + 127) / 128, 128, 0, st>>>(ix, R, c->b[1].as<int64_t>(), d_occ_off, p, chain_off, plans, lkey, rkey);
+				TRY(c->ext_plans.ensure((size_t)NCH * sizeof(ExtPlan)));
+				TRY(c->ext_keys.ensure((size_t)NCH * 4 + 64));       // lkey, rkey, and their sorted copies
+				TRY(c->ext_order.ensure((size_t)NCH * 4 * 4 + 64));  // iota x2, order_l, order_r
+				ExtPlan *plans = c->ext_plans.as<ExtPlan>();
+				uint8_t *lkey = c->ext_keys.as<uint8_t>(), *rkey = lkey + NCH, *lkey_s = rkey + NCH, *rkey_s = lkey_s + NCH;
+				int32_t *iota_l = c->ext_order.as<int32_t>(), *iota_r = iota_l + NCH, *order_l = iota_r + NCH, *order_r = order_l + NCH;
+				k_ext_plan<Pools><<<(R + 127) / 128, 128, 0, st>>>(ix, R, c->read_off.as<int64_t>(), d_occ_off, p, chain_off, plans, lkey, rkey);
 				k_iota2<<<(NCH + 255) / 256, 256, 0, st>>>(NCH, iota_l, iota_r);
 				size_t sb = 0;
 				cub::DeviceRadixSort::SortPairsDescending(nullptr, sb, lkey, lkey_s, iota_l, order_l, NCH, 0, 8, st);
-				TRY(c->b[6].ensure(sb + 16));
-				cub::DeviceRadixSort::SortPairsDescending(c->b[6].p, sb, lkey, lkey_s, iota_l, order_l, NCH, 0, 8, st);
-				cub::DeviceRadixSort::SortPairsDescending(c->b[6].p, sb, rkey, rkey_s, iota_r, order_r, NCH, 0, 8, st);
+				TRY(c->cub_tmp.ensure(sb + 16));
+				cub::DeviceRadixSort::SortPairsDescending(c->cub_tmp.p, sb, lkey, lkey_s, iota_l, order_l, NCH, 0, 8, st);
+				cub::DeviceRadixSort::SortPairsDescending(c->cub_tmp.p, sb, rkey, rkey_s, iota_r, order_r, NCH, 0, 8, st);
 				CUDA_TRY(cudaFuncSetAttribute(k_ext_wave<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
 				CUDA_TRY(cudaFuncSetAttribute(k_ext_wave<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
 				if (getenv("EMAB_EXT_HIST")) {   // measurement aid: how long the planned extensions are (query bases), both sides
@@ -716,8 +715,8 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 				// (Two length classes side by side on a second stream, the short one with a quarter of the shared memory, were
 				// measured too — 0.97 -> 1.02 ms: the waves are bound by their longest lanes, not by resident warps.)
 				const size_t smem = lanes::smem_per_warp(max_len);
-				k_ext_wave<false><<<(NCH + 31) / 32, 32, smem, st>>>(ix, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), plans, order_l, lkey_s, NCH, &c->d_counters[12], 0, 255);
-				k_ext_wave<true><<<(NCH + 31) / 32, 32, smem, st>>>(ix, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), plans, order_r, rkey_s, NCH, &c->d_counters[12], 0, 255);
+				k_ext_wave<false><<<(NCH + 31) / 32, 32, smem, st>>>(ix, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), plans, order_l, lkey_s, NCH, &c->d_counters[12], 0, 255);
+				k_ext_wave<true><<<(NCH + 31) / 32, 32, smem, st>>>(ix, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), plans, order_r, rkey_s, NCH, &c->d_counters[12], 0, 255);
 				launches += 2;
 				CUDA_TRY(cudaEventRecord(c->stage_ev[9], st));
 				launches += 4;
@@ -733,10 +732,10 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 			per_sm = per_sm > 32 ? 32 : (per_sm < 1 ? 1 : per_sm);
 			int lgrid = c->n_sm * per_sm;
 			if (lgrid > (R + 31) / 32) lgrid = (R + 31) / 32;
-			k_align1_replay<<<lgrid, 32, smem, st>>>(ix, R, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p, d_err, c->d_counters, d_plans, d_chain_off);
+			k_align1_replay<<<lgrid, 32, smem, st>>>(ix, R, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p, d_err, c->d_counters, d_plans, d_chain_off);
 		} else
-		k_align1<<<grid, PL_WARPS * 32, 0, st>>>(ix, R, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p, c->b[16].as<uint8_t>(), z_cap,
-		                                          c->b[17].as<uint32_t>(), d_err, c->d_counters, d_plans, d_chain_off);
+		k_align1<<<grid, PL_WARPS * 32, 0, st>>>(ix, R, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p, c->bt_z.as<uint8_t>(), z_cap,
+		                                          c->bt_cigar.as<uint32_t>(), d_err, c->d_counters, d_plans, d_chain_off);
 	}
 	launches += 2;
 	CUDA_TRY(cudaEventRecord(c->stage_ev[4], st));
@@ -745,22 +744,22 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 		int32_t *task_beg = nullptr, *task_n = nullptr;
 		if (c->rescue_plan) {
 			const int task_cap = 4 * n_pairs + 4096;
-			TRY(c->b[28].ensure((size_t)task_cap * sizeof(RescueTask)));   // slots 25-26 belong to launch_seed
-			TRY(c->b[29].ensure((size_t)n_pairs * 4 * 2));
-			tasks = c->b[28].as<RescueTask>(); task_beg = c->b[29].as<int32_t>(); task_n = task_beg + n_pairs;
-			k_rescue_plan<<<(n_pairs + 127) / 128, 128, 0, st>>>(ix, n_pairs, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p,
+			TRY(c->rescue_tasks.ensure((size_t)task_cap * sizeof(RescueTask)));
+			TRY(c->rescue_spans.ensure((size_t)n_pairs * 4 * 2));
+			tasks = c->rescue_tasks.as<RescueTask>(); task_beg = c->rescue_spans.as<int32_t>(); task_n = task_beg + n_pairs;
+			k_rescue_plan<<<(n_pairs + 127) / 128, 128, 0, st>>>(ix, n_pairs, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p,
 			                                                    tasks, task_cap, task_beg, task_n, c->d_counters);
 			k_rescue_sw<<<grid, PL_WARPS * 32, 0, st>>>(ix, tasks, task_cap, d_err, c->d_counters);
 			launches += 2;
 		}
-		k_rescue<<<grid, PL_WARPS * 32, 0, st>>>(ix, n_pairs, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p, c->b[16].as<uint8_t>(), z_cap,
-		                                          c->b[17].as<uint32_t>(), d_err, c->d_counters, tasks, task_beg, task_n);
+		k_rescue<<<grid, PL_WARPS * 32, 0, st>>>(ix, n_pairs, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p, c->bt_z.as<uint8_t>(), z_cap,
+		                                          c->bt_cigar.as<uint32_t>(), d_err, c->d_counters, tasks, task_beg, task_n);
 		++launches;
 	}
 	CUDA_TRY(cudaEventRecord(c->stage_ev[5], st));
 	cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, p.n_regs, d_aln_off, R + 1, st);
-	TRY(c->b[6].ensure(tmp_bytes + 16));
-	cub::DeviceScan::ExclusiveSum(c->b[6].p, tmp_bytes, p.n_regs, d_aln_off, R + 1, st);
+	TRY(c->cub_tmp.ensure(tmp_bytes + 16));
+	cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tmp_bytes, p.n_regs, d_aln_off, R + 1, st);
 	++launches;
 	int32_t A = 0;
 	CUDA_TRY(cudaMemcpyAsync(&A, d_aln_off + R, 4, cudaMemcpyDeviceToHost, st));
@@ -769,99 +768,99 @@ static int align_pairs_core(emab_ctx_t *c, int n_pairs, int max_len, int64_t tot
 	int32_t NC = 0;
 	CUDA_TRY(cudaEventRecord(c->stage_ev[6], st));
 	if (stage >= 3) {
-		TRY(c->b[18].ensure(((size_t)A + 1) * sizeof(Aln)));
+		TRY(c->alns.ensure(((size_t)A + 1) * sizeof(Aln)));
 		const GlobTask *d_gtasks = nullptr;
 		const uint32_t *d_gcigars = nullptr;
 		if (c->glob_plan && A > 0) {
 			// the first ksw_global2 of every region ahead of the per-pair control flow (glob_wave.cuh)
-			TRY(c->b[36].ensure((size_t)A * sizeof(GlobTask)));
-			TRY(c->b[37].ensure((size_t)A * 2 * 2 + (size_t)A * 4 * 2 + 64));      // keys, sorted keys | iota, order
+			TRY(c->glob_tasks.ensure((size_t)A * sizeof(GlobTask)));
+			TRY(c->glob_keys.ensure((size_t)A * 2 * 2 + (size_t)A * 4 * 2 + 64));   // keys, sorted keys | iota, order
 			const int n_gwarps = (A + 31) / 32;
-			TRY(c->b[38].ensure(((size_t)n_gwarps + 1) * 8 * 2 + 16));              // per-warp z size, z offset, k_glob_wide's task counter
-			TRY(c->b[39].ensure((size_t)A * EMAB_MAX_CIGAR * 4));
-			GlobTask *gt = c->b[36].as<GlobTask>();
-			int32_t *g_iota = c->b[37].as<int32_t>(), *g_order = g_iota + A;
+			TRY(c->glob_zoff.ensure(((size_t)n_gwarps + 1) * 8 * 2 + 16));         // per-warp z size, z offset, k_glob_wide's task counter
+			TRY(c->glob_cigars.ensure((size_t)A * EMAB_MAX_CIGAR * 4));
+			GlobTask *gt = c->glob_tasks.as<GlobTask>();
+			int32_t *g_iota = c->glob_keys.as<int32_t>(), *g_order = g_iota + A;
 			uint16_t *g_keys = (uint16_t *)(g_order + A), *g_keys_s = g_keys + A;
-			unsigned long long *zsize = c->b[38].as<unsigned long long>(), *zoff = zsize + (n_gwarps + 1);
+			unsigned long long *zsize = c->glob_zoff.as<unsigned long long>(), *zoff = zsize + (n_gwarps + 1);
 			CUDA_TRY(cudaMemsetAsync(zsize + n_gwarps, 0, 8, st));
 			unsigned long long *wide_queue = zoff + (n_gwarps + 1);
 			CUDA_TRY(cudaMemsetAsync(wide_queue, 0, 8, st));
-			k_glob_plan<Pools><<<(R + 127) / 128, 128, 0, st>>>(ix, R, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p, RESCUE_ROOM, d_aln_off, gt, g_keys);
+			k_glob_plan<Pools><<<(R + 127) / 128, 128, 0, st>>>(ix, R, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p, RESCUE_ROOM, d_aln_off, gt, g_keys);
 			k_iota1<<<(A + 255) / 256, 256, 0, st>>>(A, g_iota);
 			size_t sb = 0;
 			cub::DeviceRadixSort::SortPairsDescending(nullptr, sb, g_keys, g_keys_s, g_iota, g_order, A, 0, 16, st);
-			TRY(c->b[6].ensure(sb + 16));
-			cub::DeviceRadixSort::SortPairsDescending(c->b[6].p, sb, g_keys, g_keys_s, g_iota, g_order, A, 0, 16, st);
+			TRY(c->cub_tmp.ensure(sb + 16));
+			cub::DeviceRadixSort::SortPairsDescending(c->cub_tmp.p, sb, g_keys, g_keys_s, g_iota, g_order, A, 0, 16, st);
 			// bands of wide_cols columns or more go to the warp-per-task kernel (at most the ring: EMAB_GLOB_WIDE_COLS is a tuning knob)
 			static const int wide_cols = [] { const char *e = getenv("EMAB_GLOB_WIDE_COLS"); int v = e ? atoi(e) : GLOB_WIDE_COLS; return v < 2 ? 2 : (v > GLOB_RING_COLS ? GLOB_RING_COLS : v); }();
 			k_glob_zsize<<<(n_gwarps + 127) / 128, 128, 0, st>>>(gt, g_order, g_keys_s, A, zsize, n_gwarps, wide_cols);
 			cub::DeviceScan::ExclusiveSum(nullptr, sb, zsize, zoff, n_gwarps + 1, st);
-			TRY(c->b[6].ensure(sb + 16));
-			cub::DeviceScan::ExclusiveSum(c->b[6].p, sb, zsize, zoff, n_gwarps + 1, st);
+			TRY(c->cub_tmp.ensure(sb + 16));
+			cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, sb, zsize, zoff, n_gwarps + 1, st);
 			unsigned long long Z = 0;
 			CUDA_TRY(cudaMemcpyAsync(&Z, zoff + n_gwarps, 8, cudaMemcpyDeviceToHost, st));
 			CUDA_TRY(ctx_wait(c));
-			TRY(c->b[40].ensure((size_t)Z + 64));
+			TRY(c->glob_z.ensure((size_t)Z + 64));
 			CUDA_TRY(cudaFuncSetAttribute(k_glob_wave, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
 			CUDA_TRY(cudaEventRecord(c->stage_ev[10], st));
 			// narrow bands (up to GLOB_RING_COLS - 1 columns): one THREAD per task, the DP row a 32-column ring (13 KB of shared
 			// memory per warp instead of 28); wide bands: one WARP per task, beside it on the ctx's second stream
 			TRY(ctx_fork(c));
-			k_glob_wave<<<n_gwarps, 32, glob_smem_bytes(max_len, GLOB_RING_COLS), st>>>(ix, gt, g_order, g_keys_s, A, zoff, c->b[40].as<uint8_t>(),
-			                                                          c->b[39].as<uint32_t>(), &c->d_counters[14], max_len, GLOB_RING_COLS, 0, wide_cols - 1);
-			k_glob_wide<<<grid, PL_WARPS * 32, 0, c->stream2>>>(ix, gt, g_order, g_keys_s, A, c->b[39].as<uint32_t>(), c->b[16].as<uint8_t>(), z_cap,
-			                                                    c->b[17].as<uint32_t>(), &c->d_counters[14], wide_queue, wide_cols);
+			k_glob_wave<<<n_gwarps, 32, glob_smem_bytes(max_len, GLOB_RING_COLS), st>>>(ix, gt, g_order, g_keys_s, A, zoff, c->glob_z.as<uint8_t>(),
+			                                                          c->glob_cigars.as<uint32_t>(), &c->d_counters[14], max_len, GLOB_RING_COLS, 0, wide_cols - 1);
+			k_glob_wide<<<grid, PL_WARPS * 32, 0, c->stream2>>>(ix, gt, g_order, g_keys_s, A, c->glob_cigars.as<uint32_t>(), c->bt_z.as<uint8_t>(), z_cap,
+			                                                    c->bt_cigar.as<uint32_t>(), &c->d_counters[14], wide_queue, wide_cols);
 			TRY(ctx_join(c));
 			++launches;
 			CUDA_TRY(cudaEventRecord(c->stage_ev[11], st));
 			launches += 6;
-			d_gtasks = gt; d_gcigars = c->b[39].as<uint32_t>(); glob_waves_ran = true;
+			d_gtasks = gt; d_gcigars = c->glob_cigars.as<uint32_t>(); glob_waves_ran = true;
 		}
-		k_finalize<<<grid, PL_WARPS * 32, 0, st>>>(ix, n_pairs, c->b[0].as<uint8_t>(), c->b[1].as<int64_t>(), d_occ_off, p, d_aln_off, c->b[18].as<Aln>(),
-		                                            c->b[23].as<ScoreConsts>(), c->b[16].as<uint8_t>(), z_cap, c->b[17].as<uint32_t>(), d_err, c->d_counters,
+		k_finalize<<<grid, PL_WARPS * 32, 0, st>>>(ix, n_pairs, c->reads.as<uint8_t>(), c->read_off.as<int64_t>(), d_occ_off, p, d_aln_off, c->alns.as<Aln>(),
+		                                            c->consts.as<ScoreConsts>(), c->bt_z.as<uint8_t>(), z_cap, c->bt_cigar.as<uint32_t>(), d_err, c->d_counters,
 		                                            d_gtasks, d_gcigars);
 		++launches;
 		// compact wire format: 56-byte records + CIGAR pool
-		TRY(c->b[20].ensure(((size_t)A + 2) * 4 * 2));
-		int32_t *d_ncig = c->b[20].as<int32_t>(), *d_cig_off = d_ncig + (A + 2);
-		k_ncigar<<<(A + 256) / 256, 256, 0, st>>>(A, c->b[18].as<Aln>(), d_ncig);
+		TRY(c->cig_off.ensure(((size_t)A + 2) * 4 * 2));
+		int32_t *d_ncig = c->cig_off.as<int32_t>(), *d_cig_off = d_ncig + (A + 2);
+		k_ncigar<<<(A + 256) / 256, 256, 0, st>>>(A, c->alns.as<Aln>(), d_ncig);
 		cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_ncig, d_cig_off, A + 1, st);
-		TRY(c->b[6].ensure(tmp_bytes + 16));
-		cub::DeviceScan::ExclusiveSum(c->b[6].p, tmp_bytes, d_ncig, d_cig_off, A + 1, st);
-		TRY(c->b[21].ensure(((size_t)A + 1) * sizeof(emab_cand_t)));
-		TRY(c->b[19].ensure(((size_t)A + 1) * EMAB_MAX_CIGAR * 4));  // upper bound; only the used prefix is copied back
-		k_pack<<<(A + 255) / 256, 256, 0, st>>>(A, c->b[18].as<Aln>(), d_cig_off, c->b[21].as<emab_cand_t>(), c->b[19].as<uint32_t>());
+		TRY(c->cub_tmp.ensure(tmp_bytes + 16));
+		cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tmp_bytes, d_ncig, d_cig_off, A + 1, st);
+		TRY(c->cands.ensure(((size_t)A + 1) * sizeof(emab_cand_t)));
+		TRY(c->cigars.ensure(((size_t)A + 1) * EMAB_MAX_CIGAR * 4));  // upper bound; only the used prefix is copied back
+		k_pack<<<(A + 255) / 256, 256, 0, st>>>(A, c->alns.as<Aln>(), d_cig_off, c->cands.as<emab_cand_t>(), c->cigars.as<uint32_t>());
 		launches += 3;
 		CUDA_TRY(cudaEventRecord(c->ev1, st));
 		CUDA_TRY(cudaEventRecord(c->stage_ev[7], st));
 		CUDA_TRY(cudaMemcpyAsync(&NC, d_cig_off + A, 4, cudaMemcpyDeviceToHost, st));
 		CUDA_TRY(ctx_wait(c));
-		TRY(c->h[1].ensure(((size_t)A + 1) * sizeof(emab_cand_t)));
-		TRY(c->h[2].ensure(((size_t)NC + 1) * 4));
-		if (A) CUDA_TRY(cudaMemcpyAsync(c->h[1].p, c->b[21].p, (size_t)A * sizeof(emab_cand_t), cudaMemcpyDeviceToHost, st));
-		if (NC && want_cigars) CUDA_TRY(cudaMemcpyAsync(c->h[2].p, c->b[19].p, (size_t)NC * 4, cudaMemcpyDeviceToHost, st));
+		TRY(c->h_cands.ensure(((size_t)A + 1) * sizeof(emab_cand_t)));
+		TRY(c->h_cigars.ensure(((size_t)NC + 1) * 4));
+		if (A) CUDA_TRY(cudaMemcpyAsync(c->h_cands.p, c->cands.p, (size_t)A * sizeof(emab_cand_t), cudaMemcpyDeviceToHost, st));
+		if (NC && want_cigars) CUDA_TRY(cudaMemcpyAsync(c->h_cigars.p, c->cigars.p, (size_t)NC * 4, cudaMemcpyDeviceToHost, st));
 	} else {
 		CUDA_TRY(cudaEventRecord(c->ev1, st));
 		CUDA_TRY(cudaEventRecord(c->stage_ev[7], st));
 	}
 	if (want_regs) {
-		TRY(c->b[24].ensure(((size_t)A + 1) * 18 * 8));
-		TRY(c->h[3].ensure(((size_t)A + 1) * 18 * 8));
-		k_export_regs<<<(R + 127) / 128, 128, 0, st>>>(R, d_occ_off, d_aln_off, p, c->b[24].as<int64_t>());
-		CUDA_TRY(cudaMemcpyAsync(c->h[3].p, c->b[24].p, (size_t)A * 18 * 8, cudaMemcpyDeviceToHost, st));
+		TRY(c->regs_export.ensure(((size_t)A + 1) * 18 * 8));
+		TRY(c->h_regs_dbg.ensure(((size_t)A + 1) * 18 * 8));
+		k_export_regs<<<(R + 127) / 128, 128, 0, st>>>(R, d_occ_off, d_aln_off, p, c->regs_export.as<int64_t>());
+		CUDA_TRY(cudaMemcpyAsync(c->h_regs_dbg.p, c->regs_export.p, (size_t)A * 18 * 8, cudaMemcpyDeviceToHost, st));
 	}
-	TRY(c->h[0].ensure((size_t)R * 4 + 256));
-	CUDA_TRY(cudaMemcpyAsync(c->h[0].p, p.n_regs, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
-	int *h_err = (int *)((char *)c->h[0].p + (size_t)R * 4);
-	unsigned long long *cnt = (unsigned long long *)((char *)c->h[0].p + (((size_t)R * 4 + 16 + 7) & ~(size_t)7));
+	TRY(c->h_n_regs.ensure((size_t)R * 4 + 256));
+	CUDA_TRY(cudaMemcpyAsync(c->h_n_regs.p, p.n_regs, (size_t)R * 4, cudaMemcpyDeviceToHost, st));
+	int *h_err = (int *)((char *)c->h_n_regs.p + (size_t)R * 4);
+	unsigned long long *cnt = (unsigned long long *)((char *)c->h_n_regs.p + (((size_t)R * 4 + 16 + 7) & ~(size_t)7));
 	CUDA_TRY(cudaMemcpyAsync(h_err, d_err, 16, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(cudaMemcpyAsync(cnt, c->d_counters, 128, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	CUDA_TRY(cudaGetLastError());
-	res->n_cands = A; res->n_cigar_ops = NC; res->n_regs = (const int32_t *)c->h[0].p;
-	res->cands = stage >= 3 ? (const emab_cand_t *)c->h[1].p : nullptr;
-	res->cigars = stage >= 3 && want_cigars ? (const uint32_t *)c->h[2].p : nullptr;
-	res->regs_dbg = want_regs ? (const int64_t *)c->h[3].p : nullptr;
+	res->n_cands = A; res->n_cigar_ops = NC; res->n_regs = (const int32_t *)c->h_n_regs.p;
+	res->cands = stage >= 3 ? (const emab_cand_t *)c->h_cands.p : nullptr;
+	res->cigars = stage >= 3 && want_cigars ? (const uint32_t *)c->h_cigars.p : nullptr;
+	res->regs_dbg = want_regs ? (const int64_t *)c->h_regs_dbg.p : nullptr;
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 	c->last_ms = ms; c->last_launches = launches;
 	if (stats) {

@@ -4,48 +4,49 @@
 #include <vector>
 #include "common.cuh"
 
-struct DevBuf {  // grow-only device buffer
+// Grow-only buffer over an allocate/free pair.  ensure() drops the contents when it has to grow.  The buffer owns its
+// memory: it is freed on destruction, and a buffer can be moved but not copied.
+template <class Mem> struct GrowBuf {
 	void *p = nullptr;
 	size_t cap = 0;
+	GrowBuf() = default;
+	GrowBuf(const GrowBuf &) = delete;
+	GrowBuf &operator=(const GrowBuf &) = delete;
+	GrowBuf &operator=(GrowBuf &&o) noexcept
+	{
+		if (this != &o) { release(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+		return *this;
+	}
+	~GrowBuf() { release(); }
 	int ensure(size_t bytes)
 	{
 		if (bytes <= cap) return EMAB_OK;
-		if (p) cudaFree(p);
-		p = nullptr; cap = 0;
+		release();
 		size_t want = bytes + bytes / 4 + 256;
-		cudaError_t e = cudaMalloc(&p, want);
+		cudaError_t e = Mem::alloc(&p, want);
 		if (e != cudaSuccess) {
-			snprintf(emab_errbuf, sizeof emab_errbuf, "cudaMalloc(%zu) failed: %s", want, cudaGetErrorString(e));
+			snprintf(emab_errbuf, sizeof emab_errbuf, "%s(%zu) failed: %s", Mem::name, want, cudaGetErrorString(e));
 			p = nullptr;
 			return EMAB_ERR_NOMEM;
 		}
 		cap = want;
 		return EMAB_OK;
 	}
-	void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+	void release() { if (p) Mem::free(p); p = nullptr; cap = 0; }
 	template <class T> T *as() const { return (T *)p; }
 };
-
-struct HostBuf {  // grow-only pinned host buffer
-	void *p = nullptr;
-	size_t cap = 0;
-	int ensure(size_t bytes)
-	{
-		if (bytes <= cap) return EMAB_OK;
-		if (p) cudaFreeHost(p);
-		p = nullptr; cap = 0;
-		size_t want = bytes + bytes / 4 + 256;
-		cudaError_t e = cudaMallocHost(&p, want);
-		if (e != cudaSuccess) {
-			snprintf(emab_errbuf, sizeof emab_errbuf, "cudaMallocHost(%zu) failed: %s", want, cudaGetErrorString(e));
-			p = nullptr;
-			return EMAB_ERR_NOMEM;
-		}
-		cap = want;
-		return EMAB_OK;
-	}
-	void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
+struct DeviceMem {
+	static constexpr const char *name = "cudaMalloc";
+	static cudaError_t alloc(void **p, size_t n) { return cudaMalloc(p, n); }
+	static void free(void *p) { cudaFree(p); }
 };
+struct PinnedMem {
+	static constexpr const char *name = "cudaMallocHost";
+	static cudaError_t alloc(void **p, size_t n) { return cudaMallocHost(p, n); }
+	static void free(void *p) { cudaFreeHost(p); }
+};
+using DevBuf = GrowBuf<DeviceMem>;    // device memory
+using HostBuf = GrowBuf<PinnedMem>;   // page-locked host memory
 
 struct emab_index {
 	int device = 0;
@@ -76,31 +77,68 @@ struct emab_ctx {
 	int spin_us = 150;               // how long mode 0 polls before it starts sleeping (EMAB_SPIN_US)
 	double last_ms = 0;
 	int last_launches = 0;
-	DevBuf b[52];            // device scratch slots, meaning assigned by each entry point
-	HostBuf h[8];            // pinned host result buffers, owned by the ctx and valid until its next call
 	unsigned long long *d_counters = nullptr;  // 16 x u64 instrumentation / work counters
 	int n_sm = 148;
 	int pl_bps = 4;          // blocks per SM of the persistent warp-per-read kernels (EMAB_PL_BPS)
-	// resident SW microbench inputs
-	int res_n = 0, res_qcap = 0;
 	int sw_mode = 0;         // see emab_set_sw_mode (include/ema_b200.h)
 	int seed_mode = 0;       // see emab_set_seed_mode; 0 = EMAB_SEED_MODE or the default
 	bool rescue_plan = true; // mate-rescue alignments planned and run as one balanced batch (pipeline.cu, k_rescue_plan)
 	bool ext_plan = true;    // ksw_extend2 calls of every chain's top seed run ahead as two bucket-wide waves (ext_wave.cuh)
 	bool glob_plan = true;   // ksw_global2 calls of mem_reg2aln likewise (glob_wave.cuh)
 	bool replay_lanes = true; // the extension replay walks one read per THREAD (k_align1_replay) instead of per warp
-	bool consts_ready = false;
-	bool em_log_ready = false; // emab_em_batch's ln(n) table is resident (slot 30)
-	bool text_ready = false;   // the batch's text + pair table are resident (slots 31, 27: emab_align_pairs_text / emab_parse_bucket)
+
+	// ---- Held buffers: results that outlive the call that wrote them.  Each sits next to what says it is valid, and
+	// only the calls named with it write it.
+	// The batch, written by emab_parse_bucket and emab_align_pairs_text (emab_align_pairs clears text_ready): its text and
+	// pair table on the device, read by emab_align_pairs_resident and the formatters; the page-locked pair table and
+	// barcodes emab_parse_bucket hands out.
+	bool text_ready = false;
 	unsigned text_len = 0;
 	int text_pairs = 0;
-	bool sam_tables_ready = false;  // contig names + rid -> name map resident (slot 45: emab_sam_tables)
+	DevBuf text, pairs;
+	HostBuf h_parsed;
+	// The pipeline's results, written by the emab_align_pairs* calls: candidates and CIGAR pool on the device, which the
+	// formatters read (emab_sam_rec_t refers to candidates by index), and the host arrays of emab_pairs_result_t (h_n_regs
+	// is followed by the call's error flags and counters).  Valid until the next emab_align_pairs* or emab_parse_bucket.
+	DevBuf cands, cigars;
+	HostBuf h_n_regs, h_cands, h_cigars, h_regs_dbg;
+	bool consts_ready = false;      // score constants (emab_set_error_rate, or the first align call)
+	DevBuf consts;
+	bool em_log_ready = false;      // emab_em_batch's ln(n) table
+	DevBuf em_log;
+	bool sam_tables_ready = false;  // contig names, offsets, rid -> name and name -> @SQ maps (emab_sam_tables)
+	DevBuf sam_tables;
 	size_t sam_chrom_off = 0, sam_rid_off = 0, sam_sq_off = 0;
 	std::string bam_unmapped_contig; // a contig of the index whose .fai name no @SQ entry has (BAM refuses then); empty: none
+	// The resident SW microbench (emab_extend_resident_load; emab_extend_resident_run writes res_out).  Only the load
+	// allocates them, so a ctx that never runs it holds none.
+	int res_n = 0, res_qcap = 0;
+	DevBuf res_q, res_qoff, res_t, res_toff, res_h0, res_out, res_order;
+
+	// ---- Scratch buffers: dead when the call returns.  Named for what the pipeline keeps in them.  Other entry points
+	// borrow them under names of their own, bound at the top of the function, so a ctx's footprint stays that of its
+	// largest call.
+	DevBuf reads, read_off;                 // nt4 reads and their offsets
+	DevBuf intv, n_intv, occ;               // SA intervals per read, their counts, occurrence counts | offsets
+	DevBuf seed_lanes, seed_p3, seed_queue, packed_reads, seed_prof;   // launch_seed's
+	DevBuf sa_vals;                         // SA values of every occurrence
+	DevBuf w_seeds, w_chains, w_nodes, w_ord, seeds, chains, srt, regs, reg_counts;   // the Pools of chaining and alignment
+	DevBuf bt_z, bt_cigar;                  // per-warp backtrack matrices and CIGAR scratch
+	DevBuf chain_off, ext_plans, ext_keys, ext_order;                   // extension waves
+	DevBuf rescue_tasks, rescue_spans;      // planned mate rescue
+	DevBuf alns, glob_tasks, glob_keys, glob_zoff, glob_cigars, glob_z; // finalize and its global-alignment waves
+	DevBuf cig_off, regs_export;            // packing the candidates; want_regs
+	DevBuf err;                             // device error flags
+	DevBuf cub_tmp;                         // cub temp storage of every caller (the stream is in order: a regrown buffer waits for the work before it)
+	DevBuf em_cov;                          // emab_em_batch's per-cloud arrays
+	HostBuf em_stage, em_gamma;             // emab_em_batch's input block and result
+	DevBuf sam_job, rec_off;                // the formatters' job (descriptors, barcodes) and record offsets
+	HostBuf job_stage;
+	DevBuf bgzf_tokens, bgzf_members, bgzf_off, bgzf_out;   // bgzf_compress_device's
 };
 
 // BGZF members of d_in[0..n) (device memory) into the host buffer out (bgzf.cu); records ev1 after the last kernel.
-// Slots 48-51.  *launches = kernels launched.  d_member_off (optional) receives a device pointer to the members' offsets in
+// Uses the ctx's bgzf_* scratch.  *launches = kernels launched.  d_member_off (optional) receives a device pointer to the members' offsets in
 // out (one per chunk, then the total), valid until the ctx's next call.
 int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches,
                          const unsigned long long **d_member_off = nullptr);

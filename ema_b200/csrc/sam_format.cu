@@ -401,8 +401,11 @@ __global__ void k_bam_key(SamTables t, const emab_sam_rec_t *recs, int n, const 
 
 }  // namespace
 
-// slots: 45 chrom tables (per ctx, once), 46 record descriptors + barcode strings, 47 lengths/offsets, 33.. free after the
-// pipeline (the ExtPlan slot is reused for the output text: it is the largest buffer that is dead by now)
+// The formatters read the batch's text and pair table and the pipeline's candidates and CIGAR pool, all held by the ctx;
+// their own scratch is the job (sam_job), the record offsets (rec_off) and the record text, which goes to the pipeline's
+// extension plans: the largest buffer that is dead once the batch is aligned.
+static DevBuf &rec_text(emab_ctx *c) { return c->ext_plans; }
+
 extern "C" int emab_sam_tables(emab_ctx_t *c, int n_chrom, const char *const *names, int n_rid, const int32_t *rid2chrom)
 {
 	CTX_ENTER(c);
@@ -428,13 +431,13 @@ extern "C" int emab_sam_tables(emab_ctx_t *c, int n_chrom, const char *const *na
 	memcpy(blob.data() + o_off, off.data(), off.size() * 4);
 	if (n_rid) memcpy(blob.data() + o_rid, rid2chrom, (size_t)n_rid * 4);
 	if (n_chrom) memcpy(blob.data() + o_sq, chrom2sq.data(), (size_t)n_chrom * 4);
-	TRY(c->b[45].ensure(total + 16));
-	CUDA_TRY(cudaMemcpy(c->b[45].p, blob.data(), total, cudaMemcpyHostToDevice));
+	TRY(c->sam_tables.ensure(total + 16));
+	CUDA_TRY(cudaMemcpy(c->sam_tables.p, blob.data(), total, cudaMemcpyHostToDevice));
 	c->sam_chrom_off = o_off; c->sam_rid_off = o_rid; c->sam_sq_off = o_sq; c->sam_tables_ready = true;
 	return EMAB_OK;
 }
 
-// uploads the job's descriptors and barcode strings (slot 46) and fills the tables the emitters read
+// uploads the job's descriptors and barcode strings and fills the tables the emitters read
 static int stage_job(emab_ctx_t *c, const emab_sam_job_t *job, SamTables &t)
 {
 	const int n = job->n_recs;
@@ -442,23 +445,23 @@ static int stage_job(emab_ctx_t *c, const emab_sam_job_t *job, SamTables &t)
 	// one staging block: descriptors | barcode offsets | barcode text
 	const size_t b_recs = (size_t)n * sizeof(emab_sam_rec_t), o_bcoff = (b_recs + 15) & ~(size_t)15, b_bcoff = (size_t)(job->n_bc + 1) * 4,
 	             o_bctext = o_bcoff + ((b_bcoff + 15) & ~(size_t)15), b_bctext = (size_t)job->bc_off[job->n_bc], total = o_bctext + b_bctext;
-	TRY(c->h[6].ensure(total + 16));
-	memcpy(c->h[6].p, job->recs, b_recs);
-	memcpy((char *)c->h[6].p + o_bcoff, job->bc_off, b_bcoff);
-	memcpy((char *)c->h[6].p + o_bctext, job->bc_text, b_bctext);
-	TRY(c->b[46].ensure(total + 16));
-	CUDA_TRY(cudaMemcpyAsync(c->b[46].p, c->h[6].p, total, cudaMemcpyHostToDevice, st));
+	TRY(c->job_stage.ensure(total + 16));
+	memcpy(c->job_stage.p, job->recs, b_recs);
+	memcpy((char *)c->job_stage.p + o_bcoff, job->bc_off, b_bcoff);
+	memcpy((char *)c->job_stage.p + o_bctext, job->bc_text, b_bctext);
+	TRY(c->sam_job.ensure(total + 16));
+	CUDA_TRY(cudaMemcpyAsync(c->sam_job.p, c->job_stage.p, total, cudaMemcpyHostToDevice, st));
 	memset(&t, 0, sizeof t);
-	t.text = c->b[31].as<char>();
-	t.pairs = c->b[27].as<emab_pair_text_t>();
-	t.cands = c->b[21].as<emab_cand_t>();
-	t.cigars = c->b[19].as<uint32_t>();
-	t.chrom_names = c->b[45].as<char>();
-	t.chrom_off = (const int32_t *)(c->b[45].as<char>() + c->sam_chrom_off);
-	t.rid2chrom = (const int32_t *)(c->b[45].as<char>() + c->sam_rid_off);
-	t.chrom2sq = (const int32_t *)(c->b[45].as<char>() + c->sam_sq_off);
-	t.bc_off = (const int32_t *)(c->b[46].as<char>() + o_bcoff);
-	t.bc_text = c->b[46].as<char>() + o_bctext;
+	t.text = c->text.as<char>();
+	t.pairs = c->pairs.as<emab_pair_text_t>();
+	t.cands = c->cands.as<emab_cand_t>();
+	t.cigars = c->cigars.as<uint32_t>();
+	t.chrom_names = c->sam_tables.as<char>();
+	t.chrom_off = (const int32_t *)(c->sam_tables.as<char>() + c->sam_chrom_off);
+	t.rid2chrom = (const int32_t *)(c->sam_tables.as<char>() + c->sam_rid_off);
+	t.chrom2sq = (const int32_t *)(c->sam_tables.as<char>() + c->sam_sq_off);
+	t.bc_off = (const int32_t *)(c->sam_job.as<char>() + o_bcoff);
+	t.bc_text = c->sam_job.as<char>() + o_bctext;
 	t.bx_index_len = (int)strnlen(job->bx_index ? job->bx_index : "", sizeof t.bx_index - 1);
 	memcpy(t.bx_index, job->bx_index ? job->bx_index : "", (size_t)t.bx_index_len);
 	t.rg_len = job->rg_id ? (int)strnlen(job->rg_id, sizeof t.rg_id - 1) : -1;
@@ -478,23 +481,24 @@ extern "C" int emab_sam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *o
 	cudaStream_t st = c->stream;
 	SamTables t;
 	TRY(stage_job(c, job, t));
-	const emab_sam_rec_t *d_recs = c->b[46].as<emab_sam_rec_t>();
-	TRY(c->b[47].ensure((size_t)(n + 1) * 8 * 2));
-	unsigned long long *d_len = c->b[47].as<unsigned long long>(), *d_off = d_len + (n + 1);
+	const emab_sam_rec_t *d_recs = c->sam_job.as<emab_sam_rec_t>();
+	TRY(c->rec_off.ensure((size_t)(n + 1) * 8 * 2));
+	unsigned long long *d_len = c->rec_off.as<unsigned long long>(), *d_off = d_len + (n + 1);
 	CUDA_TRY(cudaEventRecord(c->ev0, st));
 	k_sam_len<<<(n + 1 + 127) / 128, 128, 0, st>>>(t, d_recs, n, d_len);
 	size_t tb = 0;
 	cub::DeviceScan::ExclusiveSum(nullptr, tb, d_len, d_off, n + 1, st);
-	TRY(c->b[6].ensure(tb + 16));
-	cub::DeviceScan::ExclusiveSum(c->b[6].p, tb, d_len, d_off, n + 1, st);
+	TRY(c->cub_tmp.ensure(tb + 16));
+	cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tb, d_len, d_off, n + 1, st);
 	unsigned long long total_len = 0;
 	CUDA_TRY(cudaMemcpyAsync(&total_len, d_off + n, 8, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	if (total_len > out_cap) { *out_len = total_len; snprintf(emab_errbuf, sizeof emab_errbuf, "emab_sam_format: %llu bytes do not fit the output buffer", total_len); return EMAB_ERR_OVERFLOW; }
-	TRY(c->b[33].ensure((size_t)total_len + 16));
-	k_sam_write<<<(n * 32 + 255) / 256, 256, 0, st>>>(t, d_recs, n, d_off, c->b[33].as<char>());
+	DevBuf &sam_text = rec_text(c);
+	TRY(sam_text.ensure((size_t)total_len + 16));
+	k_sam_write<<<(n * 32 + 255) / 256, 256, 0, st>>>(t, d_recs, n, d_off, sam_text.as<char>());
 	CUDA_TRY(cudaEventRecord(c->ev1, st));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[33].p, (size_t)total_len, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(out, sam_text.p, (size_t)total_len, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	CUDA_TRY(cudaGetLastError());
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
@@ -503,7 +507,7 @@ extern "C" int emab_sam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *o
 	return EMAB_OK;
 }
 
-// BAM records of a job written to slot 33 (k_bam_len -> scan -> k_bam_write), offsets in slot 47; `fn` names the caller in
+// BAM records of a job written to rec_text (k_bam_len -> scan -> k_bam_write), offsets in rec_off; `fn` names the caller in
 // the messages.  *raw = 0 and nothing launched for an empty job.
 static int bam_records_device(emab_ctx_t *c, const emab_sam_job_t *job, const char *fn, SamTables &t, unsigned long long *raw)
 {
@@ -517,16 +521,16 @@ static int bam_records_device(emab_ctx_t *c, const emab_sam_job_t *job, const ch
 	if (n == 0) return EMAB_OK;
 	cudaStream_t st = c->stream;
 	TRY(stage_job(c, job, t));
-	const emab_sam_rec_t *d_recs = c->b[46].as<emab_sam_rec_t>();
-	TRY(c->b[47].ensure((size_t)(n + 1) * 8 * 2 + 16));
-	unsigned long long *d_len = c->b[47].as<unsigned long long>(), *d_off = d_len + (n + 1), *d_refusal = d_off + (n + 1);
+	const emab_sam_rec_t *d_recs = c->sam_job.as<emab_sam_rec_t>();
+	TRY(c->rec_off.ensure((size_t)(n + 1) * 8 * 2 + 16));
+	unsigned long long *d_len = c->rec_off.as<unsigned long long>(), *d_off = d_len + (n + 1), *d_refusal = d_off + (n + 1);
 	CUDA_TRY(cudaEventRecord(c->ev0, st));
 	CUDA_TRY(cudaMemsetAsync(d_refusal, 0xff, 8, st));
 	k_bam_len<<<(n + 1 + 127) / 128, 128, 0, st>>>(t, d_recs, n, d_len, d_refusal);
 	size_t tb = 0;
 	cub::DeviceScan::ExclusiveSum(nullptr, tb, d_len, d_off, n + 1, st);
-	TRY(c->b[6].ensure(tb + 16));
-	cub::DeviceScan::ExclusiveSum(c->b[6].p, tb, d_len, d_off, n + 1, st);
+	TRY(c->cub_tmp.ensure(tb + 16));
+	cub::DeviceScan::ExclusiveSum(c->cub_tmp.p, tb, d_len, d_off, n + 1, st);
 	unsigned long long hv[2] = {0, 0};   // raw length, refusal
 	CUDA_TRY(cudaMemcpyAsync(&hv[0], d_off + n, 8, cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(cudaMemcpyAsync(&hv[1], d_refusal, 8, cudaMemcpyDeviceToHost, st));
@@ -539,12 +543,12 @@ static int bam_records_device(emab_ctx_t *c, const emab_sam_job_t *job, const ch
 		return EMAB_ERR_ARG;
 	}
 	*raw = hv[0];
-	TRY(c->b[33].ensure((size_t)*raw + 16));
-	k_bam_write<<<(n * 32 + 255) / 256, 256, 0, st>>>(t, d_recs, n, d_off, c->b[33].as<char>());
+	TRY(rec_text(c).ensure((size_t)*raw + 16));
+	k_bam_write<<<(n * 32 + 255) / 256, 256, 0, st>>>(t, d_recs, n, d_off, rec_text(c).as<char>());
 	return EMAB_OK;
 }
 
-// The BAM counterpart: records written to slot 33, compressed into BGZF members (bgzf.cu), only the members copied back.
+// The BAM counterpart: records written to rec_text, compressed into BGZF members (bgzf.cu), only the members copied back.
 extern "C" int emab_bam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len)
 {
 	CTX_ENTER(c);
@@ -555,13 +559,13 @@ extern "C" int emab_bam_format(emab_ctx_t *c, const emab_sam_job_t *job, char *o
 	TRY(bam_records_device(c, job, "emab_bam_format", t, &raw));
 	if (job->n_recs == 0) return EMAB_OK;
 	int launches = 0;
-	TRY(bgzf_compress_device(c, c->b[33].as<uint8_t>(), raw, (uint8_t *)out, out_cap, out_len, &launches));
+	TRY(bgzf_compress_device(c, rec_text(c).as<uint8_t>(), raw, (uint8_t *)out, out_cap, out_len, &launches));
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 	c->last_ms = ms; c->last_launches = 4 + launches;
 	return EMAB_OK;
 }
 
-// Sorted mode: the raw records and their sort rows (slot 34) copied back; nothing is compressed per call.
+// Sorted mode: the raw records and their sort rows copied back; nothing is compressed per call.
 extern "C" int emab_bam_records(emab_ctx_t *c, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len, emab_bam_key_t *keys)
 {
 	CTX_ENTER(c);
@@ -574,12 +578,13 @@ extern "C" int emab_bam_records(emab_ctx_t *c, const emab_sam_job_t *job, char *
 	if (n == 0) return EMAB_OK;
 	if (raw > out_cap) { *out_len = raw; snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_records: %llu bytes do not fit the output buffer", raw); return EMAB_ERR_OVERFLOW; }
 	cudaStream_t st = c->stream;
-	TRY(c->b[34].ensure((size_t)n * sizeof(emab_bam_key_t)));
-	const unsigned long long *d_off = c->b[47].as<unsigned long long>() + (n + 1);
-	k_bam_key<<<(n + 127) / 128, 128, 0, st>>>(t, c->b[46].as<emab_sam_rec_t>(), n, d_off, c->b[34].as<emab_bam_key_t>());
+	DevBuf &keys_buf = c->ext_keys;   // the extension waves' keys: dead once the batch is aligned
+	TRY(keys_buf.ensure((size_t)n * sizeof(emab_bam_key_t)));
+	const unsigned long long *d_off = c->rec_off.as<unsigned long long>() + (n + 1);
+	k_bam_key<<<(n + 127) / 128, 128, 0, st>>>(t, c->sam_job.as<emab_sam_rec_t>(), n, d_off, keys_buf.as<emab_bam_key_t>());
 	CUDA_TRY(cudaEventRecord(c->ev1, st));
-	CUDA_TRY(cudaMemcpyAsync(out, c->b[33].p, (size_t)raw, cudaMemcpyDeviceToHost, st));
-	CUDA_TRY(cudaMemcpyAsync(keys, c->b[34].p, (size_t)n * sizeof(emab_bam_key_t), cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(out, rec_text(c).p, (size_t)raw, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(cudaMemcpyAsync(keys, keys_buf.p, (size_t)n * sizeof(emab_bam_key_t), cudaMemcpyDeviceToHost, st));
 	CUDA_TRY(ctx_wait(c));
 	CUDA_TRY(cudaGetLastError());
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);

@@ -137,7 +137,8 @@ static inline int seed_blocks_per_sm()
 }
 
 // Device buffers: d_intv [R][max_intv], d_n_intv [R], d_occ_cnt [R] or null, *d_err int, *d_touches u64 (zeroed by the caller).
-// Uses ctx slots 4 (lane scratch), 25 (pass-3 lists), 26 (per-pass counts + the two queue counters), 41 (2-bit packed reads).
+// Scratch of the ctx: seed_lanes (lane scratch), seed_p3 (pass-3 lists), seed_queue (per-pass counts + the two queue
+// counters), packed_reads (2-bit packed reads), seed_prof (EMAB_SEED_PROF's counts).
 static int launch_seed(emab_ctx *c, int R, int max_len, const uint8_t *d_seq, const int64_t *d_off, Intv *d_intv, int max_intv,
                        int32_t *d_n_intv, int32_t *d_occ_cnt, int *d_err, unsigned long long *d_touches, int *launches)
 {
@@ -157,24 +158,24 @@ static int launch_seed(emab_ctx *c, int R, int max_len, const uint8_t *d_seq, co
 	SeedBatch b;
 	b.n_reads = R; b.seq = d_seq; b.off = d_off; b.intv = d_intv; b.max_intv = max_intv;
 	b.scratch_len = max_len + 1;
-	if (int rc = c->b[4].ensure(lanes * 2 * b.scratch_len * sizeof(Intv))) return rc;
-	if (int rc = c->b[25].ensure((size_t)R * EMAB_P3_CAP * sizeof(Intv))) return rc;
-	if (int rc = c->b[26].ensure((size_t)R * 8 + 16)) return rc;
-	b.scratch = c->b[4].as<Intv>();
-	b.p3 = c->b[25].as<Intv>();
-	b.queue = c->b[26].as<unsigned long long>();
+	if (int rc = c->seed_lanes.ensure(lanes * 2 * b.scratch_len * sizeof(Intv))) return rc;
+	if (int rc = c->seed_p3.ensure((size_t)R * EMAB_P3_CAP * sizeof(Intv))) return rc;
+	if (int rc = c->seed_queue.ensure((size_t)R * 8 + 16)) return rc;
+	b.scratch = c->seed_lanes.as<Intv>();
+	b.p3 = c->seed_p3.as<Intv>();
+	b.queue = c->seed_queue.as<unsigned long long>();
 	b.n12 = (int32_t *)(b.queue + 2); b.n3 = b.n12 + R;
 	b.err = d_err; b.touches = d_touches;
 	CUDA_TRY(cudaMemsetAsync(b.queue, 0, 16, st));
 	if (seed_mode() == 5 && !seed_hot_first_form()) {
-		if (int rc = c->b[41].ensure((size_t)R * RQ_PACKED_BYTES + 64)) return rc;
-		RqBatch rb{b, c->b[41].as<uint32_t>()};
-		k_pack_reads<<<(R * 24 + 255) / 256, 256, 0, st>>>(d_seq, d_off, R, c->b[41].as<uint32_t>());
+		if (int rc = c->packed_reads.ensure((size_t)R * RQ_PACKED_BYTES + 64)) return rc;
+		RqBatch rb{b, c->packed_reads.as<uint32_t>()};
+		k_pack_reads<<<(R * 24 + 255) / 256, 256, 0, st>>>(d_seq, d_off, R, c->packed_reads.as<uint32_t>());
 		++*launches;
 		static const bool prof = getenv("EMAB_SEED_PROF") && atoi(getenv("EMAB_SEED_PROF")) != 0;
 		if (prof) {   // counts land behind the sector counter: a scratch array of its own
-			if (int rc = c->b[43].ensure(32 * 8)) return rc;
-			unsigned long long *cnt = c->b[43].as<unsigned long long>();
+			if (int rc = c->seed_prof.ensure(32 * 8)) return rc;
+			unsigned long long *cnt = c->seed_prof.as<unsigned long long>();
 			CUDA_TRY(cudaMemsetAsync(cnt, 0, 32 * 8, st));
 			rb.b.touches = cnt;
 			k_seed_rq_prof<<<grid, 32, RQ_SMEM_BYTES(8), st>>>(c->ix->d, rb);

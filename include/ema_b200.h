@@ -242,7 +242,11 @@ int emab_parse_bucket(emab_ctx_t *ctx, const char *text, uint64_t text_len, int 
 int emab_align_pairs_resident(emab_ctx_t *ctx, int n_pairs, const int64_t *off, emab_pairs_result_t *result, emab_stats_t *stats);
 int emab_sam_tables(emab_ctx_t *ctx, int n_chrom, const char *const *names, int n_rid, const int32_t *rid2chrom);
 int emab_sam_format(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len);
-/* emab_bam_format = the same records as BAM (SAM spec v1 §4.2), compressed on the device into BGZF members; only the members
+/* What the formatters read stays on the device until the next emab_align_pairs* or emab_parse_bucket call on the ctx: the
+ * batch's text and pair table, and the candidates and CIGAR pool of the last align call (rec_cand, mate_cand and alt_cand
+ * index them).  emab_em_batch, the formatters and the kernel-level calls leave them alone, so EM may run between the align
+ * call and the formatters.
+ * emab_bam_format = the same records as BAM (SAM spec v1 §4.2), compressed on the device into BGZF members; only the members
  *                    are copied to `out`.  Decoded the way `samtools view` prints them they are emab_sam_format's lines.
  *                    refID / next_refID: the first @SQ entry (contig of the index) with the .fai name the SAM line prints.
  *                    Fails with EMAB_ERR_ARG where BAM cannot hold the record: a read name longer than 254 bytes, a quality
