@@ -365,13 +365,14 @@ class Session:
 
     def __init__(self, ref_path: str, platform: str = "10x", device: int = 0, rg: str | None = None, bx_index: str | None = None,
                  apply_opt: bool = False, threads: int = 1, output: str = "sam", sort: bool = False, max_host_bytes: int = 0,
-                 spill: str | None = None):
+                 spill: str | None = None, qc: bool = False):
         """output="bam": header() and every align call return BGZF members of BAM instead of SAM text
         (a BAM file is header, the calls' bytes in order, then bgzf_eof()).
         sort=True (BAM only): align calls return b"" and hold their records (at most max_host_bytes of host memory, 0: no
         cap); finish() returns them as one coordinate-sorted body and its BAI (file: header, body, bgzf_eof()).
         spill=PREFIX: with a nonzero max_host_bytes, reaching it writes the held records to PREFIX.*.spill files instead of
-        failing, and finish() merges them (see set_spill)."""
+        failing, and finish() merges them (see set_spill).
+        qc=True: the align calls count alignment and linked-read molecule QC on the device (see set_qc, qc_report)."""
         self._h = C.c_void_p()
         _check(lib().emab_session_open(ref_path.encode(), platform.encode(), device, C.byref(self._h)))
         _check(lib().emab_session_config(self._h, rg.encode() if rg else None, bx_index.encode() if bx_index else None,
@@ -381,6 +382,8 @@ class Session:
             self.set_spill(spill)
         if sort:
             self.set_sort(True, max_host_bytes)
+        if qc:
+            self.set_qc(True)
 
     def set_sort(self, on: bool, max_host_bytes: int = 0, index: bool = True):
         """emab_session_sort: coordinate-sorted BAM for the calls that follow (index=False: no BAI, any contig length)"""
@@ -391,6 +394,22 @@ class Session:
         """emab_session_sort_spill: the prefix of the temporary files a sorted run spills to when it reaches max_host_bytes
         (None: no spilling, the cap fails the run).  A session setting that set_sort keeps."""
         _check(lib().emab_session_sort_spill(self._h, prefix.encode() if prefix else None))
+
+    def set_qc(self, on: bool):
+        """emab_session_qc: True starts a fresh QC accumulation over the align calls that follow, False stops it"""
+        _check(lib().emab_session_qc(self._h, int(on)))
+
+    def qc_report(self) -> bytes:
+        """emab_session_qc_report: the QC report (format version 1, include/ema_b200.h) of the calls since set_qc(True)"""
+        text, n = C.c_void_p(), C.c_uint64()
+        _check(lib().emab_session_qc_report(self._h, C.byref(text), C.byref(n)))
+        return self._take(text, n)
+
+    def qc_cost(self) -> dict:
+        """emab_session_qc_cost: device time of the QC kernels, QC calls and their copies since set_qc(True)"""
+        ms, calls, h2d, d2h = C.c_double(), C.c_int64(), C.c_int64(), C.c_int64()
+        _check(lib().emab_session_qc_cost(self._h, C.byref(ms), C.byref(calls), C.byref(h2d), C.byref(d2h)))
+        return dict(kernel_ms=ms.value, calls=calls.value, h2d_bytes=h2d.value, d2h_bytes=d2h.value)
 
     def finish(self) -> tuple[bytes, bytes]:
         """emab_session_finish: (sorted BGZF body without the EOF block, .bai bytes; b"" without an index)"""

@@ -128,6 +128,33 @@ int emab_session_sort_spill(emab_session_t *h, const char *prefix)
 	});
 }
 
+int emab_session_qc(emab_session_t *h, int on)
+{
+	return guarded([&]() -> int {
+		if (!h) return fail(EMAB_ERR_ARG, "null session");
+		emab::session_qc(h->s, on != 0);
+		return EMAB_OK;
+	});
+}
+
+int emab_session_qc_report(emab_session_t *h, char **text, uint64_t *len)
+{
+	return guarded([&]() -> int {
+		if (!h || !text || !len) return fail(EMAB_ERR_ARG, "null argument");
+		return give(emab::session_qc_report(h->s), text, len);
+	});
+}
+
+int emab_session_qc_cost(const emab_session_t *h, double *kernel_ms, int64_t *calls, int64_t *h2d_bytes, int64_t *d2h_bytes)
+{
+	return guarded([&]() -> int {
+		if (!h || !kernel_ms || !calls || !h2d_bytes || !d2h_bytes) return fail(EMAB_ERR_ARG, "null argument");
+		std::lock_guard<std::mutex> g(h->s->qc_mu);
+		*kernel_ms = h->s->qc_kernel_ms; *calls = h->s->qc_calls; *h2d_bytes = h->s->qc_h2d; *d2h_bytes = h->s->qc_d2h;
+		return EMAB_OK;
+	});
+}
+
 int emab_session_finish(emab_session_t *h, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len)
 {
 	return guarded([&]() -> int {

@@ -407,6 +407,26 @@ static void drop_runs(Session *s)
 	s->sort_err.clear();
 }
 
+void session_qc(Session *s, bool on)
+{
+	std::lock_guard<std::mutex> g(s->qc_mu);
+	s->qc = on;
+	if (!on) return;
+	s->qc_acc.reset(s->sq_names.size());
+	s->qc_kernel_ms = 0; s->qc_calls = s->qc_h2d = s->qc_d2h = 0;
+}
+
+std::string session_qc_report(Session *s)
+{
+	std::lock_guard<std::mutex> g(s->qc_mu);
+	const qc::Acc &a = s->qc_acc;
+	if (a.ref_mapped.empty()) s->qc_acc.reset(s->sq_names.size());   // never turned on: an empty report
+	std::vector<const char *> names;
+	for (const std::string &n : s->sq_names) names.push_back(n.c_str());
+	return qc::render(a.fs.data(), a.mapq.data(), a.isize.data(), (int)names.size(), names.data(), s->sq_len.data(), a.ref_mapped.data(),
+	                  a.ref_unmapped.data(), a.molecules.data(), a.molecules.size(), a.barcodes.size());
+}
+
 void session_sort_spill(Session *s, const char *prefix)
 {
 	std::lock_guard<std::mutex> g(s->run_mu);
@@ -1060,6 +1080,28 @@ static const uint8_t *nt4_table()
 	return tab.t;
 }
 
+// QC of a batch's records (emab_qc_records), after its formatter: folded into the session's sums
+static int qc_batch(Session *s, Worker &wk, const emab_sam_job_t &job, int mi_lo, int n_mi, const std::vector<Barcode> &bcs, emab_run_stats_t &st)
+{
+	const size_t n_ref = s->sq_names.size();
+	std::unique_ptr<emab_qc_counts_t> counts(new emab_qc_counts_t);
+	std::vector<uint64_t> rm(n_ref + 1), ru(n_ref + 1);
+	std::vector<emab_qc_molecule_t> mol((size_t)n_mi);
+	std::vector<uint8_t> has(bcs.size());
+	const int rc = emab_qc_records(wk.ctx, &job, mi_lo, n_mi, (int32_t)n_ref, counts.get(), rm.data(), ru.data(), mol.data(), has.data());
+	if (rc) { wk.err = emab_last_error(); return rc; }
+	const int64_t h2d = (int64_t)job.n_recs * (int64_t)sizeof(emab_sam_rec_t) + job.bc_off[job.n_bc] + (int64_t)(job.n_bc + 1) * 4,
+	              d2h = (int64_t)sizeof(emab_qc_counts_t) + (int64_t)(n_ref + 1) * 16 + job.n_bc + counts->n_molecules * (int64_t)sizeof(emab_qc_molecule_t);
+	st.h2d_bytes += h2d; st.d2h_bytes += d2h;
+	st.launches += emab_last_launches(wk.ctx);
+	std::lock_guard<std::mutex> g(s->qc_mu);
+	s->qc_acc.add(*counts, rm.data(), ru.data(), mol.data());
+	for (size_t b = 0; b < bcs.size(); ++b) if (has[b]) s->qc_acc.barcodes.insert(bcs[b].bc_str);
+	s->qc_kernel_ms += emab_last_kernel_ms(wk.ctx);
+	s->qc_calls += 1; s->qc_h2d += h2d; s->qc_d2h += d2h;
+	return EMAB_OK;
+}
+
 // The text a batch's pairs point into: one block (a bucket's contents) or two (-1 and -2 files).
 struct TextSrc { const char *base[2] = {nullptr, nullptr}; size_t len[2] = {0, 0}; };
 
@@ -1415,6 +1457,7 @@ static int process_pairs(Session *s, Worker &wk, Ticket &tk, const std::vector<P
 		st.d2h_bytes += (int64_t)total;
 		st.h2d_bytes += (int64_t)n_out * (int64_t)sizeof(emab_sam_rec_t) + (int64_t)bc_text.size();
 		st.format_kernel_ms = emab_last_kernel_ms(wk.ctx);
+		if (s->qc && (rc = qc_batch(s, wk, job, cloud_base[0], C, bcs, st))) { text_free(buf); return rc; }
 	}
 	buf[total] = 0;
 	*out_buf = buf; *out_len = (size_t)total;

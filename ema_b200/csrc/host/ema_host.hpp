@@ -11,6 +11,7 @@
 #include <string>
 #include <vector>
 #include "../../../include/ema_b200.h"
+#include "qc.hpp"
 
 namespace emab {
 
@@ -160,6 +161,12 @@ struct Session {  // the reference's process globals (src/main.c:23-34, src/alig
 	int sort_rc = 0;                      // a call of this run failed: finish refuses with this code and message
 	std::string sort_err;
 	uint64_t header_bytes = 0;            // size of the BGZF header emab_sam_header returned last (where the body starts)
+	// QC (emab_session_qc): what the align calls since it was turned on counted, and what counting cost, under qc_mu
+	bool qc = false;
+	std::mutex qc_mu;
+	qc::Acc qc_acc;
+	double qc_kernel_ms = 0;
+	int64_t qc_calls = 0, qc_h2d = 0, qc_d2h = 0;
 	std::string err;
 	std::string gamma_dump;               // test hook: path for full-precision posteriors of the chosen alignments
 	emab_run_stats_t last{};
@@ -217,6 +224,8 @@ void session_sort_spill(Session *s, const char *prefix);         // nullptr: no 
 // the held runs as one coordinate-sorted BGZF body to w, and its BAI (EMAB_SORT_COORD, bai != nullptr); releases the runs
 int session_finish(Session *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len);
 void sort_call_failed(Session *s, int rc);    // an align call failed in sorted mode: the run cannot be finished
+void session_qc(Session *s, bool on);                           // on: a fresh accumulation
+std::string session_qc_report(Session *s);
 int session_set_workers(Session *s, int n_workers);
 int session_add_device(Session *s, int device);  // before session_set_workers
 // find_clouds_and_align (src/align.c:214) over the *contents* of the input file(s); SAM text in a malloc'ed buffer

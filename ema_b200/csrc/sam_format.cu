@@ -14,11 +14,15 @@
 //   k_sam_write  warp / record     the same emitter with a writing writer: short fields by lane 0, strings lane-strided
 //   k_bam_len / (scan) / k_bam_write   the same for BAM records (SAM spec v1 §4.2), then BGZF members (bgzf.cu)
 //   k_bam_key    thread / record   sorted mode: the record's coordinate key, end, bin and length (bam_sort.cu orders them)
+//   k_qc_records thread / record   QC (emab_qc_records): flagstat, MAPQ, insert size, per-@SQ counts, molecule extents
+//   k_qc_molecules / (select)      the molecules with a record, compacted in MI order
+#include <algorithm>
 #include <cstdio>
 #include <cstring>
 #include <string>
 #include <vector>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
 #include "../../include/ema_b200.h"
 #include "runtime.cuh"
 #include "bgzf.cuh"
@@ -399,6 +403,106 @@ __global__ void k_bam_key(SamTables t, const emab_sam_rec_t *recs, int n, const 
 	keys[i] = k;
 }
 
+// ---- QC (emab_qc_records) ----
+
+enum {   // flagstat categories, in the order of emab_qc_counts_t
+	FS_TOTAL, FS_PRIMARY, FS_SECONDARY, FS_SUPP, FS_DUP, FS_PDUP, FS_MAPPED, FS_PMAPPED, FS_PAIRED, FS_READ1, FS_READ2, FS_PROPER,
+	FS_BOTH, FS_SINGLETON, FS_DIFFCHR, FS_DIFFCHR5
+};
+
+struct QcDev {
+	unsigned long long *fs, *mapq, *isize;   // [EMAB_QC_FLAGSTAT * 2], [EMAB_QC_MAPQ_BINS], [EMAB_QC_ISIZE_BINS]
+	unsigned long long *ref;                 // [(n_ref + 1) * 2]: (refID, or n_ref without one) * 2 + (FLAG & 4 ? 1 : 0)
+	uint8_t *bc_flag;                        // [n_bc]
+	// per MI slot (MI - mi_lo); refIDs are stored + 1, so that a memset sets the neutral values
+	uint32_t *pos_min, *ref_min;             // memset 0xff
+	uint32_t *end_max, *ref_max, *reads, *xf;   // memset 0
+	int mi_lo, n_mi, n_ref;
+};
+
+// Block-private flagstat, MAPQ and insert-size tables in shared memory, flushed bin by bin (non-zero bins only) with 64-bit
+// atomics; per-@SQ counts and molecule extents go to global memory.  Every count is an integer sum, min, max or or, so the
+// result does not depend on how records fall on blocks.
+__global__ void __launch_bounds__(256) k_qc_records(SamTables t, const emab_sam_rec_t *recs, int n, QcDev q)
+{
+	__shared__ unsigned s_fs[EMAB_QC_FLAGSTAT * 2], s_mapq[EMAB_QC_MAPQ_BINS], s_isize[EMAB_QC_ISIZE_BINS];
+	for (int i = threadIdx.x; i < EMAB_QC_ISIZE_BINS; i += blockDim.x) s_isize[i] = 0;
+	for (int i = threadIdx.x; i < EMAB_QC_MAPQ_BINS; i += blockDim.x) s_mapq[i] = 0;
+	if (threadIdx.x < EMAB_QC_FLAGSTAT * 2) s_fs[threadIdx.x] = 0;
+	__syncthreads();
+	for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+		const emab_sam_rec_t &d = recs[i];
+		const RecView v = make_view(t, d);
+		const unsigned f = d.flag, w = (f >> 9) & 1;   // 0x200: QC failed
+		const int ref = v.chrom >= 0 ? t.chrom2sq[v.chrom] : -1, mref = v.mate ? t.chrom2sq[v.mate_chrom] : -1;
+		const bool unmapped = f & 4, mate_unmapped = f & 8;
+		auto count = [&](int cat) { atomicAdd(&s_fs[cat * 2 + w], 1u); };
+		count(FS_TOTAL);
+		if (f & 0x100) count(FS_SECONDARY);
+		else if (f & 0x800) count(FS_SUPP);
+		else {
+			count(FS_PRIMARY);
+			if (f & 1) {
+				count(FS_PAIRED);
+				if ((f & 2) && !unmapped) count(FS_PROPER);
+				if (f & 0x40) count(FS_READ1);
+				if (f & 0x80) count(FS_READ2);
+				if (mate_unmapped && !unmapped) count(FS_SINGLETON);
+				if (!unmapped && !mate_unmapped) {
+					count(FS_BOTH);
+					if (mref != ref) { count(FS_DIFFCHR); if (d.mapq >= 5) count(FS_DIFFCHR5); }
+				}
+			}
+			if (!unmapped) { count(FS_PMAPPED); atomicAdd(&s_mapq[d.mapq], 1u); }
+			if (f & 0x400) count(FS_PDUP);
+		}
+		if (!unmapped) count(FS_MAPPED);
+		if (f & 0x400) count(FS_DUP);
+		if ((f & 0x40) && !unmapped && !mate_unmapped && mref == ref) {
+			const long long a = v.tlen < 0 ? -v.tlen : v.tlen;
+			atomicAdd(&s_isize[a < EMAB_QC_ISIZE_BINS - 1 ? a : EMAB_QC_ISIZE_BINS - 1], 1u);
+		}
+		{   // idxstats: records of a warp that share a counter add once
+			const int key = (ref >= 0 ? ref : q.n_ref) * 2 + (unmapped ? 1 : 0);
+			const unsigned grp = __match_any_sync(__activemask(), key);
+			if ((threadIdx.x & 31) == __ffs(grp) - 1) atomicAdd(&q.ref[key], (unsigned long long)__popc(grp));
+		}
+		q.bc_flag[d.bc] = 1;
+		if (v.rec) {   // the records that carry MI:i
+			const unsigned k = (unsigned)(d.mi - q.mi_lo);
+			if (k < (unsigned)q.n_mi) {   // the host checked every MI; the bound keeps a bad descriptor inside the arrays
+				const int rl = ref_len(*v.rec, t.cigars);
+				const uint32_t pos = (uint32_t)(v.pos - 1);
+				atomicMin(&q.pos_min[k], pos);
+				atomicMax(&q.end_max[k], pos + (uint32_t)(rl > 0 ? rl : 1));
+				atomicAdd(&q.reads[k], 1u);
+				if (d.xf) atomicOr(&q.xf[k], 1u);
+				atomicMin(&q.ref_min[k], (uint32_t)(ref + 1));
+				atomicMax(&q.ref_max[k], (uint32_t)(ref + 1));
+			}
+		}
+	}
+	__syncthreads();
+	for (int i = threadIdx.x; i < EMAB_QC_ISIZE_BINS; i += blockDim.x) if (s_isize[i]) atomicAdd(&q.isize[i], (unsigned long long)s_isize[i]);
+	for (int i = threadIdx.x; i < EMAB_QC_MAPQ_BINS; i += blockDim.x) if (s_mapq[i]) atomicAdd(&q.mapq[i], (unsigned long long)s_mapq[i]);
+	if (threadIdx.x < EMAB_QC_FLAGSTAT * 2 && s_fs[threadIdx.x]) atomicAdd(&q.fs[threadIdx.x], (unsigned long long)s_fs[threadIdx.x]);
+}
+
+// one entry per MI slot and whether it has a record; DeviceSelect::Flagged then keeps the ones that do, in MI order
+__global__ void k_qc_molecules(QcDev q, emab_qc_molecule_t *mol, uint8_t *keep)
+{
+	const int k = blockIdx.x * blockDim.x + threadIdx.x;
+	if (k >= q.n_mi) return;
+	emab_qc_molecule_t m;
+	m.reads = q.reads[k];
+	m.length = m.reads ? q.end_max[k] - q.pos_min[k] : 0;
+	m.xf = (uint8_t)q.xf[k];
+	m.multi_contig = m.reads && q.ref_min[k] != q.ref_max[k] ? 1 : 0;
+	m.pad = 0;
+	mol[k] = m;
+	keep[k] = m.reads ? 1 : 0;
+}
+
 }  // namespace
 
 // The formatters read the batch's text and pair table and the pipeline's candidates and CIGAR pool, all held by the ctx;
@@ -590,5 +694,97 @@ extern "C" int emab_bam_records(emab_ctx_t *c, const emab_sam_job_t *job, char *
 	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
 	c->last_ms = ms; c->last_launches = 4;
 	*out_len = raw;
+	return EMAB_OK;
+}
+
+// QC of a job's records.  Scratch of its own, bound here: the tables and per-@SQ counts in the extension waves' keys, the
+// per-MI accumulators and molecule slots in their order buffer (both dead once the batch is aligned), the tables' way back
+// in EM's result block.  The job goes through stage_job like the formatters'.
+extern "C" int emab_qc_records(emab_ctx_t *c, const emab_sam_job_t *job, int32_t mi_lo, int32_t n_mi, int32_t n_ref, emab_qc_counts_t *counts,
+                               uint64_t *ref_mapped, uint64_t *ref_unmapped, emab_qc_molecule_t *molecules, uint8_t *bc_has_rec)
+{
+	CTX_ENTER(c);
+	if (!c || !job || !counts || !ref_mapped || !ref_unmapped || n_mi < 0 || n_ref < 0 || (n_mi && !molecules) || (job->n_bc && !bc_has_rec))
+		return EMAB_ERR_ARG;
+	DevBuf &qc_tables = c->ext_keys, &qc_acc = c->ext_order;
+	HostBuf &qc_stage = c->em_gamma;
+	if (!c->sam_tables_ready || !c->text_ready) { snprintf(emab_errbuf, sizeof emab_errbuf, "emab_qc_records: tables or batch text not on the device"); return EMAB_ERR_ARG; }
+	if (!c->ix || (size_t)n_ref != c->ix->names.size()) {
+		snprintf(emab_errbuf, sizeof emab_errbuf, "emab_qc_records: n_ref %d is not the index's %zu contigs", n_ref, c->ix ? c->ix->names.size() : (size_t)0);
+		return EMAB_ERR_ARG;
+	}
+	const int n = job->n_recs;
+	for (int i = 0; i < n; ++i) {   // what the kernels index with: checked here, so a bad descriptor is an argument error, not a fault
+		const emab_sam_rec_t &d = job->recs[i];
+		if (d.bc >= (uint32_t)job->n_bc) {
+			snprintf(emab_errbuf, sizeof emab_errbuf, "emab_qc_records: record %d (pair %u, read %d): barcode %u of %d", i, d.pair, d.which + 1, d.bc, job->n_bc);
+			return EMAB_ERR_ARG;
+		}
+		if (d.rec_cand >= 0 && (d.mi < mi_lo || (int64_t)d.mi - mi_lo >= n_mi)) {
+			snprintf(emab_errbuf, sizeof emab_errbuf, "emab_qc_records: record %d (pair %u, read %d): MI %d outside the batch's cloud ids [%d, %lld)", i, d.pair,
+			         d.which + 1, d.mi, mi_lo, (long long)mi_lo + n_mi);
+			return EMAB_ERR_ARG;
+		}
+	}
+	cudaStream_t st = c->stream;
+	// tables block: counts | per-@SQ counts | barcode flags | molecules kept; copied back in one piece
+	const size_t o_ref = sizeof(emab_qc_counts_t), n_refc = (size_t)(n_ref + 1) * 2, o_bc = o_ref + n_refc * 8,
+	             o_nsel = (o_bc + (size_t)job->n_bc + 15) & ~(size_t)15, tables = o_nsel + 8;
+	TRY(qc_tables.ensure(tables));
+	// accumulators: pos_min, ref_min | end_max, ref_max, reads, xf | molecule slots | keep flags | molecules kept
+	const size_t nm = (size_t)n_mi, o_mol = (nm * 24 + 15) & ~(size_t)15, o_keep = o_mol + nm * sizeof(emab_qc_molecule_t),
+	             o_out = (o_keep + nm + 15) & ~(size_t)15, acc = o_out + nm * sizeof(emab_qc_molecule_t);
+	TRY(qc_acc.ensure(acc + 16));
+	SamTables t;
+	TRY(stage_job(c, job, t));
+	char *tb = qc_tables.as<char>();
+	QcDev q;
+	q.fs = (unsigned long long *)tb; q.mapq = q.fs + EMAB_QC_FLAGSTAT * 2; q.isize = q.mapq + EMAB_QC_MAPQ_BINS;
+	q.ref = (unsigned long long *)(tb + o_ref);
+	q.bc_flag = (uint8_t *)(tb + o_bc);
+	uint32_t *a = qc_acc.as<uint32_t>();
+	q.pos_min = a; q.ref_min = a + nm; q.end_max = a + 2 * nm; q.ref_max = a + 3 * nm; q.reads = a + 4 * nm; q.xf = a + 5 * nm;
+	q.mi_lo = mi_lo; q.n_mi = n_mi; q.n_ref = n_ref;
+	emab_qc_molecule_t *d_mol = (emab_qc_molecule_t *)(qc_acc.as<char>() + o_mol), *d_out = (emab_qc_molecule_t *)(qc_acc.as<char>() + o_out);
+	uint8_t *d_keep = (uint8_t *)(qc_acc.as<char>() + o_keep);
+	int *d_nsel = (int *)(tb + o_nsel);
+	CUDA_TRY(cudaEventRecord(c->ev0, st));
+	CUDA_TRY(cudaMemsetAsync(tb, 0, tables, st));
+	if (nm) {
+		CUDA_TRY(cudaMemsetAsync(a, 0xff, nm * 8, st));
+		CUDA_TRY(cudaMemsetAsync(a + 2 * nm, 0, nm * 16, st));
+	}
+	int launches = 0;
+	if (n) {
+		const int blocks = std::min((n + 255) / 256, c->n_sm);
+		k_qc_records<<<blocks, 256, 0, st>>>(t, c->sam_job.as<emab_sam_rec_t>(), n, q);
+		++launches;
+	}
+	if (nm) {
+		k_qc_molecules<<<(n_mi + 255) / 256, 256, 0, st>>>(q, d_mol, d_keep);
+		size_t tmp = 0;
+		cub::DeviceSelect::Flagged(nullptr, tmp, d_mol, d_keep, d_out, d_nsel, n_mi, st);
+		TRY(c->cub_tmp.ensure(tmp + 16));
+		cub::DeviceSelect::Flagged(c->cub_tmp.p, tmp, d_mol, d_keep, d_out, d_nsel, n_mi, st);
+		launches += 2;
+	}
+	CUDA_TRY(cudaEventRecord(c->ev1, st));
+	TRY(qc_stage.ensure(tables));
+	CUDA_TRY(cudaMemcpyAsync(qc_stage.p, tb, tables, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(ctx_wait(c));
+	CUDA_TRY(cudaGetLastError());
+	const char *h = qc_stage.as<char>();
+	memcpy(counts, h, sizeof *counts);
+	for (int r = 0; r <= n_ref; ++r) { memcpy(&ref_mapped[r], h + o_ref + (size_t)r * 16, 8); memcpy(&ref_unmapped[r], h + o_ref + (size_t)r * 16 + 8, 8); }
+	if (job->n_bc) memcpy(bc_has_rec, h + o_bc, (size_t)job->n_bc);
+	int nsel = 0;
+	if (nm) memcpy(&nsel, h + o_nsel, 4);
+	counts->n_molecules = nsel;
+	if (nsel) {
+		CUDA_TRY(cudaMemcpyAsync(molecules, d_out, (size_t)nsel * sizeof(emab_qc_molecule_t), cudaMemcpyDeviceToHost, st));
+		CUDA_TRY(ctx_wait(c));
+	}
+	float ms = 0; cudaEventElapsedTime(&ms, c->ev0, c->ev1);
+	c->last_ms = ms; c->last_launches = launches;
 	return EMAB_OK;
 }

@@ -273,6 +273,40 @@ typedef struct {
 	uint32_t pad;
 } emab_bam_key_t;
 int emab_bam_records(emab_ctx_t *ctx, const emab_sam_job_t *job, char *out, uint64_t out_cap, uint64_t *out_len, emab_bam_key_t *keys);
+/* emab_qc_records = alignment and linked-read molecule QC of a job's records, counted on the device from the same view of each
+ *                    record the formatters write, so the counts are those of the records a file of the job holds.  The call
+ *                    stages the job itself (it may follow a formatter call or stand alone) and holds nothing afterwards.
+ *                    Every record counts in the flagstat table (samtools >= 1.13 rules; refIDs as BAM holds them), primary
+ *                    mapped records in the MAPQ table, and the read1 record of a pair with both reads mapped to one refID in
+ *                    the insert-size table at |TLEN| (the last bin holds everything from EMAB_QC_ISIZE_BINS - 1 up).
+ *                    ref_mapped / ref_unmapped[n_ref + 1] count records by refID and FLAG & 4; index n_ref counts the
+ *                    records without a refID.  n_ref must be the index's contig count (its @SQ entries).
+ *                    Molecules are the MI:i values of the mapped records: the job's must lie in [mi_lo, mi_lo + n_mi), or
+ *                    the call fails with EMAB_ERR_ARG naming the record before anything is launched.  molecules[n_mi]
+ *                    receives, in MI order, one entry per MI that has a record (counts->n_molecules of them).
+ *                    bc_has_rec[n_bc] receives 1 for every job barcode with a record, 0 for the others. */
+#define EMAB_QC_FLAGSTAT 16
+#define EMAB_QC_MAPQ_BINS 256
+#define EMAB_QC_ISIZE_BINS 8192
+typedef struct {
+	/* [category][0: QC passed, 1: QC failed (FLAG & 0x200)]; categories in the order of the report's FS lines: total,
+	 * primary, secondary, supplementary, duplicates, primary duplicates, mapped, primary mapped, paired in sequencing, read1,
+	 * read2, properly paired, with itself and mate mapped, singletons, with mate mapped to a different chr, the same with
+	 * mapQ>=5 */
+	uint64_t flagstat[EMAB_QC_FLAGSTAT][2];
+	uint64_t mapq[EMAB_QC_MAPQ_BINS];
+	uint64_t isize[EMAB_QC_ISIZE_BINS];
+	int64_t n_molecules;
+} emab_qc_counts_t;
+typedef struct {
+	uint32_t length;          /* largest end (POS + the CIGAR's reference length, at least 1) - smallest POS, 0-based */
+	uint32_t reads;           /* records with this MI */
+	uint8_t xf;               /* a record carries XF:i:1 */
+	uint8_t multi_contig;     /* the records lie on more than one refID (then length means nothing) */
+	uint16_t pad;
+} emab_qc_molecule_t;
+int emab_qc_records(emab_ctx_t *ctx, const emab_sam_job_t *job, int32_t mi_lo, int32_t n_mi, int32_t n_ref, emab_qc_counts_t *counts,
+                    uint64_t *ref_mapped, uint64_t *ref_unmapped, emab_qc_molecule_t *molecules, uint8_t *bc_has_rec);
 /* emab_bam_sort = one coordinate-sorted BGZF body (and its BAI) from runs of raw records in input order.  A stable radix
  *                    sort of (key, record index) on the device gives the order; records are gathered on the host in that
  *                    order into page-locked slices of slice_chunks x 65 280 bytes (0 = 1 024 chunks), each compressed by the
@@ -413,6 +447,29 @@ int emab_session_sort(emab_session_t *s, int on, uint64_t max_host_bytes);
  * runs, and emab_session_sort keeps it. */
 int emab_session_sort_spill(emab_session_t *s, const char *prefix);
 int emab_session_finish(emab_session_t *s, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len);
+/* Alignment and linked-read molecule QC (`align -Q`).  emab_session_qc(s, 1) starts a fresh accumulation, 0 stops it; a
+ * session setting like the spill prefix.  While it is on, every align call counts its records on the device as it formats
+ * them (emab_qc_records), in every output and input mode; the output bytes do not change.
+ * emab_session_qc_report renders what the calls since emab_session_qc(s, 1) counted, as tab-separated text (released with
+ * emab_free).  Version 1: the line "# ema-b200 qc 1", then
+ *   FS <category> <QC passed> <QC failed>   the 16 flagstat categories of emab_qc_counts_t, in its order
+ *   LR <key> <value>                        barcodes (distinct BX strings without the -<index> / -1 suffix), molecules
+ *                                           (distinct MI values), molecules_xf, molecules_multi_contig; then over the
+ *                                           molecules on one refID only: molecule_reads, molecule_length_sum,
+ *                                           molecule_length_mean, molecule_length_n50 (the first length, in descending
+ *                                           order, at which twice the running sum reaches the total), reads_per_molecule_mean
+ *                                           and molecules_per_barcode_mean; means "%.2f", 0.00 over nothing; N50 0 without
+ *                                           molecules
+ *   MQ <mapq> <n>                           non-zero bins, ascending; likewise
+ *   IS <|TLEN|> <n>                         (the last bin, EMAB_QC_ISIZE_BINS - 1, holds everything from there up)
+ *   ML <length bin start> <n>               molecule lengths in 1 000-bp bins (molecules on one refID)
+ *   RM <reads> <n>                          reads per molecule (molecules on one refID)
+ *   IX <@SQ name> <length> <mapped> <unmapped>   every @SQ in header order, then "*  0  0  <records without a refID>"
+ * emab_session_qc_cost: device time of the QC kernels (CUDA events around them), QC calls, and the bytes they copied to and
+ * from the device, since emab_session_qc(s, 1). */
+int emab_session_qc(emab_session_t *s, int on);
+int emab_session_qc_report(emab_session_t *s, char **text, uint64_t *len);
+int emab_session_qc_cost(const emab_session_t *s, double *kernel_ms, int64_t *calls, int64_t *h2d_bytes, int64_t *d2h_bytes);
 int emab_sam_header(emab_session_t *s, int argc, const char *const *argv, char **text, uint64_t *len);
 int emab_align_bucket(emab_session_t *s, const char *data, uint64_t len, char **sam, uint64_t *sam_len);
 int emab_align_fastq(emab_session_t *s, const char *d1, uint64_t l1, const char *d2, uint64_t l2, char **sam, uint64_t *sam_len);
