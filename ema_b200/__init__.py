@@ -8,4 +8,4 @@ when the CUDA library or a GPU is missing.
 from ._lib import (EmabError, Index, Context, lib, extend_batch, global_batch, local_batch,  # noqa: F401
                    smem_batch, sa_batch, align_pairs, ALN_DTYPE, Session, PinnedText, RunStats, set_sw_mode, set_seed_mode,
                    extend_resident_load, extend_resident_run, int_peak, index_build, index_pack_fasta, parse_bucket,
-                   bgzf_eof, bgzf_compress)
+                   bgzf_eof, bgzf_compress, bgzf_inflate, bam_merge, bam_merge_header)

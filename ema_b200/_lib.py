@@ -312,6 +312,58 @@ def bgzf_compress(ctx: Context, data: bytes) -> bytes:
     return out.raw[:n.value]
 
 
+def bgzf_inflate(ctx: Context, data: bytes) -> bytes:
+    """emab_bgzf_inflate: the content of the whole BGZF members in `data`, inflated on the device (one warp per member)"""
+    n = C.c_uint64()
+    rc = lib().emab_bgzf_inflate(ctx._h, data, C.c_uint64(len(data)), None, C.c_uint64(0), C.byref(n))
+    if rc != -4:   # EMAB_ERR_OVERFLOW gives the size needed
+        _check(rc)
+        return b""
+    out = C.create_string_buffer(max(n.value, 1))
+    _check(lib().emab_bgzf_inflate(ctx._h, data, C.c_uint64(len(data)), out, C.c_uint64(n.value), C.byref(n)))
+    return out.raw[:n.value]
+
+
+_MERGE_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64)
+
+
+def bam_merge(paths, budget: int = 4 << 30, index: bool = True, device: int = 0, slice_chunks: int = 0, stats: dict | None = None):
+    """emab_bam_merge_files: the coordinate-sorted BAM files `paths` merged on the device into one sorted file ->
+    (file bytes without the EOF block, .bai bytes; b"" with index=False).  budget: host bytes of records read per window.
+    stats (optional) receives the wall times (ms) and the counts of the call."""
+    ctx = Context.__new__(Context)
+    ctx._h, ctx.index = C.c_void_p(), None
+    _check(lib().emab_ctx_create_on(device, C.byref(ctx._h)))
+    parts = []
+
+    def write(_u, p, n):
+        parts.append(C.string_at(p, n))
+        return 0
+    cb = _MERGE_CB(write)
+    arr = (C.c_char_p * len(paths))(*[os.fsencode(p) for p in paths])
+    bai, n = C.c_void_p(), C.c_uint64()
+    ms, counts = (C.c_double * 6)(), (C.c_uint64 * 4)()
+    _check(lib().emab_bam_merge_files(ctx._h, len(paths), arr, C.c_uint64(budget), slice_chunks, cb, None,
+                                      C.byref(bai) if index else None, C.byref(n), ms, counts))
+    idx = C.string_at(bai, n.value) if bai.value else b""
+    if bai.value:
+        lib().emab_free(bai)
+    if stats is not None:
+        stats.update(zip(("inflate_ms", "rows_ms", "order_ms", "gather_ms", "compress_ms", "index_ms"), list(ms)))
+        stats.update(zip(("read_bytes", "inflated_bytes", "records", "windows"), list(counts)))
+    return b"".join(parts), idx
+
+
+def bam_merge_header(paths) -> bytes:
+    """emab_bam_merge_header: the header text `bam_merge` writes for these inputs (host code, no device)"""
+    arr = (C.c_char_p * len(paths))(*[os.fsencode(p) for p in paths])
+    text, n = C.c_void_p(), C.c_uint64()
+    _check(lib().emab_bam_merge_header(len(paths), arr, C.byref(text), C.byref(n)))
+    out = C.string_at(text, n.value)
+    lib().emab_free(text)
+    return out
+
+
 class RunStats(C.Structure):
     _fields_ = [(n, C.c_double) for n in ("parse_ms", "encode_ms", "align_ms", "kernel_ms", "cloud_ms", "flatten_ms", "em_ms",
                                           "em_kernel_ms", "format_ms", "total_ms", "ms_seed", "ms_chain", "ms_align1", "ms_rescue",

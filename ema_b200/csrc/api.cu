@@ -234,10 +234,9 @@ extern "C" double emab_index_build_ms(const emab_index_t *ix) { return ix ? ix->
 // ---------------------------------------------------------------------------------------------
 // contexts
 // ---------------------------------------------------------------------------------------------
-extern "C" int emab_ctx_create(emab_index_t *ix, emab_ctx_t **out)
+static int ctx_create(emab_index_t *ix, int dev, emab_ctx_t **out)
 {
 	*out = nullptr;
-	int dev = ix ? ix->device : 0;
 	int ndev = 0;
 	CUDA_TRY(cudaGetDeviceCount(&ndev));
 	if (ndev <= 0) { snprintf(emab_errbuf, sizeof emab_errbuf, "no CUDA device"); return EMAB_ERR_CUDA; }
@@ -264,6 +263,14 @@ extern "C" int emab_ctx_create(emab_index_t *ix, emab_ctx_t **out)
 	if (const char *e = getenv("EMAB_PL_BPS")) { int v = atoi(e); if (v >= 1 && v <= 8) c->pl_bps = v; }  // persistent SW grids: blocks per SM
 	*out = c;
 	return EMAB_OK;
+}
+
+extern "C" int emab_ctx_create(emab_index_t *ix, emab_ctx_t **out) { return ctx_create(ix, ix ? ix->device : 0, out); }
+
+extern "C" int emab_ctx_create_on(int device, emab_ctx_t **out)
+{
+	if (!out || device < 0) return EMAB_ERR_ARG;
+	return ctx_create(nullptr, device, out);
 }
 
 extern "C" int emab_ctx_make_current(emab_ctx_t *c)

@@ -32,6 +32,7 @@
 #include <cstdio>
 #include <cstring>
 #include <memory>
+#include <string>
 #include <vector>
 #include <cuda/std/tuple>
 #include <cub/device/device_radix_sort.cuh>
@@ -43,6 +44,8 @@
 #include "runtime.cuh"
 #include "bgzf.cuh"
 #include "bai.cuh"
+#include "inflate.cuh"
+#include "bam_row.cuh"
 
 #define TRY(x) do { int rc__ = (x); if (rc__) return rc__; } while (0)
 
@@ -694,46 +697,152 @@ extern "C" int emab_bam_spill(emab_ctx_t *c, int n_runs, const emab_bam_run_t *r
 }
 
 namespace {
-// one sorted run of the merge: a spill file, or the runs still in memory
+// ---- a BAM file as a sorted run of the merge (emab_bam_merge_files)
+// k_bam_rows: the sort row of every record of an inflated block (bam_row.cuh: the row and the refusals that keep the index
+// kernels' refID and window indices in range), its input position, and the order check against the previous record (the
+// block's first record against the last key of the block before).  *bad receives the smallest (record << 8 | reason) of
+// the block's refusals.
+__global__ void k_bam_rows(const uint8_t *__restrict__ d, const u64 *__restrict__ off, uint32_t n, int n_ref, const int32_t *__restrict__ ref_len,
+                           u64 prev_key, u64 seq0, SpillRow *__restrict__ rows, u64 *bad)
+{
+	const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= n) return;
+	SpillRow &o = rows[i];
+	int why = bamrow::row_of(d + off[i], n_ref, ref_len, &o.k);
+	if (!why && o.k.key < (i ? bamrow::key_of(d + off[i - 1]) : prev_key)) why = bamrow::ROW_ORDER;
+	if (why) { atomicMin(bad, (u64)i << 8 | (u64)why); return; }
+	o.seq = seq0 + i;
+}
+
+// one sorted run of the merge: a spill file, the runs still in memory, or a BAM file
 struct Source {
 	const char *path = nullptr;
 	u64 n = 0, bytes = 0, at = 0, boff = 0;   // rows, record bytes; the next row and its record's offset
-	std::vector<SpillRow> rows;               // in memory: the rows and their records
+	std::vector<SpillRow> rows;               // in memory: the rows and their records; BAM: the rows read and not yet taken
 	std::vector<const char *> ptr;
+	// a BAM file: the next member's file offset, the content to drop before the first record (the header's end), the
+	// bytes of the records read and not taken (rec_off[k] is rows[k]'s), a record cut by the end of the last block,
+	// the next record's ordinal, the last key read
+	bool bam = false, eof = false;
+	int input = 0;
+	u64 foff = 0, fsize = 0, drop = 0, ord = 0, last_key = 0;
+	std::vector<char> rec, part;
+	std::vector<u64> rec_off;
+	bool left() const { return bam ? !eof || at < rows.size() : at < n; }
 };
-}  // namespace
 
-extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *paths, int n_runs, const emab_bam_run_t *runs,
-                              const uint64_t *seq0, int n_ref, const int32_t *ref_len, uint64_t body_offset, int slice_chunks,
-                              uint64_t budget, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len, double ms[4])
+struct MergeCost { double inflate = 0, rows = 0; u64 read = 0, inflated = 0, records = 0, windows = 0; };
+
+// reads whole members from a BAM source until their content reaches `want` bytes (or the file ends), inflates them on the
+// device after the record left over from the last block, walks the block_size chain on the host over the bytes copied
+// back (Writer gathers them from the host anyway) and builds the rows on the device
+int bam_read_block(emab_ctx *c, Source &s, u64 want, int n_ref, const int32_t *d_ref_len, MergeCost &cost)
 {
-	CTX_ENTER(c);
-	if (!c || n_files < 0 || (n_files && !paths) || n_runs < 0 || (n_runs && (!runs || !seq0)) || n_ref < 0 || (n_ref && !ref_len) || !w ||
-	    (bai && !bai_len))
-		return EMAB_ERR_ARG;
-	if (bai) { *bai = nullptr; *bai_len = 0; }
-	if (ms) for (int k = 0; k < 4; ++k) ms[k] = 0;
 	cudaStream_t st = c->stream;
-	std::vector<Source> src((size_t)n_files + 1);
-	for (int f = 0; f < n_files; ++f) {
-		Source &s = src[f];
-		s.path = paths[f];
-		const int fd = ::open(s.path, O_RDONLY | O_CLOEXEC);
-		SpillHead hd;
-		if (fd < 0) return io_fail("open", s.path);
-		const bool ok = pread_all(fd, &hd, sizeof hd, 0);
-		::close(fd);
-		if (!ok) return io_fail("read", s.path);
-		if (memcmp(hd.magic, SPILL_MAGIC, 8) != 0) { snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s is not a spill file", s.path); return EMAB_ERR_IO; }
-		s.n = hd.n; s.bytes = hd.bytes;
-	}
 	double t0 = now_ms();
-	Source &mem = src.back();
-	TRY(sorted_rows(c, n_runs, runs, seq0, mem.rows, mem.ptr));
-	mem.n = mem.rows.size();
-	Writer W(c, n_ref, ref_len, body_offset, slice_chunks, w, uw, bai != nullptr);
-	W.t[0] += now_ms() - t0;
-	TRY(W.start());
+	const u64 room = std::min<u64>(s.fsize - s.foff, want + 2 * (u64)bgzf::MEMBER_MAX);
+	std::vector<uint8_t> z((size_t)room);
+	const int fd = ::open(s.path, O_RDONLY | O_CLOEXEC);
+	if (fd < 0) return io_fail("open", s.path);
+	const bool ok = pread_all(fd, z.data(), z.size(), s.foff);
+	::close(fd);
+	if (!ok) return io_fail("read", s.path);
+	u64 used = 0, content = 0;
+	while (used < room && content < want) {
+		int size = 0, at = 0;
+		if (bgzf::member_frame(z.data() + used, room - used, &size, &at)) break;   // bgzf_inflate_device names a bad one
+		content += bgzf::member_isize(z.data() + used, size);
+		used += (u64)size;
+	}
+	if (used == 0) used = room;   // the first member is bad: let the inflater report it
+	uint64_t n_out = 0;
+	const u64 skip = s.part.size();
+	TRY(bgzf_inflate_device(c, z.data(), used, s.part.data(), skip, s.path, s.foff, &n_out));
+	s.foff += used;
+	s.eof = s.foff >= s.fsize;
+	cost.read += used; cost.inflated += n_out;
+	const u64 total = skip + n_out;
+	std::vector<char> blk((size_t)total);
+	if (total) CUDA_TRY(cudaMemcpyAsync(blk.data(), c->infl_out.p, (size_t)total, cudaMemcpyDeviceToHost, st));
+	CUDA_TRY(ctx_wait(c));
+	cost.inflate += now_ms() - t0;
+	t0 = now_ms();
+	// the block_size chain
+	u64 o = std::min(s.drop, total);
+	s.drop -= o;
+	std::vector<u64> off;
+	while (o + 4 <= total) {
+		int32_t bs;
+		memcpy(&bs, blk.data() + o, 4);
+		if (bs < 32) {
+			snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s: record %llu: block_size %d is below 32", s.path, s.ord + off.size(), bs);
+			return EMAB_ERR_IO;
+		}
+		if (o + 4 + (u64)bs > total) break;
+		off.push_back(o);
+		o += 4 + (u64)bs;
+	}
+	if (s.eof && (o < total || s.drop)) {
+		snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s: the file ends inside record %llu", s.path, s.ord + off.size());
+		return EMAB_ERR_IO;
+	}
+	const uint32_t n = (uint32_t)off.size();
+	if (n) {
+		off.push_back(o);
+		// the pipeline's mate-rescue buffers, dead after it: the record offsets | the rows, and the refusal
+		DevBuf &off_buf = c->rescue_tasks, &row_buf = c->rescue_spans;
+		TRY(off_buf.ensure((size_t)(n + 1) * 8 + 16));
+		TRY(row_buf.ensure((size_t)n * sizeof(SpillRow) + 16));
+		u64 *d_off = off_buf.as<u64>(), *d_bad = d_off + n + 1;
+		SpillRow *d_rows = row_buf.as<SpillRow>();
+		const u64 none = ~0ull;
+		CUDA_TRY(cudaMemcpyAsync(d_off, off.data(), (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, st));
+		CUDA_TRY(cudaMemcpyAsync(d_bad, &none, 8, cudaMemcpyHostToDevice, st));
+		k_bam_rows<<<grid(n, 256), 256, 0, st>>>(c->infl_out.as<uint8_t>(), d_off, n, n_ref, d_ref_len, s.last_key, (u64)s.input << 40 | s.ord, d_rows, d_bad);
+		CUDA_TRY(cudaGetLastError());
+		u64 bad = 0;
+		CUDA_TRY(cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, st));
+		const size_t r0 = s.rows.size();
+		s.rows.resize(r0 + n);
+		CUDA_TRY(cudaMemcpyAsync(s.rows.data() + r0, d_rows, (size_t)n * sizeof(SpillRow), cudaMemcpyDeviceToHost, st));
+		CUDA_TRY(ctx_wait(c));
+		if (bad != ~0ull) {
+			snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s: record %llu: %s", s.path, s.ord + (bad >> 8), bamrow::reason((int)(bad & 255)));
+			return EMAB_ERR_IO;
+		}
+		const u64 b0 = s.rec.size();
+		for (uint32_t k = 0; k < n; ++k) s.rec_off.push_back(b0 + off[k] - off[0]);
+		s.rec.insert(s.rec.end(), blk.data() + off[0], blk.data() + o);
+		s.last_key = s.rows.back().k.key;
+		s.ord += n;
+		cost.records += n;
+	}
+	s.part.assign(blk.data() + o, blk.data() + total);
+	cost.rows += now_ms() - t0;
+	return EMAB_OK;
+}
+
+// tops a BAM source up to `want` bytes of records not yet taken, dropping the taken ones first
+int bam_fill(emab_ctx *c, Source &s, u64 want, int n_ref, const int32_t *d_ref_len, MergeCost &cost)
+{
+	if (s.at) {
+		const u64 cut = s.at < s.rows.size() ? s.rec_off[s.at] : s.rec.size();
+		s.rows.erase(s.rows.begin(), s.rows.begin() + (ptrdiff_t)s.at);
+		s.rec_off.erase(s.rec_off.begin(), s.rec_off.begin() + (ptrdiff_t)s.at);
+		for (u64 &x : s.rec_off) x -= cut;
+		s.rec.erase(s.rec.begin(), s.rec.begin() + (ptrdiff_t)cut);
+		s.at = 0;
+	}
+	while (!s.eof && s.rec.size() + s.rows.size() * sizeof(SpillRow) < want)
+		TRY(bam_read_block(c, s, want - s.rec.size() - s.rows.size() * sizeof(SpillRow), n_ref, d_ref_len, cost));
+	return EMAB_OK;
+}
+
+// The windows of a merge (emab_bam_merge, emab_bam_merge_files): a block of rows and records from every source, the
+// device's bound, selection, order and offsets, then the Writer.
+int merge_windows(emab_ctx *c, std::vector<Source> &src, Writer &W, u64 budget, int n_ref, const int32_t *d_ref_len, MergeCost &cost)
+{
+	cudaStream_t st = c->stream;
 	const u64 blk = std::max<u64>(1, budget / (2 * (src.size() + 1)));   // bytes of rows and records read from each run per window
 	std::vector<SpillRow> rows;
 	std::vector<char> bytes;
@@ -741,12 +850,27 @@ extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *pat
 	std::vector<uint32_t> perm;
 	std::vector<RunSeg> seg;
 	std::vector<size_t> seg_src;
+	double t0;
+	bool ended = false;
 	for (;;) {
 		// ---- the host reads a block of rows and their records from each run
 		double tg = now_ms();
 		rows.clear(); bytes.clear(); in_off.assign(1, 0); seg.clear(); seg_src.clear();
 		for (size_t r = 0; r < src.size(); ++r) {
 			Source &s = src[r];
+			if (s.bam) {
+				const double tb = now_ms();
+				TRY(bam_fill(c, s, blk, n_ref, d_ref_len, cost));
+				tg += now_ms() - tb;   // counted as inflate and rows, not as the gather
+				if (s.rows.empty()) continue;
+				const size_t r0 = rows.size();
+				rows.insert(rows.end(), s.rows.begin(), s.rows.end());
+				for (size_t i = 0; i < s.rows.size(); ++i) in_off.push_back(in_off.back() + s.rows[i].k.len);
+				bytes.insert(bytes.end(), s.rec.begin(), s.rec.end());
+				seg.push_back(RunSeg{(uint32_t)r0, (uint32_t)s.rows.size(), !s.eof, 0});
+				seg_src.push_back(r);
+				continue;
+			}
 			if (s.at >= s.n) continue;
 			const u64 lim = std::min<u64>(s.n - s.at, blk / sizeof(SpillRow) + 1);
 			const size_t r0 = rows.size();
@@ -779,6 +903,7 @@ extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *pat
 		if (rows.size() >= 0x7fffffffull) { snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_merge: window too large"); return EMAB_ERR_ARG; }
 		const uint32_t n = (uint32_t)rows.size(), ns = (uint32_t)seg.size();
 		W.t[1] += now_ms() - tg;
+		++cost.windows;
 		// ---- the device: the bound, the rows at or below it, their order by (key, seq) and their body offsets
 		t0 = now_ms();
 		// the pipeline's wave buffers, dead after it: rows | runs; bound | flags | taken | count | keys, sorted keys | perm;
@@ -833,15 +958,301 @@ extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *pat
 			Source &s = src[seg_src[i]];
 			for (const SpillRow *q = b; q < t; ++q) s.boff += q->k.len;
 			s.at += (u64)(t - b);
-			if (s.at < s.n) last = false;
 		}
-		for (const Source &s : src) if (s.at < s.n) last = false;
+		for (const Source &s : src) if (s.left()) last = false;
 		W.t[0] += now_ms() - t0;
 		TRY(W.window(T, T - unplaced, h_uoff.data(), [&](int64_t j) { return (const char *)bytes.data() + in_off[perm[(size_t)j]]; }, last));
+		ended = last;
 	}
-	if (W.U == 0) { const u64 z = 0; TRY(W.window(0, 0, &z, [&](int64_t) { return (const char *)nullptr; }, true)); }
+	// no window was the last one: no records at all, or a BAM input held only empty members after its last record
+	if (!ended) {
+		const u64 z = 0;
+		TRY(W.reserve(0));   // the rows still waiting for their member back at the front
+		TRY(W.window(0, 0, &z, [&](int64_t) { return (const char *)nullptr; }, true));
+	}
+	return EMAB_OK;
+}
+}  // namespace
+
+extern "C" int emab_bam_merge(emab_ctx_t *c, int n_files, const char *const *paths, int n_runs, const emab_bam_run_t *runs,
+                              const uint64_t *seq0, int n_ref, const int32_t *ref_len, uint64_t body_offset, int slice_chunks,
+                              uint64_t budget, emab_write_cb w, void *uw, char **bai, uint64_t *bai_len, double ms[4])
+{
+	CTX_ENTER(c);
+	if (!c || n_files < 0 || (n_files && !paths) || n_runs < 0 || (n_runs && (!runs || !seq0)) || n_ref < 0 || (n_ref && !ref_len) || !w ||
+	    (bai && !bai_len))
+		return EMAB_ERR_ARG;
+	if (bai) { *bai = nullptr; *bai_len = 0; }
+	if (ms) for (int k = 0; k < 4; ++k) ms[k] = 0;
+	std::vector<Source> src((size_t)n_files + 1);
+	for (int f = 0; f < n_files; ++f) {
+		Source &s = src[f];
+		s.path = paths[f];
+		const int fd = ::open(s.path, O_RDONLY | O_CLOEXEC);
+		SpillHead hd;
+		if (fd < 0) return io_fail("open", s.path);
+		const bool ok = pread_all(fd, &hd, sizeof hd, 0);
+		::close(fd);
+		if (!ok) return io_fail("read", s.path);
+		if (memcmp(hd.magic, SPILL_MAGIC, 8) != 0) { snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s is not a spill file", s.path); return EMAB_ERR_IO; }
+		s.n = hd.n; s.bytes = hd.bytes;
+	}
+	const double t0 = now_ms();
+	Source &mem = src.back();
+	TRY(sorted_rows(c, n_runs, runs, seq0, mem.rows, mem.ptr));
+	mem.n = mem.rows.size();
+	Writer W(c, n_ref, ref_len, body_offset, slice_chunks, w, uw, bai != nullptr);
+	W.t[0] += now_ms() - t0;
+	TRY(W.start());
+	MergeCost cost;
+	TRY(merge_windows(c, src, W, budget, n_ref, nullptr, cost));
 	TRY(W.finish(bai, bai_len));
 	if (ms) for (int k = 0; k < 4; ++k) ms[k] = W.t[k];
 	c->last_ms = W.t[0] + W.t[2] + W.t[3];
+	return EMAB_OK;
+}
+
+// ---- merging BAM files: their headers (host), then their records as sorted runs
+namespace {
+struct BamHead {
+	std::string text;
+	std::vector<std::string> names;
+	std::vector<int32_t> lens;
+	u64 body_foff = 0, body_drop = 0, fsize = 0;   // the member holding the header's end, the header's bytes in it; file size
+};
+
+int head_fail(const char *path, const char *why)
+{
+	snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s: %s", path, why);
+	return EMAB_ERR_IO;
+}
+
+// the header's size once raw holds all of it; else 0 with *need the bytes to read next; -1 when it is not a BAM header
+int64_t parse_head(const std::string &raw, BamHead &h, u64 *need)
+{
+	auto i32 = [&](u64 o) { int32_t v; memcpy(&v, raw.data() + o, 4); return v; };
+	*need = 8;
+	if (raw.size() < 8) return 0;
+	if (memcmp(raw.data(), "BAM\1", 4) != 0 || i32(4) < 0) return -1;
+	u64 o = 8 + (u64)i32(4);
+	*need = o + 4;
+	if (raw.size() < *need) return 0;
+	const int32_t n_ref = i32(o);
+	if (n_ref < 0) return -1;
+	o += 4;
+	h.names.clear(); h.lens.clear();
+	for (int32_t r = 0; r < n_ref; ++r) {
+		*need = o + 4;
+		if (raw.size() < *need) return 0;
+		const int32_t ln = i32(o);
+		if (ln < 1) return -1;
+		*need = o + 8 + (u64)ln;
+		if (raw.size() < *need) return 0;
+		h.names.emplace_back(raw.data() + o + 4, strnlen(raw.data() + o + 4, (size_t)ln));
+		h.lens.push_back(i32(o + 4 + (u64)ln));
+		if (h.lens.back() < 0) return -1;
+		o += 8 + (u64)ln;
+	}
+	h.text.assign(raw.data() + 8, (size_t)i32(4));
+	return (int64_t)o;
+}
+
+// the header of one input, inflated on the host (inflate.cuh) member by member until it is complete
+int read_head(const char *path, BamHead &h)
+{
+	const int fd = ::open(path, O_RDONLY | O_CLOEXEC);
+	if (fd < 0) return io_fail("open", path);
+	struct Close { int fd; ~Close() { ::close(fd); } } closer{fd};
+	const off_t end = ::lseek(fd, 0, SEEK_END);
+	if (end < 0) return io_fail("read", path);
+	h.fsize = (u64)end;
+	std::unique_ptr<bgzf::InflateWork> work(new bgzf::InflateWork);
+	std::vector<uint8_t> z(bgzf::MEMBER_MAX), out(bgzf::MEMBER_MAX);
+	std::string raw;
+	u64 foff = 0, need = 8;
+	for (;;) {
+		if (foff >= h.fsize) return head_fail(path, raw.empty() ? "not a BGZF file (it is empty)" : "the file ends inside the BAM header");
+		const size_t k = (size_t)std::min<u64>(z.size(), h.fsize - foff);
+		if (!pread_all(fd, z.data(), k, foff)) return io_fail("read", path);
+		int size = 0, n = 0;
+		const int rc = bgzf::inflate_member_host(z.data(), k, out.data(), &size, &n, *work);
+		if (rc) {
+			snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s: %sBGZF member at byte offset %llu: %s", path, foff || rc != bgzf::INF_HEADER ? "" : "not a BGZF file: ",
+			         foff, bgzf::inflate_reason(rc));
+			return EMAB_ERR_IO;
+		}
+		const u64 c0 = raw.size();
+		raw.append((const char *)out.data(), (size_t)n);
+		if (raw.size() >= need) {
+			const int64_t H = parse_head(raw, h, &need);
+			if (H < 0) return head_fail(path, "not a BAM file (no BAM\\1 header)");
+			if (H > 0) { h.body_foff = foff; h.body_drop = (u64)H - c0; return EMAB_OK; }
+		}
+		foff += (u64)size;
+	}
+}
+
+std::vector<std::string> split_lines(const std::string &t)
+{
+	std::vector<std::string> out;
+	size_t a = 0;
+	while (a < t.size()) {
+		size_t e = t.find('\n', a);
+		if (e == std::string::npos) e = t.size();
+		out.push_back(t.substr(a, e - a));
+		a = e + 1;
+	}
+	return out;
+}
+
+std::string field(const std::string &line, const char *tag)   // the value of TAG:value in a header line, or "" without it
+{
+	const std::string k = std::string("\t") + tag + ":";
+	const size_t p = line.find(k);
+	if (p == std::string::npos) return "";
+	const size_t a = p + k.size(), e = line.find('\t', a);
+	return line.substr(a, e == std::string::npos ? std::string::npos : e - a);
+}
+
+// The merged header text (include/ema_b200.h states the rules), after checking that every input has the first one's
+// reference list
+int merge_heads(int n, const char *const *paths, const std::vector<BamHead> &h, std::string *out)
+{
+	for (int f = 1; f < n; ++f) {
+		const size_t nr = std::min(h[0].names.size(), h[f].names.size());
+		size_t r = 0;
+		while (r < nr && h[f].names[r] == h[0].names[r] && h[f].lens[r] == h[0].lens[r]) ++r;
+		if (r == nr && h[f].names.size() == h[0].names.size()) continue;
+		if (r == nr)
+			snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s has %zu references and %s has %zu: merging needs identical @SQ lists",
+			         paths[f], h[f].names.size(), paths[0], h[0].names.size());
+		else
+			snprintf(emab_errbuf, sizeof emab_errbuf, "error: %s: reference %zu (%s, %d bp) differs from %s's (%s, %d bp): merging needs identical @SQ lists",
+			         paths[f], r, h[f].names[r].c_str(), h[f].lens[r], paths[0], h[0].names[r].c_str(), h[0].lens[r]);
+		return EMAB_ERR_ARG;
+	}
+	std::string t = h[0].text;
+	while (!t.empty() && t.back() == '\0') t.pop_back();   // l_text may count NUL padding
+	std::vector<std::string> lines = split_lines(t);
+	bool changed = false;
+	if (lines.empty() || lines[0].compare(0, 3, "@HD") != 0) {
+		lines.insert(lines.begin(), "@HD\tVN:1.6\tSO:coordinate");
+		changed = true;
+	} else if (field(lines[0], "SO") != "coordinate") {
+		const size_t p = lines[0].find("\tSO:");
+		if (p == std::string::npos) lines[0] += "\tSO:coordinate";
+		else {
+			const size_t e = lines[0].find('\t', p + 1);
+			lines[0] = lines[0].substr(0, p) + "\tSO:coordinate" + (e == std::string::npos ? "" : lines[0].substr(e));
+		}
+		changed = true;
+	}
+	std::vector<std::pair<std::string, std::pair<std::string, int>>> rg;   // ID -> (line, input)
+	std::vector<std::string> pg;
+	for (const std::string &l : lines) {
+		if (l.compare(0, 3, "@RG") == 0) rg.push_back({field(l, "ID"), {l, 0}});
+		if (l.compare(0, 3, "@PG") == 0) pg.push_back(field(l, "ID"));
+	}
+	for (int f = 1; f < n; ++f)
+		for (const std::string &l : split_lines(h[f].text.substr(0, strnlen(h[f].text.data(), h[f].text.size())))) {
+			if (l.compare(0, 3, "@RG") == 0) {
+				const std::string id = field(l, "ID");
+				auto it = std::find_if(rg.begin(), rg.end(), [&](const auto &x) { return x.first == id; });
+				if (it == rg.end()) { rg.push_back({id, {l, f}}); lines.push_back(l); changed = true; }
+				else if (it->second.first != l) {
+					snprintf(emab_errbuf, sizeof emab_errbuf, "error: @RG ID:%s differs between %s and %s", id.c_str(), paths[it->second.second], paths[f]);
+					return EMAB_ERR_ARG;
+				}
+			} else if (l.compare(0, 3, "@PG") == 0) {
+				const std::string id = field(l, "ID");
+				if (std::find(pg.begin(), pg.end(), id) == pg.end()) { pg.push_back(id); lines.push_back(l); changed = true; }
+			} else if (l.compare(0, 3, "@CO") == 0) {
+				lines.push_back(l);
+				changed = true;
+			}
+		}
+	if (!changed) { *out = h[0].text; return EMAB_OK; }
+	out->clear();
+	for (const std::string &l : lines) { out->append(l); out->push_back('\n'); }
+	return EMAB_OK;
+}
+
+int merged_head(int n, const char *const *paths, std::vector<BamHead> &h, std::string *text)
+{
+	if (n <= 0 || !paths) { snprintf(emab_errbuf, sizeof emab_errbuf, "error: no input files to merge"); return EMAB_ERR_ARG; }
+	h.resize((size_t)n);
+	for (int f = 0; f < n; ++f) TRY(read_head(paths[f], h[f]));
+	return merge_heads(n, paths, h, text);
+}
+}  // namespace
+
+extern "C" int emab_bam_merge_header(int n_inputs, const char *const *paths, char **text, uint64_t *len)
+{
+	if (!text || !len) return EMAB_ERR_ARG;
+	*text = nullptr; *len = 0;
+	std::vector<BamHead> h;
+	std::string t;
+	TRY(merged_head(n_inputs, paths, h, &t));
+	char *o = emab::text_alloc(t.size() + 1);
+	if (!o) { snprintf(emab_errbuf, sizeof emab_errbuf, "out of host memory"); return EMAB_ERR_NOMEM; }
+	memcpy(o, t.data(), t.size());
+	o[t.size()] = 0;
+	*text = o; *len = t.size();
+	return EMAB_OK;
+}
+
+extern "C" int emab_bam_merge_files(emab_ctx_t *c, int n_inputs, const char *const *paths, uint64_t budget, int slice_chunks, emab_write_cb w,
+                                    void *uw, char **bai, uint64_t *bai_len, double ms[6], uint64_t counts[4])
+{
+	CTX_ENTER(c);
+	if (!c || !w || (bai && !bai_len)) return EMAB_ERR_ARG;
+	if (bai) { *bai = nullptr; *bai_len = 0; }
+	if (ms) for (int k = 0; k < 6; ++k) ms[k] = 0;
+	if (counts) for (int k = 0; k < 4; ++k) counts[k] = 0;
+	std::vector<BamHead> h;
+	std::string text;
+	TRY(merged_head(n_inputs, paths, h, &text));
+	const int n_ref = (int)h[0].names.size();
+	if (bai)
+		for (int r = 0; r < n_ref; ++r)
+			if (h[0].lens[r] > bai::MAX_LEN) {
+				snprintf(emab_errbuf, sizeof emab_errbuf, "error: contig %s is %d bp long; a BAI index holds contigs of up to 536870911 bp (2^29 - 1), so no index can be written",
+				         h[0].names[r].c_str(), h[0].lens[r]);
+				return EMAB_ERR_ARG;
+			}
+	// the header: as emab_sam_header writes it in BAM mode, with the first input's reference list
+	std::string raw("BAM\1", 4);
+	auto u32 = [&](uint32_t v) { for (int k = 0; k < 4; ++k) raw.push_back((char)(v >> 8 * k)); };
+	u32((uint32_t)text.size());
+	raw += text;
+	u32((uint32_t)n_ref);
+	for (int r = 0; r < n_ref; ++r) {
+		u32((uint32_t)h[0].names[r].size() + 1);
+		raw += h[0].names[r];
+		raw.push_back(0);
+		u32((uint32_t)h[0].lens[r]);
+	}
+	std::vector<uint8_t> hz(raw.size() + (raw.size() / bgzf::CHUNK + 2) * 64);
+	uint64_t body_offset = 0;
+	TRY(emab_bgzf_compress(c, (const uint8_t *)raw.data(), raw.size(), hz.data(), hz.size(), &body_offset));
+	if (w(uw, (const char *)hz.data(), body_offset) != 0) { snprintf(emab_errbuf, sizeof emab_errbuf, "emab_bam_merge_files: write failed"); return EMAB_ERR_IO; }
+	std::vector<Source> src((size_t)n_inputs);
+	for (int f = 0; f < n_inputs; ++f) {
+		Source &s = src[f];
+		s.path = paths[f]; s.bam = true; s.input = f;
+		s.foff = h[f].body_foff; s.drop = h[f].body_drop; s.fsize = h[f].fsize;
+	}
+	// the @SQ lengths on the device, for k_bam_rows (declared before the Writer, whose destructor waits for the stream)
+	DevBuf d_ref_len;
+	TRY(d_ref_len.ensure((size_t)n_ref * 4 + 16));
+	if (n_ref) CUDA_TRY(cudaMemcpyAsync(d_ref_len.p, h[0].lens.data(), (size_t)n_ref * 4, cudaMemcpyHostToDevice, c->stream));
+	Writer W(c, n_ref, h[0].lens.data(), body_offset, slice_chunks, w, uw, bai != nullptr);
+	TRY(W.start());
+	MergeCost cost;
+	TRY(merge_windows(c, src, W, budget, n_ref, d_ref_len.as<int32_t>(), cost));
+	TRY(W.finish(bai, bai_len));
+	if (ms) { ms[0] = cost.inflate; ms[1] = cost.rows; for (int k = 0; k < 4; ++k) ms[2 + k] = W.t[k]; }
+	if (counts) { counts[0] = cost.read; counts[1] = cost.inflated; counts[2] = cost.records; counts[3] = cost.windows; }
+	c->last_ms = cost.inflate + cost.rows + W.t[0] + W.t[2] + W.t[3];
 	return EMAB_OK;
 }

@@ -135,6 +135,7 @@ struct emab_ctx {
 	DevBuf sam_job, rec_off;                // the formatters' job (descriptors, barcodes) and record offsets
 	HostBuf job_stage;
 	DevBuf bgzf_tokens, bgzf_members, bgzf_off, bgzf_out;   // bgzf_compress_device's
+	DevBuf infl_in, infl_off, infl_out;                     // bgzf_inflate_device's
 };
 
 // BGZF members of d_in[0..n) (device memory) into the host buffer out (bgzf.cu); records ev1 after the last kernel.
@@ -142,6 +143,13 @@ struct emab_ctx {
 // out (one per chunk, then the total), valid until the ctx's next call.
 int bgzf_compress_device(emab_ctx *c, const uint8_t *d_in, uint64_t n, uint8_t *out, uint64_t out_cap, uint64_t *out_len, int *launches,
                          const unsigned long long **d_member_off = nullptr);
+
+// The whole BGZF members in[0..len) (host memory) inflated on the device into the ctx's infl_out after prefix[0..skip)
+// (host bytes copied there first, or none); *out_len receives the members' total content.  The host walks the BSIZE chain
+// (member framing) and scans ISIZE; a bad member fails with EMAB_ERR_IO naming `what`, its offset (plus `base`) and the
+// reason.  Synchronous; the content is valid until the ctx's next call.
+int bgzf_inflate_device(emab_ctx *c, const uint8_t *in, uint64_t len, const void *prefix, uint64_t skip, const char *what, uint64_t base,
+                        uint64_t *out_len);
 
 // first statement of every entry point that takes a ctx: a worker thread of the host pipeline (or any caller's
 // thread) starts on device 0, and a stream or buffer of another device is an invalid argument there

@@ -74,6 +74,7 @@ int emab_preproc(const char *whitelist_path, const char *const *count_files, int
                  int do_h2, uint64_t buffer_size, int do_bx_format, int n_threads, int n_buckets, int is_haplotag, FILE *in);
 
 int emab_ctx_create(emab_index_t *ix, emab_ctx_t **out);  /* ix may be NULL for the sequence-only SW calls */
+int emab_ctx_create_on(int device, emab_ctx_t **out);      /* a ctx without an index on `device` (BGZF and BAM calls) */
 void emab_ctx_free(emab_ctx_t *ctx);
 /* Makes the ctx's device current on the calling thread.  Every entry point that takes a ctx does this itself; a
  * thread that allocates pinned memory before its first ctx call uses it to stay off device 0. */
@@ -340,6 +341,41 @@ int emab_bam_merge(emab_ctx_t *ctx, int n_files, const char *const *paths, int n
                    emab_write_cb w, void *uw, char **bai, uint64_t *bai_len, double ms[4]);
 int emab_bgzf_compress(emab_ctx_t *ctx, const uint8_t *in, uint64_t len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
 int emab_bgzf_eof(const uint8_t **p, uint64_t *len);
+/* emab_bgzf_inflate = the device decoder (csrc/inflate.cuh): in[0..len) is a sequence of whole BGZF members, out receives their
+ *                    content back to back.  The host takes each member's offset from the BSIZE chain and its output offset
+ *                    from a scan of the ISIZE fields; one warp decodes each member (any DEFLATE block kinds) and checks its
+ *                    CRC-32 and ISIZE.  A malformed member fails the call with EMAB_ERR_IO, and emab_last_error() names the
+ *                    first bad member's byte offset and the reason (the codes of inflate.cuh).  The host's walk of the
+ *                    chain refuses bad framing and an ISIZE over 65 536 before any device work; then, with out_cap smaller
+ *                    than the content, EMAB_ERR_OVERFLOW and *out_len = the size needed.
+ *                    emab_last_kernel_ms gives the decoding kernel's time. */
+int emab_bgzf_inflate(emab_ctx_t *ctx, const uint8_t *in, uint64_t len, uint8_t *out, uint64_t out_cap, uint64_t *out_len);
+/* emab_bam_merge_files = coordinate-sorted BAM files merged into one sorted file (what `samtools merge` / `sambamba merge`
+ *                    give), inflated, ordered, compressed and indexed on the device.  The inputs must have identical reference
+ *                    lists (names and lengths, in order).  The header text starts from the first input's: its @HD line gets
+ *                    SO:coordinate (an @HD line is added when there is none); then, input by input, each @RG line whose ID is
+ *                    new is appended (the same ID with other text is refused, naming both files), each @PG line whose ID is
+ *                    new is appended (others are dropped) and every @CO line is appended.  The reference list is the first
+ *                    input's.  w receives the header's members (compressed as emab_sam_header does in BAM mode), then the
+ *                    body, without the EOF block.  Each input is read in whole members up to budget / (2 (inputs + 1))
+ *                    bytes of content per window, inflated on the device (emab_bgzf_inflate), and its records (the
+ *                    block_size chain, a record cut by a block's end carried into the next) get their sort rows on the
+ *                    device: key, end and len as emab_bam_key_t states them, bin recomputed as reg2bin(POS, end) (records
+ *                    are copied verbatim, their own bin is not read).  Equal keys keep argument order, then file order.  A
+ *                    record with block_size < 32, l_read_name 0, fields past its end, refID outside [-1, n_ref), a POS
+ *                    outside [0, LN) of its @SQ entry (outside [-1, 2^31 - 1) without a refID), an alignment ending past
+ *                    LN, or a key below the previous record's (not coordinate-sorted; unplaced records come last) fails the
+ *                    call with EMAB_ERR_IO naming the file and the record's ordinal; so does a malformed member (its byte
+ *                    offset) and a file that ends inside a record.  With bai != NULL the index comes back as from
+ *                    emab_session_finish: a contig of 2^29 bp or more fails the call with EMAB_ERR_ARG before anything
+ *                    is written.  ms[6] (optional): wall times of inflating (with reading), rows, the device ordering, the
+ *                    host gather, the compression and the index.  counts[4] (optional): compressed bytes read, inflated
+ *                    bytes, records, windows.
+ * emab_bam_merge_header = the header text emab_bam_merge_files would write, and all its refusals, on the host alone (no
+ *                    device; release the text with emab_free). */
+int emab_bam_merge_files(emab_ctx_t *ctx, int n_inputs, const char *const *paths, uint64_t budget, int slice_chunks, emab_write_cb w,
+                         void *uw, char **bai, uint64_t *bai_len, double ms[6], uint64_t counts[4]);
+int emab_bam_merge_header(int n_inputs, const char *const *paths, char **text, uint64_t *len);
 /* pinned host memory for callers that want their input buffers to take the fast H2D path */
 void *emab_pinned_alloc(uint64_t bytes);
 void emab_pinned_free(void *p);
